@@ -21,6 +21,15 @@ run at N = 1 and reported under ``secondary``.
 * ``cpu_baseline`` the CPU oracle port (reference algorithm incl. its mask +
                  masked_select gather) on this box's host cores, bounded sample.
 * ``--impl reference``: the CPU port alone, all host threads, same metric/config.
+* ``--dump-outputs DIR``: after the timed steps of the headline workload, write what its last step
+                 computed as float32 ``DIR/<name>.npy`` (rank 0): ``losses`` [loss, path, error, actor,
+                 critic] (what Trainer.train_step returns), ``params`` and ``param_grads`` (every
+                 parameter after the Adam update / the gradient it applied, concatenated in the order
+                 of model.parameters()), and the rollout's ``step_preds``, ``step_log_probas``,
+                 ``step_values`` and ``step_pos``.  The inputs, weights and draws are seeded, so two
+                 builds run with the same arguments can be compared output for output.  Two runs of one
+                 build agree on ``step_pos`` exactly and on the rest to ~1e-6 relative L2, not bit for
+                 bit (c4, 20 steps, one B200 at its 1000 W power limit).
 """
 from __future__ import annotations
 
@@ -193,7 +202,13 @@ def main() -> None:
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline", action="store_true", help="skip the micro-benchmarks (profiling runs)")
     ap.add_argument("--cpu-budget", type=float, default=15.0, help="seconds of CPU work for cpu_baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     args.warmup = max(3, args.warmup)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -253,7 +268,8 @@ def main() -> None:
     dp = DataParallelContext()
 
     clocks = ClockSampler(local_rank) if rank == 0 else None
-    res = measure(w, nb, args, dp, dev, world, rank, args.steps, args.warmup)
+    res = measure(w, nb, args, dp, dev, world, rank, args.steps, args.warmup,
+                  dump_dir=args.dump_outputs if rank == 0 else None)
     clk = clocks.stop() if clocks else None
     global_batch = nb * world
     if rank == 0:
@@ -282,7 +298,7 @@ def main() -> None:
     if world == 1 and not args.no_secondary and args.workload != "c2":
         # the reference's own configuration (README hyper-parameters, batch 8: 128 rows per step, latency-bound)
         w2 = WORKLOADS["c2"]
-        r2 = measure(w2, w2["B"], args, dp, dev, world, rank, max(20, args.steps), args.warmup)
+        r2 = measure(w2, w2["B"], args, dp, dev, world, rank, args.steps, args.warmup)
         v2 = w2["B"] / (r2["step_ms"] * 1e-3)
         line["secondary"] = {"c2": {"workload": f"c2: {w2['desc']}", "value": v2, "unit": "image-episodes/s",
                                     "agent_steps_per_sec": v2 * w2["na"] * w2["T"], "ms_per_step": r2["step_ms"],
@@ -318,9 +334,34 @@ def e2e_block(res: dict, global_batch: int) -> dict:
                          "input": "pinned host u8[B,H,W,C] (decoded image bytes), ToTensor on the device"}}
 
 
-def measure(w: dict, nb: int, args, dp, dev, world: int, rank: int, steps: int, warmup: int) -> dict:
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, loss_out: torch.Tensor, model, eng) -> None:
+    """Write one train step's outputs (names in the module docstring) as float32 DIR/<name>.npy."""
+    import numpy as np
+
+    flat_p, flat_g = model.flat_params, model.flat_grads
+    spans = [((p.data_ptr() - flat_p.data_ptr()) // 4, p.numel()) for p in model.parameters()]
+    arrays = {"losses": loss_out[:5],
+              "params": torch.cat([flat_p[o:o + n] for o, n in spans]),
+              "param_grads": torch.cat([flat_g[o:o + n] for o, n in spans]),
+              "step_preds": eng.step_preds, "step_log_probas": eng.step_log_probas, "step_values": eng.step_values,
+              "step_pos": eng.step_pos}
+    arrays = {k: v.detach().to("cpu", torch.float32).numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
+def measure(w: dict, nb: int, args, dp, dev, world: int, rank: int, steps: int, warmup: int,
+            dump_dir: str | None = None) -> dict:
     """Time one workload at `nb` images per GPU: device-resident `value`, `e2e` from pinned host batches
-    (fp32 and uint8), forward-only `eval`.  Every figure is the max over ranks."""
+    (fp32 and uint8), forward-only `eval`.  Every figure is the max over ranks.  `dump_dir`: write the
+    outputs of the last step of the `value` window there (see dump_outputs)."""
     import torch.distributed as dist
 
     from marlclassification_b200.config import ModelConfig
@@ -353,16 +394,17 @@ def measure(w: dict, nb: int, args, dp, dev, world: int, rank: int, steps: int, 
         torch.cuda.synchronize()
 
     def run(pool, ys, n):
-        """Time `n` steps with CUDA events on the current stream; returns (device ms, wall ms)."""
+        """Time `n` steps with CUDA events on the current stream; returns (device ms, wall ms, the
+        last step's loss tensor)."""
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(n)]
         t_wall = time.perf_counter()
         for i in range(n):
             evs[i][0].record()
-            trainer.train_step(pool[i % len(pool)], ys[i % len(pool)], sampler)
+            out = trainer.train_step(pool[i % len(pool)], ys[i % len(pool)], sampler)
             evs[i][1].record()
         torch.cuda.synchronize()
         wall = (time.perf_counter() - t_wall) * 1e3
-        return sum(a.elapsed_time(b) for a, b in evs), wall
+        return sum(a.elapsed_time(b) for a, b in evs), wall, out
 
     def run_eval(pool, n):
         """Forward-only episodes (Trainer.eval_step, the eval_epoch path), inputs resident."""
@@ -394,8 +436,10 @@ def measure(w: dict, nb: int, args, dp, dev, world: int, rank: int, steps: int, 
     # warm-up (also captures the CUDA graphs: 2 eager steps, then capture)
     run(dev_pool, dev_y, max(3, warmup))
     barrier()
-    dev_ms, wall_ms = run(dev_pool, dev_y, steps)
+    dev_ms, wall_ms, loss_out = run(dev_pool, dev_y, steps)
     barrier()
+    if dump_dir:
+        dump_outputs(dump_dir, loss_out, model, sampler.engine_for(dev_pool[0], gamma=0.99))
     # the step stream is saturated only if the host keeps ahead; report the slower of
     # device-event time and wall time so host-bound runs are not flattered
     step_ms = max(dev_ms, wall_ms) / steps

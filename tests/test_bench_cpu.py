@@ -31,6 +31,13 @@ def test_reference_arm_json_contract():
     assert cfg["global_batch"] == 32 and cfg["parallelism"] == "dp1" and "l2" in cfg
 
 
+def test_unusable_arguments_are_refused():
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                             timeout=120)
+        assert out.returncode == 2 and out.stdout == "", (args, out.stderr[-500:])
+
+
 def test_default_workload_is_config_4_strong_scaling():
     sys.path.insert(0, ROOT)
     import bench
