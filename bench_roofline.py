@@ -277,7 +277,7 @@ def roofline_for(model, w: dict, nb: int, dev) -> dict:
     if os.path.exists(tpath):
         with open(tpath) as fh:
             cap = json.load(fh)["captures"]
-        best = cap.get("tile 128x256 (HU=64, default from M>=2368)", {})
+        best = cap.get("tile 128x256 (HU=64, default from M>=1793 at n=256)", {})
         try:
             traffic = (float(best["dram__bytes_read.sum"][0]) + float(best["dram__bytes_write.sum"][0])) * 1e6
             ncu_lstm = {"tensor_pipe_active_pct": float(best["sm__pipe_tensor_cycles_active.avg.pct_of_peak_sustained_active"][0]),

@@ -123,6 +123,31 @@ typedef struct marlc_engine marlc_engine;
 int marlc_engine_create(const marlc_config* cfg, marlc_engine** out);
 void marlc_engine_destroy(marlc_engine* e);
 
+/* What the engine's launchers choose for its geometry (per step: M = na*nb rows).  Host only: works on an
+ * engine that is created but not bound, and no GPU is needed.  The launchers decide with the same functions. */
+typedef struct marlc_plan {
+    /* feature-extractor forward */
+    int cnn_wide;       /* 1: persistent CTAs with stationary weights, batches of cnn_nw windows; 0: one CTA per window */
+    int cnn_nw;         /* windows per batch (1 per window) */
+    int cnn_batches;    /* ceil(M / cnn_nw) */
+    int cnn_ctas;       /* CTAs of the feature-extractor role */
+    int cnn_passes;     /* batches of the busiest CTA: ceil(cnn_batches / cnn_ctas) */
+    int cnn_tail;       /* windows in the last batch */
+    /* both LSTM cells of a step */
+    int lstm_tc;        /* 1: one fused tensor-core launch; 0: FFMA gate GEMMs + point-wise cell (the fields below are 0) */
+    int lstm_hu;        /* hidden units per CTA (x 4 gates = lstm_bn output columns) */
+    int lstm_bn;
+    int lstm_fat;       /* 1: fat pipeline stages (latency-bound launch) */
+    int lstm_ks;        /* 32-float K sub-blocks per stage */
+    int lstm_ksplit;    /* CTAs that split K (2: cluster pair with a shared-memory reduction) */
+    int lstm_tail_rows; /* rows in the last 128-row tile */
+    /* backward */
+    int sweep_chained;  /* 1: BPTT sweep with the fused chain kernels; 0: one kernel per op */
+    /* chain kernels (0 when use_chains == 0): weights staged in shared memory per CTA */
+    int staged_step_pre, staged_step_post, staged_bwd_pre, staged_bwd_post;
+} marlc_plan;
+int marlc_engine_plan(const marlc_engine* e, marlc_plan* out);
+
 /* Flat parameter layout (reference state_dict names, models.py:55-76). */
 int marlc_engine_param_count(const marlc_engine* e);
 /* name buffer >= 128 bytes; shape has 4 entries (unused = 1); offset in floats. */

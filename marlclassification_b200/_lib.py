@@ -30,6 +30,18 @@ class MarlcConfig(C.Structure):
     ]
 
 
+class MarlcPlan(C.Structure):
+    """Mirror of ``marlc_plan`` (include/marlc.h): what the engine's launchers choose for its geometry."""
+
+    _fields_ = [(name, C.c_int) for name in (
+        "cnn_wide", "cnn_nw", "cnn_batches", "cnn_ctas", "cnn_passes", "cnn_tail",
+        "lstm_tc", "lstm_hu", "lstm_bn", "lstm_fat", "lstm_ks", "lstm_ksplit", "lstm_tail_rows",
+        "sweep_chained", "staged_step_pre", "staged_step_post", "staged_bwd_pre", "staged_bwd_post")]
+
+    def as_dict(self) -> dict:
+        return {name: getattr(self, name) for name, _ in self._fields_}
+
+
 _P = C.c_void_p
 _SIGS = {
     "marlc_version": (C.c_int, []),
@@ -51,6 +63,7 @@ _SIGS = {
                                     C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), _P, _P, C.c_int, _P]),
     "marlc_engine_create": (C.c_int, [C.POINTER(MarlcConfig), C.POINTER(_P)]),
     "marlc_engine_destroy": (None, [_P]),
+    "marlc_engine_plan": (C.c_int, [_P, C.POINTER(MarlcPlan)]),
     "marlc_engine_param_count": (C.c_int, [_P]),
     "marlc_engine_param_info": (C.c_int, [_P, C.c_int, C.c_char_p, C.POINTER(C.c_int64), C.POINTER(C.c_int),
                                           C.POINTER(C.c_int64)]),

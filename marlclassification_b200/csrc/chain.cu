@@ -284,6 +284,22 @@ static int maxw_of(std::initializer_list<int> v) {
     for (int x : v) m = max(m, x);
     return (m + 3) & ~3;
 }
+ChainStage step_pre_stage(int n_m, int n1, int n2, int nd) {
+    const int maxw = maxw_of({n_m, n1, n2, nd});
+    return {maxw, staged_floats(maxw, n1, odd_pitch(n_m), n2, odd_pitch(n1))};
+}
+ChainStage step_post_stage(int M, int n1, int n2) {
+    const int maxw = maxw_of({n1, n2});
+    return {maxw, stage_weights_for(M) ? staged_floats(maxw, n2, odd_pitch(n1), 0, 0) : 0};
+}
+ChainStage bwd_pre_stage(int M, int n_m, int n1, int nb) {
+    const int maxw = maxw_of({n_m, n1, nb});
+    return {maxw, stage_weights_for(M) ? staged_floats(maxw, n_m, n1, n1, nb) : 0};
+}
+ChainStage bwd_post_stage(int M, int n_m, int n1, int n2) {
+    const int maxw = maxw_of({n_m, n1, n2});
+    return {maxw, stage_weights_for(M) ? staged_floats(maxw, n2, n1, n1, n_m) : 0};
+}
 
 // ---------------------------------------------------------------------------------
 // forward "pre": CNN role (blocks [0,M)) | decoder + position-feature role
@@ -415,27 +431,39 @@ static int persistent_blocks(int nrb, size_t smem_bytes, int waves = 1) {
 
 static int step_pre_small(const StepPreArgs& a, cudaStream_t s);
 
-int step_pre(const StepPreArgs& a, cudaStream_t s) {
-    if (a.M <= 0) return 0;
+StepPrePlan step_pre_plan(const CnnDesc& d, bool have_img, bool have_wT, int M, CnnWidePlan* wide) {
     // feature extractor: one CTA per window while a step has few windows (latency-bound, every SM gets one:
     // step_pre_kernel); from MARLC_CNN_WIDE_MIN windows on, persistent CTAs with stationary weights, 8 windows
     // per pass, next to persistent decoder CTAs (step_pre_wide_kernel)
     static const int wide_min = getenv("MARLC_CNN_WIDE_MIN") ? atoi(getenv("MARLC_CNN_WIDE_MIN")) : 256;
-    static_assert(CW_THREADS == CT, "the wide feature extractor runs inside the chain kernel's CTA shape");
-    StepPreWideArgs ka;
-    memset(&ka.wide, 0, sizeof(ka.wide));
     // 8 windows per pass; 4 (MARLC_CNN_WIDE_NW=4: twice the CTAs while 8 leave SMs idle) measured slower at
     // 512 and 1024 windows (476 vs 438 us, 795 vs 745 us per 16 steps): a pass is bound by the latency of its
     // phases, not by its FMA count
     static const int nw_env = getenv("MARLC_CNN_WIDE_NW") ? atoi(getenv("MARLC_CNN_WIDE_NW")) : 0;
     const int nw = nw_env ? nw_env : CW_NW;
-    if (a.M >= wide_min) ka.wide = cnn_wide_plan(a.cnn.d, a.cnn.img != nullptr && a.cnn.patch == nullptr, nw);
+    CnnWidePlan w;
+    memset(&w, 0, sizeof(w));
+    if (M >= wide_min) w = cnn_wide_plan(d, have_img, have_wT, nw);
+    if (wide) *wide = w;
+    StepPrePlan p;
+    p.nw = w.ok ? nw : 1;
+    p.cnn_blocks = w.ok ? min((M + nw - 1) / nw, MARLC_SMS) : 0;
+    return p;
+}
+
+int step_pre(const StepPreArgs& a, cudaStream_t s) {
+    if (a.M <= 0) return 0;
+    static_assert(CW_THREADS == CT, "the wide feature extractor runs inside the chain kernel's CTA shape");
+    StepPreWideArgs ka;
+    // (the chain path keeps transposed conv weights: engine.cu allocates them whenever the chains are on)
+    const StepPrePlan pl = step_pre_plan(a.cnn.d, a.cnn.img != nullptr && a.cnn.patch == nullptr, true, a.M, &ka.wide);
     if (!ka.wide.ok) return step_pre_small(a, s);
     ka.a = a;
-    ka.maxw = maxw_of({a.d0.n_in, a.d0.n_out, a.d3.n_out, a.pos.n_out});
-    const int wfl = staged_floats(ka.maxw, a.d0.n_out, odd_pitch(a.d0.n_in), a.d3.n_out, odd_pitch(a.d3.n_in));
+    const ChainStage st = step_pre_stage(a.d0.n_in, a.d0.n_out, a.d3.n_out, a.pos.n_out);
+    ka.maxw = st.maxw;
+    const int wfl = st.wfl;
     ka.staged = wfl > 0;
-    ka.cnn_blocks = min((a.M + nw - 1) / nw, MARLC_SMS);
+    ka.cnn_blocks = pl.cnn_blocks;
     const size_t smem = max(chain_smem_bytes(ka.maxw) + sizeof(float) * (size_t)wfl, sizeof(float) * (size_t)ka.wide.smem_floats);
     MARLC_CHECK(smem <= 226 * 1024, "step_pre: shared memory %zu B too large", smem);
     static size_t attr = 0;
@@ -558,8 +586,9 @@ static int step_pre_small(const StepPreArgs& a, cudaStream_t s) {
     if (a.M <= 0) return 0;
     StepPreKernelArgs ka;
     ka.a = a;
-    ka.maxw = maxw_of({a.d0.n_in, a.d0.n_out, a.d3.n_out, a.pos.n_out});
-    const int wfl = staged_floats(ka.maxw, a.d0.n_out, odd_pitch(a.d0.n_in), a.d3.n_out, odd_pitch(a.d3.n_in));
+    const ChainStage st = step_pre_stage(a.d0.n_in, a.d0.n_out, a.d3.n_out, a.pos.n_out);
+    ka.maxw = st.maxw;
+    const int wfl = st.wfl;
     ka.staged = wfl > 0;
     const size_t smem = max(chain_smem_bytes(ka.maxw) + sizeof(float) * (size_t)wfl, cnn_fwd_smem_bytes(a.cnn));
     MARLC_CHECK(smem <= 200 * 1024, "step_pre: shared memory %zu B too large", smem);
@@ -770,9 +799,10 @@ int step_post(const StepPostArgs& a, cudaStream_t s) {
     MARLC_CHECK(a.act.nA <= MAX_ACT, "step_post: nb_action=%d > %d", a.act.nA, MAX_ACT);
     StepPostKernelArgs ka;
     ka.a = a;
-    ka.maxw = maxw_of({a.e3.n_in, a.e3.n_out});
+    const ChainStage st = step_post_stage(a.M, a.e3.n_in, a.e3.n_out);
+    ka.maxw = st.maxw;
     ka.pol_blocks = (a.M + CT / 32 - 1) / (CT / 32);
-    const int wfl = stage_weights_for(a.M) ? staged_floats(ka.maxw, a.e3.n_out, odd_pitch(a.e3.n_in), 0, 0) : 0;
+    const int wfl = st.wfl;
     ka.staged = wfl > 0;
     const size_t smem = max(chain_smem_bytes(ka.maxw) + sizeof(float) * (size_t)wfl, sizeof(float) * (size_t)(CT / 32) * a.act.nl);
     MARLC_CHECK(smem <= 200 * 1024, "step_post: shared memory %zu B too large", smem);
@@ -1045,8 +1075,9 @@ int bwd_pre(const BwdPreArgs& a, cudaStream_t s) {
     if (a.M <= 0) return 0;
     BwdPreKernelArgs ka;
     ka.a = a;
-    ka.maxw = maxw_of({a.n_m, a.e0.n_out, a.n[0]});
-    const int wfl = stage_weights_for(a.M) ? staged_floats(ka.maxw, a.n_m, a.e0.n_out, a.e0.n_out, a.n[0]) : 0;
+    const ChainStage st = bwd_pre_stage(a.M, a.n_m, a.e0.n_out, a.n[0]);
+    ka.maxw = st.maxw;
+    const int wfl = st.wfl;
     ka.staged = wfl > 0;
     const size_t smem = chain_smem_bytes(ka.maxw) + sizeof(float) * (size_t)wfl;
     MARLC_CHECK(smem <= 200 * 1024, "bwd_pre: shared memory %zu B too large", smem);
@@ -1166,8 +1197,9 @@ int bwd_post(const BwdPostArgs& a, cudaStream_t s) {
     if (a.M <= 0) return 0;
     BwdPostKernelArgs ka;
     ka.a = a;
-    ka.maxw = maxw_of({a.n_m, a.d0.n_out, a.n_m_o});
-    const int wfl = stage_weights_for(a.M) ? staged_floats(ka.maxw, a.n_m_o, a.d0.n_out, a.d0.n_out, a.n_m) : 0;
+    const ChainStage st = bwd_post_stage(a.M, a.n_m, a.d0.n_out, a.n_m_o);
+    ka.maxw = st.maxw;
+    const int wfl = st.wfl;
     ka.staged = wfl > 0;
     const size_t smem = chain_smem_bytes(ka.maxw) + sizeof(float) * (size_t)wfl;
     MARLC_CHECK(smem <= 200 * 1024, "bwd_post: shared memory %zu B too large", smem);

@@ -96,4 +96,18 @@ struct BwdPostArgs {
 };
 int bwd_post(const BwdPostArgs& a, cudaStream_t s);
 
+// ---- host-side launch plans: the launchers above and marlc_engine_plan call the same functions
+struct CnnWidePlan;
+// Feature-extractor role of step_pre for M windows: the wide extractor (cnn_wide.cuh) in cnn_blocks persistent CTAs,
+// nw windows per batch, or (cnn_blocks == 0) one CTA per window.  `wide` (optional) receives the wide layout.
+struct StepPrePlan { int nw, cnn_blocks; };
+StepPrePlan step_pre_plan(const CnnDesc& d, bool have_img, bool have_wT, int M, CnnWidePlan* wide = nullptr);
+// Shared memory of one chain launcher: row-buffer width and floats of weights staged per CTA (0: the weights are
+// read through L1 / L2).
+struct ChainStage { int maxw, wfl; };
+ChainStage step_pre_stage(int n_m, int n1, int n2, int nd);
+ChainStage step_post_stage(int M, int n1, int n2);
+ChainStage bwd_pre_stage(int M, int n_m, int n1, int nb);
+ChainStage bwd_post_stage(int M, int n_m, int n1, int n2);
+
 }  // namespace marlc

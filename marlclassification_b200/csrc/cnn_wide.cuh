@@ -42,18 +42,20 @@ struct CnnWidePlan {
     int smem_floats;
 };
 
-inline CnnWidePlan cnn_wide_plan(const CnnDesc& d, bool have_img, int nw = CW_NW) {
+// have_wT: the engine keeps transposed conv weights (d.wT, one buffer per layer; with the chain kernels).  A flag
+// rather than a test of d.wT[0], which is only set at bind, so that an engine's plan can be queried before.
+inline CnnWidePlan cnn_wide_plan(const CnnDesc& d, bool have_img, bool have_wT, int nw = CW_NW) {
     CnnWidePlan p;
     memset(&p, 0, sizeof(p));
     p.nw = nw;
 #ifdef MARLC_CW_NW4
-    if (!have_img || !d.wT[0] || (nw != 8 && nw != 4)) return p;
+    if (!have_img || !have_wT || (nw != 8 && nw != 4)) return p;
 #else
-    if (!have_img || !d.wT[0] || nw != 8) return p;
+    if (!have_img || !have_wT || nw != 8) return p;
 #endif
     int off = 0;
     for (int l = 0; l < d.L; ++l) {
-        if (!d.wT[l] || (d.cout[l] & 3) || d.groups[l] > 32 || d.cout[l] % d.groups[l]) return p;
+        if ((d.cout[l] & 3) || d.groups[l] > 32 || d.cout[l] % d.groups[l]) return p;
         p.w_off[l] = off;
         off += d.cout[l] * d.cin[l] * 9;
     }

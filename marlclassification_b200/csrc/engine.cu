@@ -471,6 +471,54 @@ static int refresh_lo(marlc_engine* e, const float* h0, const float* hc0, cudaSt
 
 // ---- GEMM dispatch: tcgen05 TF32 when enabled and TMA-addressable, else exact fp32 FFMA ----------
 static inline int x3_of(const marlc_engine* e) { return e->cfg.use_tc == 2 ? 1 : 0; }
+
+// ---- launch decisions that depend on the geometry only (the launchers and marlc_engine_plan share them)
+// both LSTM cells in one tensor-core launch (tc_lstm_pair) rather than FFMA gate GEMMs + point-wise cells
+static bool lstm_on_tc(const marlc_engine* e) {
+    const marlc_config& c = e->cfg;
+    return c.use_tc && c.n_a == c.n_b && tc_lstm_shapes_ok(e->Kin, c.n_b);
+}
+// Fused chain kernels for the sweep while a step has fewer than 4096 rows (latency-bound: 3 launches per step).
+// From 4096 rows per step on (config 4 on ONE GPU) the one-kernel-per-op sweep with its products on the
+// tensor cores wins: the chains run 4 rows per CTA, one CTA per SM.  Measured (sweep of 16 steps): 4096 rows
+// 2.72 vs 3.01 ms, 2048 rows 2.91 vs 2.48 ms -- hence the threshold (MARLC_SWEEP_UNFUSED_MIN_M).
+static bool sweep_chained(const marlc_engine* e) {
+    static const int unfused_min_m = getenv("MARLC_SWEEP_UNFUSED_MIN_M") ? atoi(getenv("MARLC_SWEEP_UNFUSED_MIN_M")) : 4096;
+    return e->cfg.use_chains && e->M < unfused_min_m;
+}
+
+extern "C" int marlc_engine_plan(const marlc_engine* e, marlc_plan* out) {
+    MARLC_CHECK(e && out, "plan: null argument");
+    const marlc_config& c = e->cfg;
+    const int M = e->M;
+    marlc_plan p;
+    memset(&p, 0, sizeof(p));
+    // feature extractor of the episode forward: step_pre with the chains, else cnn_fwd (one CTA per window)
+    const StepPrePlan sp = c.use_chains ? step_pre_plan(e->cnn, true, true, M) : StepPrePlan{1, 0};
+    p.cnn_wide = sp.cnn_blocks > 0;
+    p.cnn_nw = sp.nw;
+    p.cnn_batches = (M + sp.nw - 1) / sp.nw;
+    p.cnn_ctas = p.cnn_wide ? sp.cnn_blocks : M;
+    p.cnn_passes = (p.cnn_batches + p.cnn_ctas - 1) / p.cnn_ctas;
+    p.cnn_tail = M - (p.cnn_batches - 1) * sp.nw;
+    if (lstm_on_tc(e)) {
+        const TcLstmPlan lp = tc_lstm_plan(M, c.n_b, c.n_a, x3_of(e) != 0);
+        p.lstm_tc = 1;
+        p.lstm_hu = lp.hu; p.lstm_bn = lp.bn; p.lstm_fat = lp.fat; p.lstm_ks = lp.ks; p.lstm_ksplit = lp.ksplit;
+        p.lstm_tail_rows = lp.tail_rows;
+    }
+    p.sweep_chained = sweep_chained(e);
+    if (c.use_chains) {
+        p.staged_step_pre = step_pre_stage(c.n_m, 2 * c.n_m, c.n_m_o, c.n_d).wfl > 0;
+        p.staged_step_post = step_post_stage(M, 2 * c.n_m, c.n_m).wfl > 0;
+    }
+    if (p.sweep_chained) {
+        p.staged_bwd_pre = bwd_pre_stage(M, c.n_m, 2 * c.n_m, c.n_b).wfl > 0;
+        p.staged_bwd_post = bwd_post_stage(M, c.n_m, 2 * c.n_m, c.n_m_o).wfl > 0;
+    }
+    *out = p;
+    return 0;
+}
 static bool tc_worth(int m_out, int n_out, int k_red) { return n_out >= 16 && k_red >= 32 && m_out >= 1; }
 
 // Y[M,N] = X[M,K] W[N,K]^T + bias
@@ -621,7 +669,7 @@ static int step_networks(marlc_engine* e, int t, const float* img, const int* po
     float* gb = e->buf("gates_b") + (size_t)t * M * 4 * c.n_b;
     float* ga = e->buf("gates_a") + (size_t)t * M * 4 * c.n_a;
     bool fused = false;
-    if (c.use_tc && c.n_a == c.n_b) {
+    if (lstm_on_tc(e)) {
         TcLstmArgs la[2];
         for (int k = 0; k < 2; ++k) {
             const std::string pre = k ? LSTM_A : LSTM_B;
@@ -1149,12 +1197,7 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
     MARLC_CUDA(cudaMemsetAsync(dc[0], 0, sizeof(float) * (size_t)M * c.n_b, s));
     MARLC_CUDA(cudaMemsetAsync(dcc[0], 0, sizeof(float) * (size_t)M * c.n_a, s));
     int cur = 0;
-    // Fused chain kernels for the sweep while a step has fewer than 4096 rows (latency-bound: 3 launches per step).
-    // From 4096 rows per step on (config 4 on ONE GPU) the one-kernel-per-op sweep with its products on the
-    // tensor cores wins: the chains run 4 rows per CTA, one CTA per SM.  Measured (sweep of 16 steps): 4096 rows
-    // 2.72 vs 3.01 ms, 2048 rows 2.91 vs 2.48 ms -- hence the threshold (MARLC_SWEEP_UNFUSED_MIN_M).
-    static const int unfused_min_m = getenv("MARLC_SWEEP_UNFUSED_MIN_M") ? atoi(getenv("MARLC_SWEEP_UNFUSED_MIN_M")) : 4096;
-    const bool chain_sweep = c.use_chains && M < unfused_min_m;
+    const bool chain_sweep = sweep_chained(e);  // fused chain kernels, or one kernel per op from 4096 rows on
     if (chain_sweep) {
         float* dcoll = e->buf("dcoll");
         float* dh_hist = e->buf("dh_hist");

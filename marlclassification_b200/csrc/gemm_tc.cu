@@ -1064,17 +1064,17 @@ static int launch_lstm(TcKernelGroup& kp, int gx, int gy, int nkb, cudaStream_t 
     return 0;
 }
 
+bool tc_lstm_shapes_ok(int Kin, int n) { return Kin % 4 == 0 && n % 8 == 0 && n >= 8; }
+
 bool tc_lstm_supported(const TcLstmArgs& a) {
     return tc_operand_ok(a.U) && tc_operand_ok(a.Hprev) && (((uintptr_t)a.Wih | (uintptr_t)a.Whh) & 15) == 0 &&
-           a.Kin % 4 == 0 && a.n % 8 == 0 && a.n >= 8 && (((uintptr_t)a.c_prev | (uintptr_t)a.c_new | (uintptr_t)a.h_new |
+           tc_lstm_shapes_ok(a.Kin, a.n) && (((uintptr_t)a.c_prev | (uintptr_t)a.c_new | (uintptr_t)a.h_new |
            (uintptr_t)a.gates) & 15) == 0;
 }
 
-int tc_lstm_pair(const TcLstmArgs& c0, const TcLstmArgs& c1, cudaStream_t s) {
-    MARLC_CHECK(tc_lstm_supported(c0) && tc_lstm_supported(c1), "tc_lstm_pair: unsupported shapes / alignment");
-    MARLC_CHECK(c0.M == c1.M, "tc_lstm_pair: row counts differ");
+TcLstmPlan tc_lstm_plan(int M, int n0, int n1, bool x3) {
     // hidden units per CTA: small tiles when M is small (more CTAs), 32 when rows are plentiful
-    const int mt = (c0.M + BM - 1) / BM;
+    const int mt = (M + BM - 1) / BM;
     int HU = mt >= 8 ? 32 : (mt >= 2 ? 16 : 8);
     // 128 x 256 tiles (64 hidden units x 4 gates) once they still fill the machine: a kind::tf32 MMA reads its
     // operands from shared memory at 128 B/clk for a 128 x 128 tile (the whole shared-memory bandwidth of the
@@ -1082,20 +1082,13 @@ int tc_lstm_pair(const TcLstmArgs& c0, const TcLstmArgs& c1, cudaStream_t s) {
     // 25 % fewer operand bytes per flop (MARLC_LSTM_HU64=0 switches it off)
     static const int hu64 = getenv("MARLC_LSTM_HU64") ? atoi(getenv("MARLC_LSTM_HU64")) : 1;
     // (measured, 16 steps at n = 256: M = 2048 -> 796 us with 64 units per tile vs 858 with 32; M = 1024 -> 673 vs 439)
-    if (hu64 && c0.n % 64 == 0 && c1.n % 64 == 0 && 2 * mt * (c0.n / 64) >= 120) HU = 64;
+    if (hu64 && n0 % 64 == 0 && n1 % 64 == 0 && 2 * mt * (n0 / 64) >= 120) HU = 64;
     static const int hu_force = getenv("MARLC_LSTM_HU") ? atoi(getenv("MARLC_LSTM_HU")) : 0;  // A/B toggle
     if (hu_force == 8 || hu_force == 16 || hu_force == 32 || hu_force == 64) HU = hu_force;
-    while (HU > 8 && (c0.n % HU != 0 || c1.n % HU != 0)) HU >>= 1;
-    MARLC_CHECK(c0.n % HU == 0 && c1.n % HU == 0, "tc_lstm_pair: hidden size not a multiple of %d", HU);
-    TcKernelGroup kp;
-    memset(&kp, 0, sizeof(kp));
-    kp.count = 2;
-    kp.zofs[0] = 0; kp.zofs[1] = 1; kp.zofs[2] = 2;
+    while (HU > 8 && (n0 % HU != 0 || n1 % HU != 0)) HU >>= 1;
     // few CTAs (small M): fat stages, KS sub-blocks of 32 floats per barrier round trip
-    const bool fat = HU <= 16 && 2 * mt * (c0.n / HU) <= MARLC_SMS;
-    const int KSv = !fat ? 1 : (c0.x3 ? 2 : (HU == 8 ? 4 : 2));
-    const int BKS = BK * KSv;
-    const TcLstmArgs* cs[2] = {&c0, &c1};
+    const bool fat = HU <= 16 && 2 * mt * (n0 / HU) <= MARLC_SMS;
+    const int KSv = !fat ? 1 : (x3 ? 2 : (HU == 8 ? 4 : 2));
     // A-tile multicast: the n/HU CTAs of one M tile all read the same 128 x K activations; in a cluster
     // of `cl` of them each CTA requests 1/cl of every A tile and the TMA unit delivers it to all
     // (the main loop is bound by what one SM's TMA engine can request, ~40-50 B/clk measured)
@@ -1103,12 +1096,32 @@ int tc_lstm_pair(const TcLstmArgs& c0, const TcLstmArgs& c1, cudaStream_t s) {
     // bytes ARRIVING in each SM, not the requests its TMA engine issues; off unless MARLC_LSTM_CLUSTER)
     int cl = 1;
     if (const char* env = getenv("MARLC_LSTM_CLUSTER")) cl = atoi(env);
-    while (cl > 1 && ((c0.n / HU) % cl != 0 || (BM / cl) % 8 != 0)) cl >>= 1;
+    while (cl > 1 && ((n0 / HU) % cl != 0 || (BM / cl) % 8 != 0)) cl >>= 1;
     if (cl < 1) cl = 1;
     // K split over CTA pairs (DSMEM reduction): halves the bytes each SM streams; used when the launch is
     // small enough that twice the CTAs still fit in one wave
-    int ksplit = (fat && HU == 8 && cl == 1 && 2 * 2 * mt * (c0.n / HU) <= MARLC_SMS) ? 2 : 1;
+    int ksplit = (fat && HU == 8 && cl == 1 && 2 * 2 * mt * (n0 / HU) <= MARLC_SMS) ? 2 : 1;
     if (const char* env = getenv("MARLC_LSTM_KSPLIT")) ksplit = (atoi(env) == 2 && fat && HU == 8 && cl == 1) ? 2 : 1;
+    TcLstmPlan p;
+    p.hu = HU; p.bn = 4 * HU; p.fat = fat ? 1 : 0; p.ks = KSv; p.ksplit = ksplit; p.cluster = cl;
+    p.tail_rows = M - (mt - 1) * BM;
+    return p;
+}
+
+int tc_lstm_pair(const TcLstmArgs& c0, const TcLstmArgs& c1, cudaStream_t s) {
+    MARLC_CHECK(tc_lstm_supported(c0) && tc_lstm_supported(c1), "tc_lstm_pair: unsupported shapes / alignment");
+    MARLC_CHECK(c0.M == c1.M, "tc_lstm_pair: row counts differ");
+    const int mt = (c0.M + BM - 1) / BM;
+    const TcLstmPlan pl = tc_lstm_plan(c0.M, c0.n, c1.n, c0.x3 != 0);
+    const int HU = pl.hu, KSv = pl.ks, cl = pl.cluster, ksplit = pl.ksplit;
+    const bool fat = pl.fat != 0;
+    MARLC_CHECK(c0.n % HU == 0 && c1.n % HU == 0, "tc_lstm_pair: hidden size not a multiple of %d", HU);
+    TcKernelGroup kp;
+    memset(&kp, 0, sizeof(kp));
+    kp.count = 2;
+    kp.zofs[0] = 0; kp.zofs[1] = 1; kp.zofs[2] = 2;
+    const int BKS = BK * KSv;
+    const TcLstmArgs* cs[2] = {&c0, &c1};
     const int abox = BM / cl;
     int gx = 0;
     for (int k = 0; k < 2; ++k) {

@@ -134,6 +134,12 @@ class EpisodeEngine:
         if self.model.flat_params.data_ptr() != self._params.data_ptr():
             raise RuntimeError("model parameters were re-allocated after the engine was built; rebuild the engine")
 
+    def plan(self) -> dict:
+        """What the launchers choose for this geometry (``marlc_plan``, include/marlc.h)."""
+        plan = _lib.MarlcPlan()
+        _lib.check(self._L.marlc_engine_plan(self._h, ct.byref(plan)))
+        return plan.as_dict()
+
     def seed(self, seed: int) -> None:
         _lib.check(self._L.marlc_engine_seed(self._h, ct.c_uint64(seed), self._stream()))
 
@@ -209,6 +215,19 @@ class EpisodeEngine:
 
 def C_void_p():
     return ct.c_void_p()
+
+
+def engine_plan(cfg: MarlcConfig) -> dict:
+    """``marlc_plan`` of an engine created for ``cfg`` and never bound: no device memory, no GPU needed."""
+    L = _lib.lib()
+    h = ct.c_void_p()
+    _lib.check(L.marlc_engine_create(ct.byref(cfg), ct.byref(h)))
+    try:
+        plan = _lib.MarlcPlan()
+        _lib.check(L.marlc_engine_plan(h, ct.byref(plan)))
+        return plan.as_dict()
+    finally:
+        L.marlc_engine_destroy(h)
 
 
 def get_engine(model, *, na, nb, T, C, H, W, actions, gamma=0.99) -> EpisodeEngine:

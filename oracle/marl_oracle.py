@@ -148,10 +148,11 @@ def transition(
     return torch.where(ok.unsqueeze(-1), new, pos)
 
 
-def normalized_positions(pos: torch.Tensor, sizes: Sequence[int]) -> torch.Tensor:
-    """environment.py:74-81: float(pos) / float(size), true fp32 division."""
+def normalized_positions(pos: torch.Tensor, sizes: Sequence[int], dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    """environment.py:74-81: float(pos) / float(size), true fp32 division (what the reference and the
+    engine compute, whatever precision the networks run in), returned as ``dtype``."""
     s = torch.tensor([[list(sizes)]], dtype=torch.float32, device=pos.device)
-    return pos.to(torch.float32) / s
+    return (pos.to(torch.float32) / s).to(dtype)
 
 
 # --------------------------------------------------------------------------
@@ -200,16 +201,19 @@ def lstm_cell(p, prefix: str, u, h, c):
     return h2, c2
 
 
-def step_forward(p, cfg: OracleConfig, patch, msg, npos, hid):
+def step_forward(p, cfg: OracleConfig, patch, msg, npos, hid, record: Optional[dict] = None):
     """models.py:78-138, one step of every network for all Na*Nb rows.
     patch [Na,Nb,C,f,f]; msg [Na,Nb,n_m]; npos [Na,Nb,2];
-    hid = (h, c, h^, c^).  Returns probs, values, preds, new_msg, new_hid."""
+    hid = (h, c, h^, c^).  Returns probs, values, preds, new_msg, new_hid.
+    ``record`` (a dict) receives the LSTM input u [Na*Nb, Kin]."""
     na, nb = patch.shape[:2]
     h, c, hc, cc = hid
     b_t = cnn_forward(p, cfg, patch.flatten(0, 1)).view(na, nb, -1)
     d_bar = lin_ln_silu(p, "decode_msg", 3, lin_ln_silu(p, "decode_msg", 0, aggregate_messages(msg)))
     lam = lin_ln_silu(p, "map_pos", 0, npos)
     u = torch.cat((b_t, d_bar, lam), dim=2).flatten(0, 1)
+    if record is not None:
+        record["u"] = u
     h2, c2 = lstm_cell(p, LSTM_B, u, h.flatten(0, 1), c.flatten(0, 1))
     h2, c2 = h2.view(na, nb, -1), c2.view(na, nb, -1)
     new_msg = lin_ln_silu(p, "encode_msg", 3, lin_ln_silu(p, "encode_msg", 0, h2))
@@ -236,6 +240,10 @@ class Rollout:
     patches: List[torch.Tensor]  # T+1 observations (o_0 .. o_T)
     actions: torch.Tensor  # [T,Na,Nb] int64
     final_hidden: Tuple[torch.Tensor, ...]
+    # per-step values (rollout(record=True)): for each step t a dict with the LSTM input "u" [Na*Nb, Kin]
+    # (CNN features | decoded message | position features), the new state "h", "c", "h_caret", "c_caret"
+    # [Na,Nb,n] and the message "msg" [Na,Nb,n_m] it emits
+    steps: Optional[List[Dict[str, torch.Tensor]]] = None
 
 
 def rollout(
@@ -249,24 +257,32 @@ def rollout(
     *,
     faithful_gather: bool = False,
     generator: Optional[torch.Generator] = None,
+    record: bool = False,
 ) -> Rollout:
     """episode.py:32-82 + agent.py:40-68 + environment.py:23-68 with the three
     random sites injected: initial positions (environment.py:33-43), initial
     recurrent state (models.py:148-159) and the per-step action sample
-    (agent.py:53-55).  ``actions=None`` samples with torch.multinomial."""
+    (agent.py:53-55).  ``actions=None`` samples with torch.multinomial.  Runs in the dtype of ``img``
+    (fp64 parameters, image and state give an fp64 reference); ``record`` keeps the per-step values
+    in ``Rollout.steps``."""
     sizes = list(img.shape[2:])
     gather = observation_masked if faithful_gather else observation
     table = torch.tensor(cfg.actions, dtype=torch.long, device=img.device)
     na, nb = pos0.shape[:2]
     pos = pos0.clone()
     hid = tuple(hidden0)
-    msg = torch.zeros(na, nb, cfg.n_m, device=img.device)
+    msg = torch.zeros(na, nb, cfg.n_m, dtype=img.dtype, device=img.device)
     obs = gather(img, pos, cfg.f)
     patches = [obs]
     preds_l, logp_l, val_l, pos_l, prob_l, act_l = [], [], [], [], [], []
+    steps = [] if record else None
     for t in range(nb_step):
-        npos = normalized_positions(pos, sizes)
-        probs, values, preds, msg, hid = step_forward(p, cfg, obs, msg, npos, hid)
+        npos = normalized_positions(pos, sizes, img.dtype)
+        rec = {} if record else None
+        probs, values, preds, msg, hid = step_forward(p, cfg, obs, msg, npos, hid, rec)
+        if record:
+            rec.update(h=hid[0], c=hid[1], h_caret=hid[2], c_caret=hid[3], msg=msg)
+            steps.append(rec)
         if actions is None:
             a = torch.multinomial(probs.flatten(0, 1), 1, True, generator=generator).view(na, nb)
         else:
@@ -290,6 +306,7 @@ def rollout(
         patches,
         torch.stack(act_l),
         hid,
+        steps,
     )
 
 
@@ -308,7 +325,7 @@ def classification_rewards(step_preds: torch.Tensor, targets: torch.Tensor) -> t
 def discounted_returns(rewards: torch.Tensor, gamma: float) -> torch.Tensor:
     """functions.py:35-51: flip-cumsum-flip of r*gamma^t, divided by gamma^t."""
     T = rewards.shape[0]
-    g = (gamma ** torch.arange(T, dtype=torch.float32, device=rewards.device)).view(T, *([1] * (rewards.dim() - 1)))
+    g = (gamma ** torch.arange(T, dtype=rewards.dtype, device=rewards.device)).view(T, *([1] * (rewards.dim() - 1)))
     return (rewards * g).flip(0).cumsum(0).flip(0) / g
 
 
