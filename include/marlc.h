@@ -187,6 +187,16 @@ int marlc_loss_phase_b(marlc_engine* e, void* stream);
  * (zeroed first unless accumulate != 0). img must be the forward's batch. */
 int marlc_episode_backward(marlc_engine* e, const float* img, int accumulate, void* stream);
 
+/* Backward of marlc_model_step on a T = 1 engine (the step-wise API in training).  patch / msg / npos /
+ * hidden are the inputs that were given to marlc_model_step; the step is re-run from them first (the
+ * workspace is shared by every step-wise call of the geometry).  d_out[8], each nullable (= zero):
+ * gradients on probs, values, preds, msg', h', c', h^', c^'.  d_in[5], each nullable (= not wanted):
+ * receive the gradients on msg, h, c, h^, c^.  grads: marlc_engine_param_floats floats, overwritten with
+ * the parameter gradients (the engine's bound grads buffer is left untouched). */
+int marlc_model_step_backward(marlc_engine* e, const float* patch, const float* msg, const float* npos,
+                              const float* const* hidden, const float* const* d_out, float* const* d_in,
+                              float* grads, void* stream);
+
 /* optim.step(), trainer.py:33,116: torch.optim.Adam semantics (no weight decay,
  * no amsgrad) over the flat bucket; g is multiplied by grad_scale first (1/world
  * under data parallelism).  `step` is a device int64 counter, incremented here. */

@@ -941,7 +941,7 @@ __global__ void __launch_bounds__(CT) bwd_pre_kernel(const BwdPreKernelArgs ka) 
     float* dhx = S.bufC;  // [RB][mw] encoder contribution to dh (belief cell only)
     float* W3s = S.wres;             // encode_msg.3 weight [n_m][n1]
     float* W0s = W3s + n_m * n1;     // encode_msg.0 weight [n1][nb]
-    const bool enc = a.dcoll != nullptr;
+    const bool enc = a.dcoll != nullptr || a.dmsg != nullptr;
     CHAIN_TRACE_DECL();
     if (ka.trig) pdl_trigger();  // sweep chain: the input-gradient GEMM's CTAs may set up while this kernel runs (common.cuh)
     pdl_wait();     // at entry: the operand loads must be queued AHEAD of the weight copies (see below)
@@ -971,7 +971,8 @@ __global__ void __launch_bounds__(CT) bwd_pre_kernel(const BwdPreKernelArgs ka) 
             if (tid < RB * n_m) {
                 const int r = tid / n_m, j = tid - r * n_m;
                 if (r < rows_valid) {
-                    meanv = other_agents_mean(a.dcoll, row0 + r, j, a.Na, a.Nb, n_m);
+                    meanv = a.dmsg ? a.dmsg[(long)(row0 + r) * n_m + j]
+                                   : other_agents_mean(a.dcoll, row0 + r, j, a.Na, a.Nb, n_m);
                     y2v = a.enc_y2[(long)(row0 + r) * n_m + j];
                 }
             }
@@ -1036,11 +1037,13 @@ __global__ void __launch_bounds__(CT) bwd_pre_kernel(const BwdPreKernelArgs ka) 
                   a.c_new[1], nullptr, 0, a.dgates[1], a.dgates_lo[1], a.dc_prev[1]);
     CHAIN_TRACE();  // 1: action cell
     if (enc) {
-        // gradient of the message produced at step t = adjoint mean of dcoll(t+1); encoder block 3 backward
+        // gradient of the message produced at step t = adjoint mean of dcoll(t+1) (or dmsg); encoder block 3 backward
         for (int e = threadIdx.x; e < RB * n_m; e += CT) {
             const int r = e / n_m, j = e % n_m;
             const bool ok = r < rows_valid;
-            S.bufA[r * mw + j] = ok ? other_agents_mean(a.dcoll, row0 + r, j, a.Na, a.Nb, n_m) : 0.f;
+            S.bufA[r * mw + j] = !ok ? 0.f
+                                 : a.dmsg ? a.dmsg[(long)(row0 + r) * n_m + j]
+                                          : other_agents_mean(a.dcoll, row0 + r, j, a.Na, a.Nb, n_m);
             S.bufB[r * mw + j] = ok ? a.enc_y2[(long)(row0 + r) * n_m + j] : 0.f;
         }
         __syncthreads();

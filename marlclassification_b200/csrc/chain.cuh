@@ -61,6 +61,8 @@ int step_post(const StepPostArgs& a, cudaStream_t s);
 //      + point-wise backward of both LSTM cells
 struct BwdPreArgs {
     const float* dcoll;   // [M,n_m] from step t+1's decoder backward (nullptr at t = T-1)
+    const float* dmsg = nullptr;  // [M,n_m] gradient of the emitted message itself (a stand-alone step's d msg');
+                                  // when set, used instead of the adjoint mean of dcoll
     ChainLin e0, e3;      // encode_msg blocks (with gradient pointers)
     const float* enc_y1;  // saved forward values of step t
     const float* enc_y2;

@@ -72,32 +72,33 @@ int cnn_weights_transpose(const CnnDesc& d, float* const* wT, cudaStream_t s) {
 // ---------------------------------------------------------------------------
 struct CnnBwdArgs {
     CnnDesc d;
-    const float* img;
-    const int* pos_hist;
+    CnnWindows win;
     const float* y_save[MAX_CNN_LAYERS];
     const float* dOut;
     long lddo;
     CnnBwdBuffers buf;
     int offA[MAX_CNN_LAYERS], offY[MAX_CNN_LAYERS], offStat[MAX_CNN_LAYERS];
     int offD0, offD1, offW, wbuf;
-    int B, H, W, M, P, p0;
+    int P, p0;
 };
 
+template <bool PATCH>
 __global__ void __launch_bounds__(256) cnn_bwd_kernel(const CnnBwdArgs a) {
     extern __shared__ float sm[];
     const CnnDesc& d = a.d;
-    const int p = a.p0 + blockIdx.x, m = p % a.M, b = m % a.B;
+    const int p = a.p0 + blockIdx.x;
     const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = nt >> 5;
     const int f = d.f, ff = f * f;
 
     // ---- A_0: the input window
     {
-        const int py = a.pos_hist[2 * (long)p], px = a.pos_hist[2 * (long)p + 1];
-        const float* src = a.img + (long)b * d.img_c * a.H * a.W;
+        long chan;
+        int row;
+        const float* src = cnn_window<PATCH>(a.win, p, chan, row);
         float* A0 = sm + a.offA[0];
         for (int e = tid; e < d.cin[0] * ff; e += nt) {
             const int c = e / ff, i = (e / f) % f, j = e % f;
-            A0[e] = __ldg(src + ((long)c * a.H + py + i) * a.W + px + j);
+            A0[e] = __ldg(src + c * chan + (long)i * row + j);
         }
     }
     // ---- Y_l, group statistics, A_{l+1} = SiLU(GN(Y_l))
@@ -247,13 +248,13 @@ __global__ void __launch_bounds__(256) cnn_bwd_kernel(const CnnBwdArgs a) {
     }
 }
 
-int cnn_bwd(const CnnDesc& d, const float* img, const int* pos_hist, int B, int H, int W, int M, int p0, int P,
-            const float* const* y_save, const float* dOut, long lddo, const CnnBwdBuffers& buf, cudaStream_t s) {
+int cnn_bwd(const CnnDesc& d, const CnnWindows& win, int p0, int P, const float* const* y_save, const float* dOut,
+            long lddo, const CnnBwdBuffers& buf, cudaStream_t s) {
     if (P <= 0) return 0;
     CnnBwdArgs a;
     a.p0 = p0;
-    a.d = d; a.img = img; a.pos_hist = pos_hist; a.dOut = dOut; a.lddo = lddo; a.buf = buf;
-    a.B = B; a.H = H; a.W = W; a.M = M; a.P = P;
+    a.d = d; a.win = win; a.dOut = dOut; a.lddo = lddo; a.buf = buf;
+    a.P = P;
     int off = 0, mx = 0;
     for (int l = 0; l < d.L; ++l) {
         a.y_save[l] = y_save[l];
@@ -275,10 +276,12 @@ int cnn_bwd(const CnnDesc& d, const float* img, const int* pos_hist, int B, int 
     MARLC_CHECK(smem <= 200 * 1024, "cnn_bwd: window too large for shared memory (%zu B)", smem);
     static size_t attr_b = 0;
     if (smem > 48 * 1024 && smem > attr_b) {
-        MARLC_CUDA(cudaFuncSetAttribute(cnn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        MARLC_CUDA(cudaFuncSetAttribute(cnn_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        MARLC_CUDA(cudaFuncSetAttribute(cnn_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_b = smem;
     }
-    cnn_bwd_kernel<<<P, 256, smem, s>>>(a);
+    if (win.patch) cnn_bwd_kernel<true><<<P, 256, smem, s>>>(a);
+    else cnn_bwd_kernel<false><<<P, 256, smem, s>>>(a);
     MARLC_LAUNCH_CHECK();
     return 0;
 }

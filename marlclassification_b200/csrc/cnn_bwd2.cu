@@ -217,39 +217,43 @@ int cnn_bwd_layer(const CnnBwdLayerArgs& a, cudaStream_t s) {
     return 0;
 }
 
-// im2col of the gathered input windows (operand of the first layer's weight gradient):
-// col[(p*npos + o), ci*9 + ky*3 + kx] = img[b, ci, py + 2oy-1+ky, px + 2ox-1+kx] (0 outside the window)
+// im2col of the input windows (operand of the first layer's weight gradient):
+// col[(p*npos + o), ci*9 + ky*3 + kx] = window_p[ci, 2oy-1+ky, 2ox-1+kx] (0 outside the window)
 // Rows are padded with zeros to kkp = round_up(cin*9, 4) floats so that the matrix is a TMA-addressable
 // (16-byte row pitch) operand of the tensor-core weight-gradient GEMM: the 27-float rows of an RGB
 // first layer otherwise sent that product to the FFMA kernel (470 us at 65 536 windows).
-template <bool FAST>
-__global__ void __launch_bounds__(256) cnn_im2col_input_kernel(const float* __restrict__ img,
-                                                               const int* __restrict__ pos_hist, float* __restrict__ col,
-                                                               int P, int M, int B, int img_c, int cin, int H, int W,
-                                                               int f, int ho, FastDiv d_kk, FastDiv d_ho) {
+template <bool FAST, bool PATCH>
+__global__ void __launch_bounds__(256) cnn_im2col_input_kernel(const CnnWindows win, float* __restrict__ col, int P,
+                                                               int cin, int ho, FastDiv d_kk, FastDiv d_ho) {
     const int lane = threadIdx.x & 31;
     const int p = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (p >= P) return;
-    const int b = (p % M) % B, py = pos_hist[2 * (long)p], px = pos_hist[2 * (long)p + 1];
-    const float* src = img + (long)b * img_c * H * W;
-    const int kk = cin * 9, kkp = (kk + 3) & ~3, npos = ho * ho;
+    long chan;
+    int row;
+    const float* src = cnn_window<PATCH>(win, p, chan, row);
+    const int f = win.f, kk = cin * 9, kkp = (kk + 3) & ~3, npos = ho * ho;
     float* cg = col + (long)p * npos * kkp;
     for (int e = lane; e < npos * kkp; e += 32) {
         const int o = MARLC_DIV(e, d_kk, kkp), r = e - o * kkp, c = r / 9, q = r - c * 9, ky = q / 3, kx = q - ky * 3;
         const int oy = MARLC_DIV(o, d_ho, ho);
         const int iy = 2 * oy - 1 + ky, ix = 2 * (o - oy * ho) - 1 + kx;
-        cg[e] = (r < kk && iy >= 0 && iy < f && ix >= 0 && ix < f) ? __ldg(src + ((long)c * H + py + iy) * W + px + ix) : 0.f;
+        cg[e] = (r < kk && iy >= 0 && iy < f && ix >= 0 && ix < f) ? __ldg(src + c * chan + (long)iy * row + ix) : 0.f;
     }
 }
 
-int cnn_im2col_input(const float* img, const int* pos_hist, float* col, int P, int M, int B, int img_c, int cin, int H,
-                     int W, int f, int ho, cudaStream_t s) {
+int cnn_im2col_input(const CnnWindows& win, float* col, int P, int cin, int ho, cudaStream_t s) {
     if (P <= 0) return 0;
     const int kkp = (cin * 9 + 3) & ~3;
     const FastDiv d_kk((unsigned)kkp), d_ho((unsigned)ho);
     const bool fast = FastDiv::exact_up_to((long long)ho * ho * kkp, kkp) && !cnn_bwd_use_div();
-    if (fast) cnn_im2col_input_kernel<true><<<(P * 32 + 255) / 256, 256, 0, s>>>(img, pos_hist, col, P, M, B, img_c, cin, H, W, f, ho, d_kk, d_ho);
-    else cnn_im2col_input_kernel<false><<<(P * 32 + 255) / 256, 256, 0, s>>>(img, pos_hist, col, P, M, B, img_c, cin, H, W, f, ho, d_kk, d_ho);
+    const unsigned grid = (P * 32 + 255) / 256;
+    if (win.patch) {
+        if (fast) cnn_im2col_input_kernel<true, true><<<grid, 256, 0, s>>>(win, col, P, cin, ho, d_kk, d_ho);
+        else cnn_im2col_input_kernel<false, true><<<grid, 256, 0, s>>>(win, col, P, cin, ho, d_kk, d_ho);
+    } else {
+        if (fast) cnn_im2col_input_kernel<true, false><<<grid, 256, 0, s>>>(win, col, P, cin, ho, d_kk, d_ho);
+        else cnn_im2col_input_kernel<false, false><<<grid, 256, 0, s>>>(win, col, P, cin, ho, d_kk, d_ho);
+    }
     MARLC_LAUNCH_CHECK();
     return 0;
 }

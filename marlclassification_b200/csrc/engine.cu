@@ -887,13 +887,8 @@ extern "C" int marlc_episode_forward(marlc_engine* e, const float* img, const in
 // ModelsWrapper.forward, models.py:78-138: one step on caller-provided tensors.
 // Outputs land in workspace slot 0/1: probs[0:M], step_values[0:M], step_preds[0:M],
 // msg[1], H[1], Cb[1], Hc[1], Cc[1].
-extern "C" int marlc_model_step(marlc_engine* e, const float* patch, const float* msg, const float* npos,
-                                const float* const* hidden, void* stream) {
-    MARLC_CHECK(e && e->ws, "engine not bound");
-    MARLC_CHECK(patch && msg && npos && hidden && hidden[0] && hidden[1] && hidden[2] && hidden[3],
-                "model_step: null input");
-    cudaStream_t s = (cudaStream_t)stream;
-    const int start = g_launch_count;
+static int model_step_fwd(marlc_engine* e, const float* patch, const float* msg, const float* npos,
+                          const float* const* hidden, cudaStream_t s) {
     MARLC_TRY(refresh_lo(e, nullptr, nullptr, s));
     if (e->cfg.use_chains && e->cfg.use_tc) {
         MARLC_CUDA(cudaMemsetAsync(e->buf("enc_y1"), 0, sizeof(float) * (size_t)e->M * 2 * e->cfg.n_m, s));
@@ -904,6 +899,15 @@ extern "C" int marlc_model_step(marlc_engine* e, const float* patch, const float
     // (only probs are read back by ModelsWrapper.forward)
     MARLC_TRY(step_act(e, 0, e->buf<int64_t>("zero_act"), s));
     MARLC_TRY(value_pred_heads(e, e->M, s));
+    return 0;
+}
+extern "C" int marlc_model_step(marlc_engine* e, const float* patch, const float* msg, const float* npos,
+                                const float* const* hidden, void* stream) {
+    MARLC_CHECK(e && e->ws, "engine not bound");
+    MARLC_CHECK(patch && msg && npos && hidden && hidden[0] && hidden[1] && hidden[2] && hidden[3],
+                "model_step: null input");
+    const int start = g_launch_count;
+    MARLC_TRY(model_step_fwd(e, patch, msg, npos, hidden, (cudaStream_t)stream));
     e->last_launches = g_launch_count - start;
     return 0;
 }
@@ -991,14 +995,27 @@ static int head_bwd_params(marlc_engine* e, const std::string& name, const float
     return G_tn(e, Y, nl, state, n_state, e->grd(name + ".0.weight"), n_state, TM, nl, n_state, s);
 }
 
-extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int accumulate, void* stream) {
+// The two ends of the BPTT sweep when it serves one stand-alone step (marlc_model_step_backward, T = 1) instead
+// of an episode.  Outer end: gradients arriving on the step's outputs, each nullable (= zero), in the order
+// probs, values, preds, msg', h', c', h^', c^'.  Inner end: gradients leaving through its inputs msg, h, c, h^,
+// c^, each nullable (= not wanted).  The feature-extractor backward reads the caller's windows.
+struct StepEnds {
+    const float* patch;
+    const float* const* d_out;
+    float* const* d_in;
+};
+
+// se == nullptr: the episode's BPTT (marlc_episode_backward); otherwise one step with the ends above
+static int episode_backward(marlc_engine* e, const float* img, int accumulate, const StepEnds* se, cudaStream_t s) {
     MARLC_CHECK(e && e->ws && e->G, "backward: engine not bound (need a grads buffer)");
-    MARLC_CHECK(img, "null image batch");
     NvtxRange nvtx_bwd("marlc/backward");
-    cudaStream_t s = (cudaStream_t)stream;
     const marlc_config& c = e->cfg;
     const int M = e->M, T = c.T, TM = e->TM, Kin = e->Kin, F = e->F;
     const int start = g_launch_count;
+    const float* d_probs = se ? se->d_out[0] : nullptr;
+    const float* d_msg_out = se ? se->d_out[3] : nullptr;  // seeds the encoder backward of the last step
+    const bool want_dh0 = se && (se->d_in[1] || se->d_in[3]);  // input gradients of step 0's recurrent states
+    const bool want_dmsg0 = se && se->d_in[0];                 // ... and of its message
     if (!accumulate) MARLC_CUDA(cudaMemsetAsync(e->G, 0, sizeof(float) * (size_t)e->param_floats, s));
 
     float* H = e->buf("H");
@@ -1023,7 +1040,7 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
         MARLC_TRY(G_nn(e, Yq, c.nl_b, e->prm("predict.0.weight"), c.n_b, e->buf("dH_heads"), c.n_b, TM, c.nl_b, c.n_b, 0, sp));
         MARLC_TRY(head_bwd_state(e, "critic", e->buf("d_values"), 1, e->buf("cri_y1"), c.nl_a, e->buf("scratchS3"), Yc, sc));
         MARLC_TRY(policy_logit_grad(e->buf("d_logp"), e->buf("probs"), e->buf<int>("act"), e->buf("d_pol_logits"), TM,
-                                    c.n_actions, s));
+                                    c.n_actions, s, d_probs));
         MARLC_TRY(head_bwd_state(e, "policy", e->buf("d_pol_logits"), c.n_actions, e->buf("pol_y1"), c.nl_a,
                                  e->buf("scratchS"), Yp, s));
         MARLC_TRY(e->chain(sc, s));
@@ -1055,7 +1072,7 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
         MARLC_TRY(head_bwd(e, "predict", e->buf("d_preds"), c.nb_class, e->buf("prd_s1"), e->buf("prd_y1"),
                            H + (size_t)M * c.n_b, c.n_b, c.nl_b, e->buf("dH_heads"), 0, s, 1));
         MARLC_TRY(policy_logit_grad(e->buf("d_logp"), e->buf("probs"), e->buf<int>("act"), e->buf("d_pol_logits"), TM,
-                                    c.n_actions, s));
+                                    c.n_actions, s, d_probs));
         MARLC_TRY(head_bwd(e, "policy", e->buf("d_pol_logits"), c.n_actions, e->buf("pol_s1"), e->buf("pol_y1"),
                            Hc + (size_t)M * c.n_a, c.n_a, c.nl_a, e->buf("dHc_heads"), 0, s));
         MARLC_TRY(head_bwd(e, "critic", e->buf("d_values"), 1, e->buf("cri_s1"), e->buf("cri_y1"), Hc + (size_t)M * c.n_a,
@@ -1096,7 +1113,7 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
             MARLC_TRY(colsum_add2(dga, 4 * c.n_a, e->grd(pa + "bias_ih"), e->grd(pa + "bias_hh"), R, 4 * c.n_a, sL));
         }
         {
-            const int Re = (std::min(t1, T - 1) - t0) * M;  // the last message is never consumed
+            const int Re = (std::min(t1, d_msg_out ? T : T - 1) - t0) * M;  // an episode's last message is never consumed
             const TnProblem enc[2] = {
                 {e->buf("d_enc_y2") + r0 * c.n_m, c.n_m, e->buf("enc_s1") + r0 * 2 * c.n_m, 2L * c.n_m,
                  e->grd("encode_msg.3.weight"), 2L * c.n_m, Re, c.n_m, 2 * c.n_m},
@@ -1118,6 +1135,8 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
         // feature extractor: layer-wise, batched over the chunk's windows (cnn_bwd2.cu); every conv product
         // (input gradient dCol_l = dY_l W_l, weight gradient dW_l = dY_l^T col_l) is a tensor-core GEMM
         const CnnDesc& d = e->cnn;
+        CnnWindows win{img, e->buf<int>("pos_hist") + r0 * 2, se ? se->patch : nullptr, M, c.nb, c.C, c.H, c.W, c.f};
+        if (win.patch) win.patch += r0 * c.C * c.f * c.f;
         const float* ysave[MAX_CNN_LAYERS];
         CnnBwdBuffers bb;
         float* dcol[MAX_CNN_LAYERS] = {nullptr};
@@ -1136,7 +1155,7 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
                         R * npos, co, kk, st);
         };
         if (!par) {  // unfused reference path: one whole-episode call of the per-window kernel
-            MARLC_TRY(cnn_bwd(e->cnn, img, e->buf<int>("pos_hist"), c.nb, c.H, c.W, M, 0, TM, ysave, dU, Kin, bb, s0));
+            MARLC_TRY(cnn_bwd(e->cnn, win, 0, TM, ysave, dU, Kin, bb, s0));
             for (int l = 0; l < e->L; ++l) {
                 const int npos = d.hout[l] * d.hout[l], co = d.cout[l];
                 const std::string cw = CNN_PREFIX + std::to_string(3 * l), gn = CNN_PREFIX + std::to_string(3 * l + 1);
@@ -1151,8 +1170,7 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
         // of the input windows is independent of it (stream s1), and the weight-gradient GEMMs wait at
         // the end and fan out over the three streams.  GroupNorm-affine and conv-bias gradients are
         // accumulated inside the layer kernel.
-        MARLC_TRY(cnn_im2col_input(img, e->buf<int>("pos_hist") + r0 * 2, bb.col[0], R, M, c.nb, c.C, d.cin[0], c.H, c.W,
-                                   c.f, d.hout[0], s1));
+        MARLC_TRY(cnn_im2col_input(win, bb.col[0], R, d.cin[0], d.hout[0], s1));
         for (int l = e->L - 1; l >= 0; --l) {
             CnnBwdLayerArgs la;
             memset(&la, 0, sizeof(la));
@@ -1192,10 +1210,17 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
     float* dcc[2] = {e->buf("dcc0"), e->buf("dcc1")};
     float* dmsg = e->buf("dmsg");
     float* tmpS = e->buf("tmpS");
-    MARLC_CUDA(cudaMemsetAsync(dh, 0, sizeof(float) * (size_t)M * c.n_b, s));
-    MARLC_CUDA(cudaMemsetAsync(dhc, 0, sizeof(float) * (size_t)M * c.n_a, s));
-    MARLC_CUDA(cudaMemsetAsync(dc[0], 0, sizeof(float) * (size_t)M * c.n_b, s));
-    MARLC_CUDA(cudaMemsetAsync(dcc[0], 0, sizeof(float) * (size_t)M * c.n_a, s));
+    // carries into the last step: zero for an episode, d h' / d c' / d h^' / d c^' for a stand-alone step
+    auto seed = [&](float* dst, int k, int n) -> int {
+        const float* src = se ? se->d_out[k] : nullptr;
+        if (src) MARLC_CUDA(cudaMemcpyAsync(dst, src, sizeof(float) * (size_t)M * n, cudaMemcpyDeviceToDevice, s));
+        else MARLC_CUDA(cudaMemsetAsync(dst, 0, sizeof(float) * (size_t)M * n, s));
+        return 0;
+    };
+    MARLC_TRY(seed(dh, 4, c.n_b));
+    MARLC_TRY(seed(dhc, 6, c.n_a));
+    MARLC_TRY(seed(dc[0], 5, c.n_b));
+    MARLC_TRY(seed(dcc[0], 7, c.n_a));
     int cur = 0;
     const bool chain_sweep = sweep_chained(e);  // fused chain kernels, or one kernel per op from 4096 rows on
     if (chain_sweep) {
@@ -1220,19 +1245,20 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
             // fused: adjoint mean + encoder backward + dh accumulation + both LSTM cells' point-wise backward
             BwdPreArgs bp;
             memset(&bp, 0, sizeof(bp));
-            bp.dcoll = (t < T - 1) ? dcoll : nullptr;  // the last message is never consumed
+            bp.dcoll = (t < T - 1) ? dcoll : nullptr;  // an episode's last message is never consumed
+            bp.dmsg = (t == T - 1) ? d_msg_out : nullptr;
             bp.e0 = chain_lin(e, "encode_msg", 0, c.n_b, 2 * c.n_m, true);
             bp.e3 = chain_lin(e, "encode_msg", 3, 2 * c.n_m, c.n_m, true);
             bp.enc_y1 = e->buf("enc_y1") + (size_t)t * M * 2 * c.n_m;
             bp.enc_y2 = e->buf("enc_y2") + (size_t)t * M * c.n_m;
             bp.d_enc_y1 = e->buf("d_enc_y1") + (size_t)t * M * 2 * c.n_m;
             bp.d_enc_y2 = e->buf("d_enc_y2") + (size_t)t * M * c.n_m;
-            bp.dh_carry[0] = (t < T - 1) ? dh_hist + (size_t)(t + 1) * M * c.n_b : nullptr;
-            bp.dh_carry[1] = (t < T - 1) ? dhc_hist + (size_t)(t + 1) * M * c.n_a : nullptr;
+            bp.dh_carry[0] = (t < T - 1) ? dh_hist + (size_t)(t + 1) * M * c.n_b : se ? dh : nullptr;
+            bp.dh_carry[1] = (t < T - 1) ? dhc_hist + (size_t)(t + 1) * M * c.n_a : se ? dhc : nullptr;
             bp.dh_heads[0] = e->buf("dH_heads") + (size_t)t * M * c.n_b;
             bp.dh_heads[1] = e->buf("dHc_heads") + (size_t)t * M * c.n_a;
-            bp.dc_next[0] = (t < T - 1) ? dc[cur] : nullptr;
-            bp.dc_next[1] = (t < T - 1) ? dcc[cur] : nullptr;
+            bp.dc_next[0] = (t < T - 1 || se) ? dc[cur] : nullptr;
+            bp.dc_next[1] = (t < T - 1 || se) ? dcc[cur] : nullptr;
             bp.gates[0] = e->buf("gates_b") + (size_t)t * M * 4 * c.n_b;
             bp.gates[1] = e->buf("gates_a") + (size_t)t * M * 4 * c.n_a;
             bp.c_prev[0] = Cb + (size_t)t * M * c.n_b;
@@ -1272,7 +1298,7 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
                 ok = ok && tc_operand_ok(g[0].A2) && tc_operand_ok(g[0].B2);
                 if (ok) {
                     PdlScope pdl(pdl_edge(PDL_DX), pdl_trig_mode(1));
-                    MARLC_TRY(tc_gemm_group(g, t > 0 ? 3 : 1, sw));  // at t == 0 nothing consumes dh / dh^
+                    MARLC_TRY(tc_gemm_group(g, t > 0 || want_dh0 ? 3 : 1, sw));  // at t == 0 only a step's caller consumes dh / dh^
                     tc_dx = true;
                 }
             }
@@ -1316,7 +1342,7 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
             bq.dec_y2 = e->buf("dec_y2") + (size_t)t * M * c.n_m_o;
             bq.d_dec_y1 = e->buf("d_dec_y1") + (size_t)t * M * 2 * c.n_m;
             bq.d_dec_y2 = e->buf("d_dec_y2") + (size_t)t * M * c.n_m_o;
-            bq.dcoll = t > 0 ? dcoll : nullptr;
+            bq.dcoll = (t > 0 || want_dmsg0) ? dcoll : nullptr;
             bq.M = M; bq.n_m = c.n_m; bq.n_m_o = c.n_m_o;
             {
                 PdlScope pdl(pdl_edge(PDL_BWD_POST), pdl_trig_mode(1));
@@ -1336,12 +1362,13 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
         MARLC_TRY(e->chain(sw, s));
     } else
     for (int t = T - 1; t >= 0; --t) {
-        if (t < T - 1) {
-            // message produced at step t was consumed at t+1: encoder backward (models.py:114-116)
+        if (t < T - 1 || d_msg_out) {
+            // message produced at step t was consumed at t+1 (or has a gradient of its own): encoder backward
+            // (models.py:114-116)
             float* dy2 = e->buf("d_enc_y2") + (size_t)t * M * c.n_m;
             float* dy1 = e->buf("d_enc_y1") + (size_t)t * M * 2 * c.n_m;
-            MARLC_TRY(block_bwd_norm(e, "encode_msg", 3, dmsg, c.n_m, e->buf("enc_y2") + (size_t)t * M * c.n_m, M,
-                                     c.n_m, dy2, s));
+            MARLC_TRY(block_bwd_norm(e, "encode_msg", 3, t < T - 1 ? dmsg : d_msg_out, c.n_m,
+                                     e->buf("enc_y2") + (size_t)t * M * c.n_m, M, c.n_m, dy2, s));
             MARLC_TRY(G_nn(e, dy2, c.n_m, e->prm("encode_msg.3.weight"), 2 * c.n_m, tmpS, 2 * c.n_m, M, c.n_m,
                               2 * c.n_m, 0, s));
             MARLC_TRY(block_bwd_norm(e, "encode_msg", 0, tmpS, 2 * c.n_m,
@@ -1418,11 +1445,24 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
                           2 * c.n_m, 0, s));
         MARLC_TRY(block_bwd_norm(e, "decode_msg", 0, tmpS, 2 * c.n_m, e->buf("dec_y1") + (size_t)t * M * 2 * c.n_m, M,
                                  2 * c.n_m, ddy1, s));
-        if (t > 0) {
+        if (t > 0 || want_dmsg0) {
             MARLC_TRY(G_nn(e, ddy1, 2 * c.n_m, e->prm("decode_msg.0.weight"), c.n_m, e->buf("dcoll"), c.n_m, M,
                               2 * c.n_m, c.n_m, 0, s));
-            MARLC_TRY(msg_mean(e->buf("dcoll"), dmsg, c.na, c.nb, c.n_m, s));  // symmetric operator = own adjoint
+            if (t > 0) MARLC_TRY(msg_mean(e->buf("dcoll"), dmsg, c.na, c.nb, c.n_m, s));  // symmetric operator = own adjoint
         }
+    }
+    if (se) {  // inner end: the gradients that leave through the step's inputs
+        auto emit = [&](int k, const float* src, int n) -> int {
+            if (se->d_in[k])
+                MARLC_CUDA(cudaMemcpyAsync(se->d_in[k], src, sizeof(float) * (size_t)M * n, cudaMemcpyDeviceToDevice, s));
+            return 0;
+        };
+        MARLC_TRY(emit(1, chain_sweep ? e->buf("dh_hist") : dh, c.n_b));
+        MARLC_TRY(emit(2, dc[cur], c.n_b));
+        MARLC_TRY(emit(3, chain_sweep ? e->buf("dhc_hist") : dhc, c.n_a));
+        MARLC_TRY(emit(4, dcc[cur], c.n_a));
+        // d msg = adjoint message mean of the decoder's input gradient (zero with one agent, message.py:12-17)
+        if (want_dmsg0) MARLC_TRY(msg_mean(e->buf("dcoll"), se->d_in[0], c.na, c.nb, c.n_m, s));
     }
 
     if (e->debug_stop == 2 || e->debug_stop == 21 || e->debug_stop == 22) {
@@ -1437,6 +1477,56 @@ extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int acc
         MARLC_TRY(batched(0, T, s, e->side[1], e->side[0]));
     }
     if (par) MARLC_TRY(join_sides());
+    e->last_launches = g_launch_count - start;
+    return 0;
+}
+
+extern "C" int marlc_episode_backward(marlc_engine* e, const float* img, int accumulate, void* stream) {
+    MARLC_CHECK(img, "null image batch");
+    return episode_backward(e, img, accumulate, nullptr, (cudaStream_t)stream);
+}
+
+// The backward of marlc_model_step.  Every step-wise call of one geometry shares this T = 1 engine's workspace,
+// so the activations of the forward being differentiated are gone by now: the step is re-run from its inputs
+// first.  Split-K reduce-adds are unordered, so the recomputed activations may differ from the forward's in the
+// last bits.  The inputs are then copied into slot 0 of the state histories, where every read of step 0's
+// inputs in the sweep finds them (weight_hh gradients, c_prev, position-feature weight gradient).
+extern "C" int marlc_model_step_backward(marlc_engine* e, const float* patch, const float* msg, const float* npos,
+                                         const float* const* hidden, const float* const* d_out, float* const* d_in,
+                                         float* grads, void* stream) {
+    MARLC_CHECK(e && e->ws, "engine not bound");
+    MARLC_CHECK(e->cfg.T == 1, "model_step_backward: needs a T = 1 engine (T = %d)", e->cfg.T);
+    MARLC_CHECK(patch && msg && npos && hidden && hidden[0] && hidden[1] && hidden[2] && hidden[3],
+                "model_step_backward: null input");
+    MARLC_CHECK(d_out && d_in && grads, "model_step_backward: null gradient array / buffer");
+    NvtxRange nvtx_step_bwd("marlc/model_step_backward");
+    cudaStream_t s = (cudaStream_t)stream;
+    const marlc_config& c = e->cfg;
+    const size_t M = e->M;
+    const int start = g_launch_count;
+    MARLC_TRY(model_step_fwd(e, patch, msg, npos, hidden, s));
+    const struct { float* dst; const float* src; size_t n; } in[6] = {
+        {e->buf("H"), hidden[0], M * c.n_b}, {e->buf("Cb"), hidden[1], M * c.n_b},
+        {e->buf("Hc"), hidden[2], M * c.n_a}, {e->buf("Cc"), hidden[3], M * c.n_a},
+        {e->buf("msg"), msg, M * c.n_m}, {e->buf("npos"), npos, M * 2}};
+    for (const auto& x : in)
+        MARLC_CUDA(cudaMemcpyAsync(x.dst, x.src, sizeof(float) * x.n, cudaMemcpyDeviceToDevice, s));
+    // the heads' seeds: d values / d preds as given (zero when absent); d probs replaces d log p (kept zero)
+    const struct { float* dst; const float* src; size_t n; } head[3] = {
+        {e->buf("d_values"), d_out[1], M}, {e->buf("d_preds"), d_out[2], M * c.nb_class}, {e->buf("d_logp"), nullptr, M}};
+    for (const auto& x : head) {
+        if (x.src) MARLC_CUDA(cudaMemcpyAsync(x.dst, x.src, sizeof(float) * x.n, cudaMemcpyDeviceToDevice, s));
+        else MARLC_CUDA(cudaMemsetAsync(x.dst, 0, sizeof(float) * x.n, s));
+    }
+    // the parameter gradients go to the caller's buffer for the duration of the call
+    struct GradBase {
+        marlc_engine* e;
+        float* saved;
+        ~GradBase() { e->G = saved; }
+    } base{e, e->G};
+    e->G = grads;
+    const StepEnds se{patch, d_out, d_in};
+    MARLC_TRY(episode_backward(e, nullptr, 0, &se, s));
     e->last_launches = g_launch_count - start;
     return 0;
 }

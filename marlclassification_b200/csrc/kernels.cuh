@@ -74,11 +74,33 @@ struct CnnBwdBuffers {
     float* col[MAX_CNN_LAYERS];     // [P*hout^2, cin*9] im2col of the layer input
     float* gnpart[MAX_CNN_LAYERS];  // [P, 2*cout] per-window partial sums for dgamma | dbeta
 };
-// Backward through the CNN for windows p0 .. p0+P-1 of the T*M stack (window p uses image
-// (p % M) % B): re-gathers the input windows, recomputes the activations from y_save, writes
-// dY / col / gnpart rows of those windows.  All buffer pointers are for window 0.
-int cnn_bwd(const CnnDesc& d, const float* img, const int* pos_hist, int B, int H, int W, int M, int p0, int P,
-            const float* const* y_save, const float* dOut, long lddo, const CnnBwdBuffers& buf, cudaStream_t s);
+// Where the feature-extractor backward reads its input windows: gathered from the image batch at the
+// episode's positions (window p = image (p % M) % B at pos_hist[p]), or, when `patch` is set, the caller's
+// [P, img_c, f, f] windows of a stand-alone step (only the first cin[0] channels are read either way).
+struct CnnWindows {
+    const float* img;
+    const int* pos_hist;
+    const float* patch;
+    int M, B, img_c, H, W, f;
+};
+// Pixel (c, y, x) of window p is origin[c * chan + y * row + x].
+template <bool PATCH>
+__device__ __forceinline__ const float* cnn_window(const CnnWindows& w, int p, long& chan, int& row) {
+    if (PATCH) {
+        chan = (long)w.f * w.f;
+        row = w.f;
+        return w.patch + (long)p * w.img_c * chan;
+    }
+    chan = (long)w.H * w.W;
+    row = w.W;
+    return w.img + (long)((p % w.M) % w.B) * w.img_c * chan + (long)w.pos_hist[2 * (long)p] * w.W +
+           w.pos_hist[2 * (long)p + 1];
+}
+// Backward through the CNN for windows p0 .. p0+P-1 of the T*M stack: reads the input windows,
+// recomputes the activations from y_save, writes dY / col / gnpart rows of those windows.  All
+// buffer pointers are for window 0.
+int cnn_bwd(const CnnDesc& d, const CnnWindows& win, int p0, int P, const float* const* y_save, const float* dOut,
+            long lddo, const CnnBwdBuffers& buf, cudaStream_t s);
 
 int cnn_weights_transpose(const CnnDesc& d, float* const* wT, cudaStream_t s);
 
@@ -102,8 +124,7 @@ struct CnnBwdLayerArgs {
     float* colNext;         // out im2col of this layer's activation for layer l+1 (nullptr for the top layer)
 };
 int cnn_bwd_layer(const CnnBwdLayerArgs& a, cudaStream_t s);
-int cnn_im2col_input(const float* img, const int* pos_hist, float* col, int P, int M, int B, int img_c, int cin, int H,
-                     int W, int f, int ho, cudaStream_t s);
+int cnn_im2col_input(const CnnWindows& win, float* col, int P, int cin, int ho, cudaStream_t s);
 
 // ---- loss.cu ------------------------------------------------------------------
 struct LossArgs {
@@ -124,8 +145,9 @@ struct LossArgs {
 };
 int loss_phase_a(const LossArgs& a, cudaStream_t s);  // rewards, returns, advantages, local stats
 int loss_phase_b(const LossArgs& a, cudaStream_t s);  // standardise, loss parts, gradients
-// policy head: dlogits[r,j] = dlogp[r] * (1[j==a_r] - p[r,j])
+// policy head: dlogits[r,j] = dlogp[r] * (1[j==a_r] - p[r,j]), or, when d_probs is set (gradients on the
+// probabilities of a stand-alone step), the softmax backward dlogits[r,j] = p[r,j] (g[r,j] - sum_a p[r,a] g[r,a])
 int policy_logit_grad(const float* d_logp, const float* probs, const int* act, float* dlogits, int R, int nA,
-                      cudaStream_t s);
+                      cudaStream_t s, const float* d_probs = nullptr);
 
 }  // namespace marlc

@@ -181,19 +181,28 @@ int loss_phase_b(const LossArgs& a, cudaStream_t s) {
 }
 
 __global__ void policy_logit_grad_kernel(const float* __restrict__ d_logp, const float* __restrict__ probs,
-                                         const int* __restrict__ act, float* __restrict__ dlogits, long R, int nA) {
+                                         const int* __restrict__ act, const float* __restrict__ d_probs,
+                                         float* __restrict__ dlogits, long R, int nA) {
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= R * nA) return;
     const long r = i / nA;
     const int j = (int)(i % nA);
+    if (d_probs) {  // softmax backward; nA <= MAX_ACTIONS, so each thread forms its row's dot product
+        const float* p = probs + r * nA;
+        const float* g = d_probs + r * nA;
+        float dot = 0.f;
+        for (int a = 0; a < nA; ++a) dot = fmaf(p[a], g[a], dot);
+        dlogits[i] = p[j] * (g[j] - dot);
+        return;
+    }
     dlogits[i] = d_logp[r] * ((j == act[r] ? 1.f : 0.f) - probs[i]);
 }
 
 int policy_logit_grad(const float* d_logp, const float* probs, const int* act, float* dlogits, int R, int nA,
-                      cudaStream_t s) {
+                      cudaStream_t s, const float* d_probs) {
     long n = (long)R * nA;
     if (n <= 0) return 0;
-    policy_logit_grad_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_logp, probs, act, dlogits, R, nA);
+    policy_logit_grad_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_logp, probs, act, d_probs, dlogits, R, nA);
     MARLC_LAUNCH_CHECK();
     return 0;
 }

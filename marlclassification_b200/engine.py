@@ -212,6 +212,18 @@ class EpisodeEngine:
         _lib.check(self._L.marlc_model_step(self._h, patch.data_ptr(), msg.data_ptr(), npos.data_ptr(), hid,
                                             self._stream()))
 
+    def model_step_backward(self, patch, msg, npos, hidden, d_out, d_in, grads) -> None:
+        """``marlc_model_step_backward``: re-runs the step from its inputs, then backpropagates ``d_out``
+        (8 tensors or None) into ``d_in`` (5 tensors or None) and the flat ``grads`` buffer."""
+        self._check_model()
+        ptrs = lambda ts: (ct.c_void_p * len(ts))(*[_lib.ptr(t) for t in ts])  # noqa: E731
+        self._keep = [patch, msg, npos, *hidden, *d_out, *d_in, grads]
+        self.generation += 1
+        _lib.check(self._L.marlc_model_step_backward(self._h, patch.data_ptr(), msg.data_ptr(), npos.data_ptr(),
+                                                     ptrs(hidden), ptrs(d_out), ptrs(d_in), grads.data_ptr(),
+                                                     self._stream()))
+        self.launches["backward"] = self._L.marlc_engine_last_launches(self._h)
+
 
 def C_void_p():
     return ct.c_void_p()
@@ -302,7 +314,68 @@ class _ForwardOnly(th.autograd.Function):
         raise RuntimeError(
             "ModelsWrapper.forward / MultiAgent.act are forward-only in this build: gradients flow through "
             "EpisodeSampler.run_episode(...) (whole episode = one autograd node with hand-written BPTT) or "
-            "Trainer.train_step; wrap step-wise inference in torch.no_grad().")
+            "Trainer.train_step; wrap step-wise inference in torch.no_grad().  Set "
+            "model.differentiable_steps = True to backpropagate through the step-wise API instead.")
+
+
+def _step_outputs(eng: EpisodeEngine):
+    """probs, values, preds, msg', h', c', h^', c^' of the last marlc_model_step, copied out of the workspace."""
+    return (eng.probs[0].clone(), eng.step_values[0].clone(), eng.step_preds[0].clone(), eng.msg[1].clone(),
+            eng.H_state[1].clone(), eng.C_state[1].clone(), eng.Hc_state[1].clone(), eng.Cc_state[1].clone())
+
+
+class _StepFn(th.autograd.Function):
+    """ModelsWrapper.forward as one autograd node (``model.differentiable_steps``).  Forward = marlc_model_step;
+    backward = marlc_model_step_backward, which re-runs the step from the saved inputs (the next step-wise call
+    of the geometry overwrites the workspace, so nothing but the inputs is kept) and then runs the engine's
+    BPTT at T = 1 with the output gradients as its outer end.  Parameter gradients land in a fresh flat buffer
+    per call, handed to autograd as one view per parameter."""
+
+    @staticmethod
+    def forward(ctx, eng: EpisodeEngine, model, patch, msg, npos, h, c, hc, cc, *params):
+        eng.model_step(patch, msg, npos, [h, c, hc, cc])
+        ctx.eng, ctx.model, ctx.params = eng, model, params
+        ctx.param_generation = model.param_generation
+        ctx.save_for_backward(patch, msg, npos, h, c, hc, cc)
+        ctx.set_materialize_grads(False)  # an output nothing depends on passes nullptr: no seed, no copy
+        return _step_outputs(eng)
+
+    @staticmethod
+    def backward(ctx, *d_out):
+        eng: EpisodeEngine = ctx.eng
+        model = ctx.model
+        if model.param_generation != ctx.param_generation:
+            raise RuntimeError(
+                "ModelsWrapper.forward: a parameter was updated (optimizer step or in-place write) between this "
+                "step's forward and its backward; the step's gradients would be those of different weights.  "
+                "Call backward() before updating the parameters.")
+        patch, msg, npos, h, c, hc, cc = ctx.saved_tensors
+        d_out = [None if g is None else g.float().contiguous() for g in d_out]
+        need = ctx.needs_input_grad
+        d_in = [th.empty_like(x) if need[i] else None for i, x in ((3, msg), (5, h), (6, c), (7, hc), (8, cc))]
+        flat = model.flat_params
+        grads = th.empty_like(flat)
+        eng.model_step_backward(patch, msg, npos, (h, c, hc, cc), d_out, d_in, grads)
+        # autograd adds each parameter gradient into param.grad in place: make sure param.grad is the parameter's
+        # slot of model.flat_grads, so the bucket the fused Adam reads and param.grad stay one tensor.  After
+        # zero_grad(set_to_none=True) param.grad is None: the slot starts from zero.  A gradient held outside
+        # the bucket (e.g. the one a run_episode backward left after set_to_none) moves into the slot.
+        base, bucket = flat.data_ptr(), model.flat_grads
+        out = []
+        for i, p in enumerate(ctx.params):
+            if not need[9 + i]:
+                out.append(None)
+                continue
+            off = (p.data.data_ptr() - base) // 4
+            if p.grad is None or p.grad.untyped_storage().data_ptr() != bucket.untyped_storage().data_ptr():
+                slot = bucket[off: off + p.numel()].view(p.shape)
+                if p.grad is None:
+                    slot.zero_()
+                else:
+                    slot.copy_(p.grad)
+                p.grad = slot
+            out.append(grads[off: off + p.numel()].view(p.shape))
+        return (None, None, None, d_in[0], None, *d_in[1:], *out)
 
 
 def model_step(model, img_patch, msg_t, norm_pos, hidden):
@@ -319,14 +392,16 @@ def model_step(model, img_patch, msg_t, norm_pos, hidden):
     if f != model.feature_extractor.cnn_spec[0] or f2 != f:
         raise RuntimeError(f"img_patch window {f}x{f2} != model window {model.feature_extractor.cnn_spec[0]}")
     eng = get_engine(model, na=na, nb=nb, T=1, C=Cc, H=f + 1, W=f + 1, actions=[[0, 0]] * d["nb_action"], gamma=1.0)
+    if th.is_grad_enabled() and getattr(model, "differentiable_steps", False):
+        for t, name in ((img_patch, "img_patch"), (norm_pos, "norm_pos")):
+            if t.requires_grad:
+                raise RuntimeError(f"ModelsWrapper.forward: {name} requires grad, but the step-wise backward computes "
+                                   f"no gradient for it; pass {name}.detach()")
+        o = _StepFn.apply(eng, model, patch, msg, npos, *hid, *model.parameters())
+        return ModelOutput(*o[:4]), RecurrentOutput(*o[4:])
     eng.model_step(patch, msg, npos, hid)
-    out = ModelOutput(
-        actions_probabilities=eng.probs[0].clone(),
-        values=eng.step_values[0].clone(),
-        predictions=eng.step_preds[0].clone(),
-        messages=eng.msg[1].clone(),
-    )
-    rec = RecurrentOutput(eng.H_state[1].clone(), eng.C_state[1].clone(), eng.Hc_state[1].clone(), eng.Cc_state[1].clone())
+    o = _step_outputs(eng)
+    out, rec = ModelOutput(*o[:4]), RecurrentOutput(*o[4:])
     if th.is_grad_enabled():
         anchor = next((p for p in model.parameters() if p.requires_grad), None)
         if anchor is not None:  # same values; a backward() through them raises (see _ForwardOnly)

@@ -89,6 +89,10 @@ class ModelsWrapper(nn.Module):
         self.use_tc = True  # tensor-core GEMMs where shapes allow; False = exact fp32 FFMA everywhere
         self.precision = "tf32x3"  # "tf32x3" (error-compensated, fp32-class) | "tf32" (fastest, ~1e-3)
         self.use_chains = True  # fused per-step chain kernels; False = one kernel per op (debug / comparison)
+        # True: forward() / MultiAgent.act in grad mode carry a backward (engine.model_step); False: they are
+        # forward-only and a backward() reaching them raises
+        self.differentiable_steps = False
+        self._param_updates = 0  # parameter writes torch cannot see (the fused Adam): see param_generation
 
     # ---- reference surface ------------------------------------------------------
     @property
@@ -112,9 +116,10 @@ class ModelsWrapper(nn.Module):
     def forward(
         self, img_patch: th.Tensor, msg_t: th.Tensor, norm_pos: th.Tensor, recurrent_hidden: RecurrentOutput
     ) -> tuple[ModelOutput, RecurrentOutput]:
-        """One step of every network (models.py:78-138) on CUDA.  Forward-only:
-        training goes through EpisodeSampler.run_episode, whose outputs carry
-        the hand-written BPTT backward."""
+        """One step of every network (models.py:78-138) on CUDA.  With ``differentiable_steps`` set, the
+        outputs carry a backward to every parameter, ``msg_t`` and ``recurrent_hidden`` (not to
+        ``img_patch`` / ``norm_pos``); otherwise this is forward-only and training goes through
+        EpisodeSampler.run_episode, whose outputs carry the hand-written BPTT backward."""
         from ..engine import model_step
 
         return model_step(self, img_patch, msg_t, norm_pos, recurrent_hidden)
@@ -123,6 +128,18 @@ class ModelsWrapper(nn.Module):
     @property
     def dims(self) -> dict:
         return dict(self.__dims)
+
+    @property
+    def param_generation(self) -> int:
+        """Changes whenever a parameter is written: in place through torch, on a parameter or on the flat buffer
+        they all view (version counters), or by the fused Adam (``note_param_update``).  A step-wise backward
+        refuses to run across such a write."""
+        flat = self._flat_params._version if self._flat_params is not None else 0
+        return self._param_updates + flat + sum(p._version for p in self.parameters())
+
+    def note_param_update(self) -> None:
+        """Record a parameter write that bypasses torch (a kernel writing ``flat_params`` through its pointer)."""
+        self._param_updates += 1
 
     @property
     def feature_extractor(self) -> _Generic2dCnnModule:

@@ -31,3 +31,4 @@ class FlatAdam:
             m.flat_params.data_ptr(), m.flat_grads.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
             m.flat_params.numel(), self.lr, self.betas[0], self.betas[1], self.eps, float(grad_scale),
             self.step_count.data_ptr(), _lib.stream_ptr(m.flat_params.device)))
+        m.note_param_update()

@@ -124,6 +124,10 @@ class TrainStep:
             segs[2]()
         else:
             segs[0]()
+        if self._graphs[injected] is not None:
+            # a replay runs the fused Adam without calling FlatAdam.step(): record the parameter write here, so a
+            # step-wise backward across it refuses to run (ModelsWrapper.param_generation)
+            eng.model.note_param_update()
         return eng.loss_out
 
     def __call__(self, img: th.Tensor, y: th.Tensor, **inject) -> th.Tensor:
