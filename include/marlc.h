@@ -187,6 +187,16 @@ int marlc_loss_phase_b(marlc_engine* e, void* stream);
  * (zeroed first unless accumulate != 0). img must be the forward's batch. */
 int marlc_episode_backward(marlc_engine* e, const float* img, int accumulate, void* stream);
 
+/* Gradient on the image batch of the engine's last rollout: overwrites d_img (f32 [nb, C, H, W], every
+ * element) with d(whatever the last marlc_episode_backward was seeded with) / d img.  Only the T observations
+ * the networks consumed count; pixels no window covers and channels the feature extractor does not read are
+ * 0.  Call it after marlc_episode_backward, on the same stream and before the parameters change (the first
+ * conv layer's weights are read here).  Deterministic; neither allocates nor synchronises (capturable).
+ * Fails when there was no complete episode backward since the last marlc_episode_forward /
+ * marlc_model_step, after marlc_model_step_backward, or after a backward cut short by
+ * marlc_engine_debug_stop. */
+int marlc_episode_image_grad(marlc_engine* e, float* d_img, void* stream);
+
 /* Backward of marlc_model_step on a T = 1 engine (the step-wise API in training).  patch / msg / npos /
  * hidden are the inputs that were given to marlc_model_step; the step is re-run from them first (the
  * workspace is shared by every step-wise call of the geometry).  d_out[8], each nullable (= zero):

@@ -77,6 +77,7 @@ _SIGS = {
     "marlc_loss_phase_a": (C.c_int, [_P, _P, _P]),
     "marlc_loss_phase_b": (C.c_int, [_P, _P]),
     "marlc_episode_backward": (C.c_int, [_P, _P, C.c_int, _P]),
+    "marlc_episode_image_grad": (C.c_int, [_P, _P, _P]),
     "marlc_model_step_backward": (C.c_int, [_P, _P, _P, _P, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), _P, _P]),
     "marlc_adam_step": (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                                   _P, _P]),

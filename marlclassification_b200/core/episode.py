@@ -3,7 +3,8 @@
 ``run_episode`` executes the whole episode inside the CUDA engine (one host
 call: gather -> CNN -> messages -> LSTMs -> heads -> sample -> transition, T
 times) and returns tensors that carry the hand-written BPTT backward as a single
-autograd node, so the reference's loss code and ``loss.backward()`` work as is.
+autograd node, so the reference's loss code and ``loss.backward()`` work as is: the
+gradients reach the parameters and, when it requires grad, the image batch.
 """
 from __future__ import annotations
 
@@ -52,7 +53,9 @@ class EpisodeSampler:
         if img.dim() != 4:
             raise RuntimeError(f"only 2-D images [B,C,H,W] are supported, got {tuple(img.shape)}")
         eng = self.engine_for(img)
-        if th.is_grad_enabled() and any(p.requires_grad for p in eng.model.parameters()):
+        # the autograd node is built for the parameters or for the image (attribution on a frozen model); the
+        # conversion above is differentiable, so the image gradient reaches img_batch itself
+        if th.is_grad_enabled() and (img.requires_grad or any(p.requires_grad for p in eng.model.parameters())):
             preds, logp, values, pos = rollout_autograd(eng, img, pos0, hidden0, actions)
         else:
             eng.forward(img, pos0, hidden0, actions)

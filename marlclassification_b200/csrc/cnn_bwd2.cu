@@ -258,4 +258,195 @@ int cnn_im2col_input(const CnnWindows& win, float* col, int P, int cin, int ho, 
     return 0;
 }
 
+// Image gradient (marlc_episode_image_grad): for conv 3x3, stride 2, padding 1 and the window gather,
+//     d_img[b,c,y,x] = sum over windows (t,a) of image b that cover (y,x), in (t,a) order,
+//                      sum over taps (ky,kx) with 2*oy-1+ky = y-py, 2*ox-1+kx = x-px, and co,
+//                      dY0[t,a,b][oy,ox][co] * W0[co,c,ky,kx].
+// One CTA per (image, 32x16 pixel tile), 2 pixels per thread (16x2 pixels per warp in each 16x16 half), the sums
+// in registers: no atomics, no intermediate in global memory, and every pixel adds its windows in the same
+// order on every call.  The image's windows are tested against the tile IG_THREADS at a time; each chunk's
+// overlapping windows are compacted in order into shared memory and consumed before the next chunk is tested,
+// so the list never overflows whatever the number of windows per image.  The dY0 blocks of the listed windows
+// are staged in shared memory `batch` windows at a time with all loads in flight (read one after the other
+// from global memory, each tap waited a full memory latency).  A pixel at window row ly gets 1 tap row (ly
+// even: ky = 1) or 2 (ly odd: ky = 2, and ky = 0 unless oy = (ly+1)/2 falls off the last output row), the same
+// for columns: the taps are found without division.
+constexpr int IG_TW = 32, IG_TH = 16;  // pixel tile: columns, rows
+constexpr int IG_THREADS = 256;
+constexpr int IG_PX = 2;   // pixels per thread
+constexpr int IG_CB = 4;   // input channels per accumulation pass (W_0 rows padded to a multiple of 4)
+constexpr int IG_STAGE_BYTES = 24 * 1024;  // dY0 staging budget per CTA
+// 3 CTAs per SM: the register budget (80) at which the two pixels' accumulators and taps fit without spills
+
+__global__ void __launch_bounds__(IG_THREADS, 3) cnn_image_grad_kernel(const ImageGradArgs a, FastDiv d_na,
+                                                                     FastDiv d_cin, FastDiv d_blk4, int cinp,
+                                                                     int batch) {
+    extern __shared__ float4 sm4[];
+    const int co_n = a.cout, ci_n = a.cin, f = a.f, ho = a.ho, M = a.Na * a.B, n_win = a.T * a.Na;
+    const int wsz = co_n * cinp;     // floats per tap of W_0
+    const int blk = ho * ho * co_n;  // floats of one window's dY0 block (a multiple of 4)
+    float* sw = reinterpret_cast<float*>(sm4);  // W_0 as [tap][cout][cinp], zero in the padded channels
+    float* sdy = sw + 9 * wsz;                  // dY0 blocks of `batch` listed windows
+    __shared__ int list_p[IG_THREADS], list_y[IG_THREADS], list_x[IG_THREADS];
+    __shared__ int warp_n[IG_THREADS / 32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int b = blockIdx.z, y0 = blockIdx.y * IG_TH, x0 = blockIdx.x * IG_TW;
+    for (int i = tid; i < 9 * wsz; i += IG_THREADS) sw[i] = 0.f;
+    __syncthreads();
+    for (int j = tid; j < co_n * ci_n * 9; j += IG_THREADS) {  // source index (co*cin + c)*9 + tap
+        const int q = j / 9, tap = j - q * 9, co = d_cin.div(q), c = q - co * ci_n;
+        sw[tap * wsz + co * cinp + c] = __ldg(a.w0 + j);
+    }
+    int py[IG_PX], px[IG_PX];
+#pragma unroll
+    for (int k = 0; k < IG_PX; ++k) {
+        py[k] = y0 + (tid >> 4);
+        px[k] = x0 + (tid & 15) + 16 * k;
+    }
+    const long plane = (long)a.H * a.W;
+    float* out = a.d_img + (long)b * a.C * plane;
+    const float4* dy4 = reinterpret_cast<const float4*>(a.dY0);
+    const int blk4 = blk >> 2;
+    for (int c0 = 0; c0 < ci_n; c0 += IG_CB) {
+        float acc[IG_PX][IG_CB];
+#pragma unroll
+        for (int k = 0; k < IG_PX; ++k)
+#pragma unroll
+            for (int u = 0; u < IG_CB; ++u) acc[k][u] = 0.f;
+        for (int w0 = 0; w0 < n_win; w0 += IG_THREADS) {
+            // 1. this chunk's windows overlapping the tile, compacted in (t, a) order
+            const int w = w0 + tid;
+            int p = 0, wy = 0, wx = 0;
+            bool hit = false;
+            if (w < n_win) {
+                const int t = d_na.div(w), ag = w - t * a.Na;
+                p = t * M + ag * a.B + b;
+                wy = a.pos_hist[2 * (long)p];
+                wx = a.pos_hist[2 * (long)p + 1];
+                hit = wy < y0 + IG_TH && wy + f > y0 && wx < x0 + IG_TW && wx + f > x0;
+            }
+            const unsigned bal = __ballot_sync(0xffffffffu, hit);
+            __syncthreads();  // the previous chunk's list is consumed
+            if (lane == 0) warp_n[warp] = __popc(bal);
+            __syncthreads();
+            int off = 0, n = 0;
+#pragma unroll
+            for (int k = 0; k < IG_THREADS / 32; ++k) {
+                const int v = warp_n[k];
+                off += k < warp ? v : 0;
+                n += v;
+            }
+            if (hit) {
+                const int slot = off + __popc(bal & ((1u << lane) - 1u));
+                list_p[slot] = p;
+                list_y[slot] = wy;
+                list_x[slot] = wx;
+            }
+            for (int i0 = 0; i0 < n; i0 += batch) {
+                const int nb = min(batch, n - i0);
+                __syncthreads();  // the list is written / the previous batch is consumed
+                // 2. stage the batch's dY0 blocks
+                float4* s4 = reinterpret_cast<float4*>(sdy);
+#pragma unroll 4
+                for (int e = tid; e < nb * blk4; e += IG_THREADS) {
+                    const int jw = d_blk4.div(e);
+                    s4[e] = __ldg(dy4 + (long)list_p[i0 + jw] * blk4 + (e - jw * blk4));
+                }
+                __syncthreads();
+                // 3. the transposed convolution of each staged window at this thread's pixels
+                for (int jw = 0; jw < nb; ++jw) {
+                    const int wyj = list_y[i0 + jw], wxj = list_x[i0 + jw];
+                    const float* g = sdy + jw * blk;
+#pragma unroll
+                    for (int k = 0; k < IG_PX; ++k) {
+                        const int ly = py[k] - wyj, lx = px[k] - wxj;
+                        if ((unsigned)ly >= (unsigned)f || (unsigned)lx >= (unsigned)f) continue;
+#pragma unroll
+                        for (int iy = 0; iy < 2; ++iy) {
+                            int ky, oy;
+                            if (ly & 1) {
+                                ky = iy ? 0 : 2;
+                                oy = iy ? (ly + 1) >> 1 : (ly - 1) >> 1;
+                                if (oy >= ho) continue;
+                            } else {
+                                if (iy) continue;
+                                ky = 1;
+                                oy = ly >> 1;
+                            }
+#pragma unroll
+                            for (int ix = 0; ix < 2; ++ix) {
+                                int kx, ox;
+                                if (lx & 1) {
+                                    kx = ix ? 0 : 2;
+                                    ox = ix ? (lx + 1) >> 1 : (lx - 1) >> 1;
+                                    if (ox >= ho) continue;
+                                } else {
+                                    if (ix) continue;
+                                    kx = 1;
+                                    ox = lx >> 1;
+                                }
+                                const float4* gp = reinterpret_cast<const float4*>(g + (oy * ho + ox) * co_n);
+                                const float4* wp = reinterpret_cast<const float4*>(sw + (ky * 3 + kx) * wsz + c0);
+                                const int wstride = cinp >> 2;
+                                for (int q = 0; q < (co_n >> 2); ++q) {
+                                    const float4 gv = gp[q];
+                                    const float gs[4] = {gv.x, gv.y, gv.z, gv.w};
+#pragma unroll
+                                    for (int u = 0; u < 4; ++u) {
+                                        const float4 wv = wp[(4 * q + u) * wstride];
+                                        acc[k][0] += gs[u] * wv.x;
+                                        acc[k][1] += gs[u] * wv.y;
+                                        acc[k][2] += gs[u] * wv.z;
+                                        acc[k][3] += gs[u] * wv.w;
+                                    }
+                                }
+                            }
+                        }
+                    }
+                }
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < IG_PX; ++k)
+            if (py[k] < a.H && px[k] < a.W)
+#pragma unroll
+                for (int u = 0; u < IG_CB; ++u)
+                    if (c0 + u < ci_n) out[(c0 + u) * plane + (long)py[k] * a.W + px[k]] = acc[k][u];
+    }
+#pragma unroll
+    for (int k = 0; k < IG_PX; ++k)  // channels the network does not read (MnistCnn on a 3-channel batch)
+        if (py[k] < a.H && px[k] < a.W)
+            for (int c = ci_n; c < a.C; ++c) out[c * plane + (long)py[k] * a.W + px[k]] = 0.f;
+}
+
+int cnn_image_grad(const ImageGradArgs& a, cudaStream_t s) {
+    MARLC_CHECK(a.dY0 && a.w0 && a.pos_hist && a.d_img, "image_grad: null pointer");
+    MARLC_CHECK(a.cin >= 1 && a.cin <= a.C && a.cout >= 1 && a.ho == (a.f - 1) / 2 + 1, "image_grad: bad CNN shape");
+    // dY0 rows are read as float4: every feature extractor of the package has a multiple of 4 first-layer channels
+    MARLC_CHECK((a.cout & 3) == 0 && (reinterpret_cast<uintptr_t>(a.dY0) & 15) == 0,
+                "image_grad: the first conv layer needs a multiple of 4 output channels (has %d)", a.cout);
+    const unsigned tx = (a.W + IG_TW - 1) / IG_TW, ty = (a.H + IG_TH - 1) / IG_TH;
+    MARLC_CHECK(ty <= 65535 && a.B <= 65535, "image_grad: image batch %d x %d rows too large for the grid", a.B, a.H);
+    const long n_win = (long)a.T * a.Na;
+    MARLC_CHECK(n_win < (1L << 31) && FastDiv::exact_up_to(n_win, a.Na), "image_grad: %ld windows per image", n_win);
+    const int cinp = (a.cin + IG_CB - 1) / IG_CB * IG_CB;
+    const int blk = a.ho * a.ho * a.cout;
+    const int batch = std::max(1, std::min(IG_THREADS, IG_STAGE_BYTES / (blk * (int)sizeof(float))));
+    MARLC_CHECK(FastDiv::exact_up_to((long long)batch * blk / 4, blk / 4) &&
+                    FastDiv::exact_up_to((long long)a.cout * a.cin * 9, a.cin),
+                "image_grad: window block of %d floats too large", blk);
+    const size_t smem = ((size_t)9 * a.cout * cinp + (size_t)batch * blk) * sizeof(float);
+    MARLC_CHECK(smem <= 200 * 1024, "image_grad: first-layer shapes too large for shared memory (%zu B)", smem);
+    static size_t attr = 0;
+    if (smem > 48 * 1024 && smem > attr) {
+        MARLC_CUDA(cudaFuncSetAttribute(cnn_image_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr = smem;
+    }
+    const dim3 grid(tx, ty, (unsigned)a.B);
+    cnn_image_grad_kernel<<<grid, IG_THREADS, smem, s>>>(a, FastDiv((unsigned)a.Na), FastDiv((unsigned)a.cin),
+                                                         FastDiv((unsigned)(blk / 4)), cinp, batch);
+    MARLC_LAUNCH_CHECK();
+    return 0;
+}
+
 }  // namespace marlc

@@ -91,6 +91,9 @@ struct marlc_engine {
     // 1, 2 and 4 chunks take the same time (the overlapped launches delay the sweep as much as they save), 8 is
     // slower, so the default is one chunk after the sweep.
     int bwd_chunks = 1;
+    // cnn_dY0 holds the first layer's conv-output gradients of the last rollout: set by a complete
+    // marlc_episode_backward, cleared by every forward and by a step-wise backward (marlc_episode_image_grad)
+    bool dy0_ready = false;
     cudaEvent_t ev[64];
     int n_ev = 0, ev_i = 0;
     cudaEvent_t next_event() { cudaEvent_t x = ev[ev_i]; ev_i = (ev_i + 1) % n_ev; return x; }
@@ -832,6 +835,7 @@ extern "C" int marlc_episode_forward(marlc_engine* e, const float* img, const in
     MARLC_CHECK(e && e->ws, "engine not bound");
     MARLC_CHECK(img, "null image batch");
     NvtxRange nvtx_fwd("marlc/forward");
+    e->dy0_ready = false;
     cudaStream_t s = (cudaStream_t)stream;
     const marlc_config& c = e->cfg;
     const int M = e->M, T = c.T;
@@ -889,6 +893,7 @@ extern "C" int marlc_episode_forward(marlc_engine* e, const float* img, const in
 // msg[1], H[1], Cb[1], Hc[1], Cc[1].
 static int model_step_fwd(marlc_engine* e, const float* patch, const float* msg, const float* npos,
                           const float* const* hidden, cudaStream_t s) {
+    e->dy0_ready = false;
     MARLC_TRY(refresh_lo(e, nullptr, nullptr, s));
     if (e->cfg.use_chains && e->cfg.use_tc) {
         MARLC_CUDA(cudaMemsetAsync(e->buf("enc_y1"), 0, sizeof(float) * (size_t)e->M * 2 * e->cfg.n_m, s));
@@ -1012,6 +1017,7 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
     const marlc_config& c = e->cfg;
     const int M = e->M, T = c.T, TM = e->TM, Kin = e->Kin, F = e->F;
     const int start = g_launch_count;
+    e->dy0_ready = false;  // until this backward runs to its end
     const float* d_probs = se ? se->d_out[0] : nullptr;
     const float* d_msg_out = se ? se->d_out[3] : nullptr;  // seeds the encoder backward of the last step
     const bool want_dh0 = se && (se->d_in[1] || se->d_in[3]);  // input gradients of step 0's recurrent states
@@ -1476,7 +1482,8 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
         MARLC_TRY(e->chain(s, e->side[1]));
         MARLC_TRY(batched(0, T, s, e->side[1], e->side[0]));
     }
-    if (par) MARLC_TRY(join_sides());
+    if (par) MARLC_TRY(join_sides());  // dY0 included: the caller's stream is ordered after every side-stream launch
+    e->dy0_ready = se == nullptr;
     e->last_launches = g_launch_count - start;
     return 0;
 }
@@ -1529,6 +1536,26 @@ extern "C" int marlc_model_step_backward(marlc_engine* e, const float* patch, co
     MARLC_TRY(episode_backward(e, nullptr, 0, &se, s));
     e->last_launches = g_launch_count - start;
     return 0;
+}
+
+// d img of the last rollout from cnn_dY0 (see include/marlc.h).  The first conv layer's weights are read as they
+// are now: call it before the parameters change.
+extern "C" int marlc_episode_image_grad(marlc_engine* e, float* d_img, void* stream) {
+    MARLC_CHECK(e && e->ws, "engine not bound");
+    MARLC_CHECK(d_img, "episode_image_grad: null output");
+    MARLC_CHECK(e->dy0_ready,
+                "episode_image_grad: no complete marlc_episode_backward of the engine's last rollout (none since the "
+                "last forward / model step, a step-wise backward, or a backward cut short by marlc_engine_debug_stop)");
+    const marlc_config& c = e->cfg;
+    ImageGradArgs a;
+    a.dY0 = e->buf("cnn_dY0");
+    a.w0 = e->cnn.w[0];
+    a.pos_hist = e->buf<int>("pos_hist");
+    a.d_img = d_img;
+    a.T = c.T; a.Na = c.na; a.B = c.nb; a.C = c.C; a.H = c.H; a.W = c.W; a.f = c.f;
+    a.cin = e->cnn.cin[0]; a.cout = e->cnn.cout[0]; a.ho = e->cnn.hout[0];
+    NvtxRange nvtx("marlc/image_grad");
+    return cnn_image_grad(a, (cudaStream_t)stream);
 }
 
 extern "C" int marlc_engine_last_launches(const marlc_engine* e) { return e->last_launches; }

@@ -125,6 +125,16 @@ struct CnnBwdLayerArgs {
 };
 int cnn_bwd_layer(const CnnBwdLayerArgs& a, cudaStream_t s);
 int cnn_im2col_input(const CnnWindows& win, float* col, int P, int cin, int ho, cudaStream_t s);
+// Gradient on the image batch from the first layer's conv-output gradients of all T*M windows: the transposed
+// convolution with W_0 fused with the adjoint of the window gather (a pixel sums every window covering it).
+struct ImageGradArgs {
+    const float* dY0;     // [T*M windows][ho*ho][cout] (cnn_dY0; window p = t*M + a*B + b)
+    const float* w0;      // [cout][cin][3][3]
+    const int* pos_hist;  // [T][M][2] window corners (row, column) of the observations the networks consumed
+    float* d_img;         // out [B][C][H][W], every element written
+    int T, Na, B, C, H, W, f, cin, cout, ho;
+};
+int cnn_image_grad(const ImageGradArgs& a, cudaStream_t s);
 
 // ---- loss.cu ------------------------------------------------------------------
 struct LossArgs {

@@ -6,6 +6,7 @@
 * ``forward``  -- the whole T-step rollout (episode.py:32-85),
 * ``loss``     -- the fused actor-critic loss and its gradients (trainer.py:75-111),
 * ``backward`` -- hand-written BPTT into the model's flat gradient buffer,
+* ``image_grad`` -- the gradient that backward leaves on the image batch,
 
 plus ``rollout_autograd`` which wraps forward/backward in ONE autograd node so
 the reference's own loss code (``loss.backward()``) works unchanged.
@@ -205,6 +206,19 @@ class EpisodeEngine:
         _lib.check(self._L.marlc_episode_backward(self._h, img.data_ptr(), 1 if accumulate else 0, self._stream()))
         self.launches["backward"] = self._L.marlc_engine_last_launches(self._h)
 
+    def image_grad(self, out: Optional[th.Tensor] = None) -> th.Tensor:
+        """d(what the last ``backward`` was seeded with) / d img, f32 [nb, C, H, W] (``marlc_episode_image_grad``),
+        written into ``out`` when given.  Call it after ``backward`` of the last rollout and before the parameters
+        change; raises when that backward is missing."""
+        shape = (self.nb, self.C, self.H, self.W)
+        if out is None:
+            out = th.empty(shape, dtype=th.float32, device=self.device)
+        elif (tuple(out.shape) != shape or out.dtype != th.float32 or out.device != th.device(self.device)
+              or not out.is_contiguous()):
+            raise RuntimeError(f"image_grad(out): need a contiguous float32 {shape} tensor on {self.device}")
+        _lib.check(self._L.marlc_episode_image_grad(self._h, out.data_ptr(), self._stream()))
+        return out
+
     def model_step(self, patch, msg, npos, hidden) -> None:
         hid = (ct.c_void_p * 4)(*[h.data_ptr() for h in hidden])
         self._keep = [patch, msg, npos, *hidden]
@@ -257,7 +271,8 @@ def get_engine(model, *, na, nb, T, C, H, W, actions, gamma=0.99) -> EpisodeEngi
 class _RolloutFn(th.autograd.Function):
     """The whole episode as ONE autograd node: forward = fused rollout, backward =
     hand-written BPTT.  Parameter gradients are returned to autograd as clones
-    of the flat-bucket views so ``loss.backward()`` accumulates them normally."""
+    of the flat-bucket views so ``loss.backward()`` accumulates them normally; the
+    image gradient, when the image requires grad, comes from ``image_grad``."""
 
     @staticmethod
     def forward(ctx, engine: EpisodeEngine, img, pos0, hidden0, actions, *params):
@@ -284,12 +299,16 @@ class _RolloutFn(th.autograd.Function):
         # BPTT into a scratch use of the flat bucket: save + restore what was there
         saved = eng.model.flat_grads.clone()
         eng.backward(ctx.img, accumulate=False)
+        d_img = eng.image_grad() if ctx.needs_input_grad[1] else None
         grads = []
-        for p in eng.model.parameters():
+        for i, p in enumerate(eng.model.parameters()):
+            if not ctx.needs_input_grad[5 + i]:
+                grads.append(None)
+                continue
             off = (p.data.data_ptr() - eng.model.flat_params.data_ptr()) // 4
             grads.append(eng.model.flat_grads[off: off + p.numel()].view(p.shape).clone())
         eng.model.flat_grads.copy_(saved)
-        return (None, None, None, None, None, *grads)
+        return (None, d_img, None, None, None, *grads)
 
 
 def rollout_autograd(engine: EpisodeEngine, img, pos0=None, hidden0=None, actions=None):
