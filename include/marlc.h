@@ -34,6 +34,13 @@ long marlc_selftest_fastdiv(int d_max, int stride);
  * pos i64[Na,B,2], obs f32[Na,B,C,f,f]. */
 int marlc_patch_gather(const float* img, const int64_t* pos, float* obs, int Na, int B, int C, int H, int W, int f,
                        void* stream);
+/* Backward of marlc_patch_gather (the adjoint of the window gather): overwrites d_img f32[B,C,H,W], every
+ * element, with d_img[b,c,y,x] = sum over a = 0..Na-1 whose window covers (y,x), in that order, of
+ * d_obs[a,b,c,y-pos[a,b,0],x-pos[a,b,1]]; d_obs f32[Na,B,C,f,f], pos as for marlc_patch_gather.  Pixels no
+ * window covers get 0.  Each pixel sums in fp32 from 0 in agent order: deterministic, the same bits as that
+ * sequential loop.  Neither allocates nor synchronises (capturable). */
+int marlc_patch_gather_backward(const float* d_obs, const int64_t* pos, float* d_img, int Na, int B, int C, int H,
+                                int W, int f, void* stream);
 
 /* Environment.step / __transition, environment.py:56-66,128-150 (+ the
  * normalized_positions property, 74-81).  pos i64[Na*B,2] updated in place;
@@ -206,6 +213,15 @@ int marlc_episode_image_grad(marlc_engine* e, float* d_img, void* stream);
 int marlc_model_step_backward(marlc_engine* e, const float* patch, const float* msg, const float* npos,
                               const float* const* hidden, const float* const* d_out, float* const* d_in,
                               float* grads, void* stream);
+
+/* Gradients on the window and position inputs of the last marlc_model_step_backward (the step-wise API with
+ * input gradients): d_patch f32[na,nb,C,f,f] (0 in the channels the feature extractor does not read) and
+ * d_npos f32[na,nb,2], each nullable (= not wanted), at least one non-null; both overwritten.  Call it after
+ * marlc_model_step_backward, on the same stream and before the parameters change (the first conv layer's and
+ * map_pos.0's weights are read here).  Deterministic; neither allocates nor synchronises (capturable).  Fails
+ * when there was no complete marlc_model_step_backward since the last marlc_episode_forward / marlc_model_step
+ * / marlc_episode_backward, or after a backward cut short by marlc_engine_debug_stop. */
+int marlc_model_step_input_grad(marlc_engine* e, float* d_patch, float* d_npos, void* stream);
 
 /* optim.step(), trainer.py:33,116: torch.optim.Adam semantics (no weight decay,
  * no amsgrad) over the flat bucket; g is multiplied by grad_scale first (1/world

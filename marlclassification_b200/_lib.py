@@ -48,6 +48,7 @@ _SIGS = {
     "marlc_selftest_fastdiv": (C.c_long, [C.c_int, C.c_int]),
     "marlc_last_error": (C.c_char_p, []),
     "marlc_patch_gather": (C.c_int, [_P, _P, _P] + [C.c_int] * 6 + [_P]),
+    "marlc_patch_gather_backward": (C.c_int, [_P, _P, _P] + [C.c_int] * 6 + [_P]),
     "marlc_transition": (C.c_int, [_P, _P, _P] + [C.c_int] * 5 + [_P, _P, _P]),
     "marlc_normalized_positions": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P]),
     "marlc_images_u8_to_f32": (C.c_int, [_P, _P] + [C.c_int] * 5 + [_P]),
@@ -79,6 +80,7 @@ _SIGS = {
     "marlc_episode_backward": (C.c_int, [_P, _P, C.c_int, _P]),
     "marlc_episode_image_grad": (C.c_int, [_P, _P, _P]),
     "marlc_model_step_backward": (C.c_int, [_P, _P, _P, _P, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), _P, _P]),
+    "marlc_model_step_input_grad": (C.c_int, [_P, _P, _P, _P]),
     "marlc_adam_step": (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                                   _P, _P]),
     "marlc_engine_debug_stop": (C.c_int, [_P, C.c_int]),

@@ -8,6 +8,38 @@ import torch as th
 from .. import _lib
 
 
+def _gather(img: th.Tensor, pos: th.Tensor, f: int) -> th.Tensor:
+    na, nb = pos.shape[0], pos.shape[1]
+    _, c, h, w = img.shape
+    obs = th.empty(na, nb, c, f, f, dtype=th.float32, device=img.device)
+    _lib.check(_lib.lib().marlc_patch_gather(img.data_ptr(), pos.data_ptr(), obs.data_ptr(), na, nb, c, h, w, f,
+                                             _lib.stream_ptr(img.device)))
+    return obs
+
+
+class _ObserveFn(th.autograd.Function):
+    """Environment.observe as an autograd node: forward = marlc_patch_gather, backward = its adjoint
+    marlc_patch_gather_backward (a pixel sums the gradients of the windows covering it, in agent order).  The
+    positions of the call are saved: ``step`` binds a new tensor, so they stay those of this observation."""
+
+    @staticmethod
+    def forward(ctx, img, pos, f):
+        ctx.save_for_backward(pos)
+        ctx.f, ctx.img_shape = f, img.shape
+        return _gather(img, pos, f)
+
+    @staticmethod
+    def backward(ctx, d_obs):
+        (pos,) = ctx.saved_tensors
+        d_obs = d_obs.float().contiguous()
+        na, nb = pos.shape[0], pos.shape[1]
+        _, c, h, w = ctx.img_shape
+        d_img = th.empty(ctx.img_shape, dtype=th.float32, device=d_obs.device)
+        _lib.check(_lib.lib().marlc_patch_gather_backward(d_obs.data_ptr(), pos.data_ptr(), d_img.data_ptr(), na, nb,
+                                                          c, h, w, ctx.f, _lib.stream_ptr(d_obs.device)))
+        return d_img, None, None
+
+
 class Environment:
     def __init__(self, actions: list[list[int]], window_size: int) -> None:
         self.__actions = actions
@@ -39,14 +71,13 @@ class Environment:
         return self.observe()
 
     def observe(self) -> th.Tensor:
+        """The agents' windows [Na, B, C, f, f].  When the image batch requires grad (in grad mode) they carry
+        a backward to it, as the reference's masked_select does (environment.py:96-126)."""
         assert self.__img_batch is not None, "reset() must be called before observe()"
         img, pos, f = self.__img_batch, self.__pos, self.__window_size
-        na, nb = pos.shape[0], pos.shape[1]
-        _, c, h, w = img.shape
-        obs = th.empty(na, nb, c, f, f, dtype=th.float32, device=img.device)
-        _lib.check(_lib.lib().marlc_patch_gather(img.data_ptr(), pos.data_ptr(), obs.data_ptr(), na, nb, c, h, w, f,
-                                                 _lib.stream_ptr(img.device)))
-        return obs
+        if th.is_grad_enabled() and img.requires_grad:
+            return _ObserveFn.apply(img, pos, f)
+        return _gather(img, pos, f)
 
     def step(self, action_indices: th.Tensor) -> th.Tensor:
         """Apply the chosen actions (integer rule of environment.py:128-150: a

@@ -449,4 +449,138 @@ int cnn_image_grad(const ImageGradArgs& a, cudaStream_t s) {
     return 0;
 }
 
+// W_0 [cout][cin][3][3] -> shared [tap][cout][cinp], zero in the padded channels (nt threads)
+__device__ __forceinline__ void stage_w0(float* sw, const float* w0, int co_n, int ci_n, int cinp, FastDiv d_cin,
+                                         int nt) {
+    const int wsz = co_n * cinp;
+    for (int i = threadIdx.x; i < 9 * wsz; i += nt) sw[i] = 0.f;
+    __syncthreads();
+    for (int j = threadIdx.x; j < co_n * ci_n * 9; j += nt) {  // source index (co*cin + c)*9 + tap
+        const int q = j / 9, tap = j - q * 9, co = d_cin.div(q), c = q - co * ci_n;
+        sw[tap * wsz + co * cinp + c] = __ldg(w0 + j);
+    }
+}
+
+// Input channels c0 .. c0+3 of the first conv layer's input gradient at pixel (ly, lx) of one window
+// (0 <= ly, lx < f): acc[u] += sum over the pixel's taps, in (ky, kx) order, and over co of
+// g[(oy*ho + ox)*cout + co] * W0[co, c0+u, ky, kx].  g: the window's dY0 block; sw: W_0 as stage_w0 left it.
+// The tap walk of cnn_image_grad_kernel, which keeps it inline: as a call there it costs a spill at the image
+// kernel's 80-register budget.
+__device__ __forceinline__ void conv0_pixel_grad(const float* g, const float* sw, int ly, int lx, int ho, int co_n,
+                                                 int cinp, int c0, float (&acc)[IG_CB]) {
+    const int wsz = co_n * cinp;
+#pragma unroll
+    for (int iy = 0; iy < 2; ++iy) {
+        int ky, oy;
+        if (ly & 1) {
+            ky = iy ? 0 : 2;
+            oy = iy ? (ly + 1) >> 1 : (ly - 1) >> 1;
+            if (oy >= ho) continue;
+        } else {
+            if (iy) continue;
+            ky = 1;
+            oy = ly >> 1;
+        }
+#pragma unroll
+        for (int ix = 0; ix < 2; ++ix) {
+            int kx, ox;
+            if (lx & 1) {
+                kx = ix ? 0 : 2;
+                ox = ix ? (lx + 1) >> 1 : (lx - 1) >> 1;
+                if (ox >= ho) continue;
+            } else {
+                if (ix) continue;
+                kx = 1;
+                ox = lx >> 1;
+            }
+            const float4* gp = reinterpret_cast<const float4*>(g + (oy * ho + ox) * co_n);
+            const float4* wp = reinterpret_cast<const float4*>(sw + (ky * 3 + kx) * wsz + c0);
+            const int wstride = cinp >> 2;
+            for (int q = 0; q < (co_n >> 2); ++q) {
+                const float4 gv = gp[q];
+                const float gs[4] = {gv.x, gv.y, gv.z, gv.w};
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const float4 wv = wp[(4 * q + u) * wstride];
+                    acc[0] += gs[u] * wv.x;
+                    acc[1] += gs[u] * wv.y;
+                    acc[2] += gs[u] * wv.z;
+                    acc[3] += gs[u] * wv.w;
+                }
+            }
+        }
+    }
+}
+
+// Gradient on the caller's windows of one stand-alone step (marlc_model_step_input_grad): the first conv
+// layer's input gradient, window by window,
+//     d_patch[p,c,ly,lx] = sum over taps (ky,kx) with 2*oy-1+ky = ly, 2*ox-1+kx = lx, and co,
+//                          dY0[p][oy,ox][co] * W0[co,c,ky,kx],
+// and 0 in the channels c >= cin the network does not read.  No gather: the windows are the caller's.  Each
+// output element has one owner thread, which sums its taps in a fixed order (conv0_pixel_grad): no atomics.
+// One CTA per `batch` consecutive windows: W_0 staged once, then the windows' dY0 blocks (one contiguous
+// range) with all loads in flight, then one thread per (window, pixel), consecutive threads on consecutive
+// pixels of a channel plane (coalesced stores).
+constexpr int PG_THREADS = 256;
+constexpr int PG_MAX_BATCH = 8;            // windows per CTA: 8 x 144 pixels at f = 12
+constexpr int PG_STAGE_BYTES = 24 * 1024;  // dY0 staging budget per CTA
+
+__global__ void __launch_bounds__(PG_THREADS) cnn_patch_grad_kernel(const PatchGradArgs a, FastDiv d_cin, FastDiv d_ff,
+                                                                    FastDiv d_f, int cinp, int batch) {
+    extern __shared__ float4 sm4[];
+    const int co_n = a.cout, ci_n = a.cin, f = a.f, ff = f * f, ho = a.ho;
+    const int blk = ho * ho * co_n;
+    float* sw = reinterpret_cast<float*>(sm4);
+    float* sdy = sw + 9 * co_n * cinp;
+    const int p0 = blockIdx.x * batch, nb = min(batch, a.M - p0);
+    stage_w0(sw, a.w0, co_n, ci_n, cinp, d_cin, PG_THREADS);
+    {
+        const float4* src = reinterpret_cast<const float4*>(a.dY0) + (long)p0 * (blk >> 2);
+        float4* s4 = reinterpret_cast<float4*>(sdy);
+#pragma unroll 4
+        for (int e = threadIdx.x; e < nb * (blk >> 2); e += PG_THREADS) s4[e] = __ldg(src + e);
+    }
+    __syncthreads();
+    for (int it = threadIdx.x; it < nb * ff; it += PG_THREADS) {
+        const int jw = d_ff.div(it), q = it - jw * ff, ly = d_f.div(q), lx = q - ly * f;
+        const float* g = sdy + jw * blk;
+        float* out = a.d_patch + (long)(p0 + jw) * a.C * ff + q;
+        for (int c0 = 0; c0 < ci_n; c0 += IG_CB) {
+            float acc[IG_CB] = {0.f, 0.f, 0.f, 0.f};
+            conv0_pixel_grad(g, sw, ly, lx, ho, co_n, cinp, c0, acc);
+#pragma unroll
+            for (int u = 0; u < IG_CB; ++u)
+                if (c0 + u < ci_n) out[(c0 + u) * ff] = acc[u];
+        }
+        for (int c = ci_n; c < a.C; ++c) out[c * ff] = 0.f;  // MnistCnn on 3-channel windows
+    }
+}
+
+int cnn_patch_grad(const PatchGradArgs& a, cudaStream_t s) {
+    MARLC_CHECK(a.dY0 && a.w0 && a.d_patch, "patch_grad: null pointer");
+    MARLC_CHECK(a.cin >= 1 && a.cin <= a.C && a.cout >= 1 && a.f >= 1 && a.ho == (a.f - 1) / 2 + 1,
+                "patch_grad: bad CNN shape");
+    MARLC_CHECK((a.cout & 3) == 0 && (reinterpret_cast<uintptr_t>(a.dY0) & 15) == 0,
+                "patch_grad: the first conv layer needs a multiple of 4 output channels (has %d)", a.cout);
+    if (a.M <= 0) return 0;
+    const int cinp = (a.cin + IG_CB - 1) / IG_CB * IG_CB;
+    const int blk = a.ho * a.ho * a.cout, ff = a.f * a.f;
+    const int batch = std::max(1, std::min(PG_MAX_BATCH, PG_STAGE_BYTES / (blk * (int)sizeof(float))));
+    MARLC_CHECK(FastDiv::exact_up_to((long long)batch * ff, ff) && FastDiv::exact_up_to(ff, a.f) &&
+                    FastDiv::exact_up_to((long long)a.cout * a.cin * 9, a.cin),
+                "patch_grad: window of %d x %d too large", a.f, a.f);
+    const size_t smem = ((size_t)9 * a.cout * cinp + (size_t)batch * blk) * sizeof(float);
+    MARLC_CHECK(smem <= 200 * 1024, "patch_grad: first-layer shapes too large for shared memory (%zu B)", smem);
+    static size_t attr = 0;
+    if (smem > 48 * 1024 && smem > attr) {
+        MARLC_CUDA(cudaFuncSetAttribute(cnn_patch_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr = smem;
+    }
+    const unsigned grid = (unsigned)((a.M + batch - 1) / batch);
+    cnn_patch_grad_kernel<<<grid, PG_THREADS, smem, s>>>(a, FastDiv((unsigned)a.cin), FastDiv((unsigned)ff),
+                                                          FastDiv((unsigned)a.f), cinp, batch);
+    MARLC_LAUNCH_CHECK();
+    return 0;
+}
+
 }  // namespace marlc

@@ -91,9 +91,11 @@ struct marlc_engine {
     // 1, 2 and 4 chunks take the same time (the overlapped launches delay the sweep as much as they save), 8 is
     // slower, so the default is one chunk after the sweep.
     int bwd_chunks = 1;
-    // cnn_dY0 holds the first layer's conv-output gradients of the last rollout: set by a complete
-    // marlc_episode_backward, cleared by every forward and by a step-wise backward (marlc_episode_image_grad)
-    bool dy0_ready = false;
+    // Whose first-layer conv-output gradients cnn_dY0 holds: those of the last rollout after a complete
+    // marlc_episode_backward (read by marlc_episode_image_grad), those of a stand-alone step after a complete
+    // marlc_model_step_backward (read by marlc_model_step_input_grad), or neither: every forward, model step and
+    // backward clears it first, and a backward cut short by marlc_engine_debug_stop leaves it cleared.
+    enum class Dy0Owner { none, episode, step } dy0_owner = Dy0Owner::none;
     cudaEvent_t ev[64];
     int n_ev = 0, ev_i = 0;
     cudaEvent_t next_event() { cudaEvent_t x = ev[ev_i]; ev_i = (ev_i + 1) % n_ev; return x; }
@@ -835,7 +837,7 @@ extern "C" int marlc_episode_forward(marlc_engine* e, const float* img, const in
     MARLC_CHECK(e && e->ws, "engine not bound");
     MARLC_CHECK(img, "null image batch");
     NvtxRange nvtx_fwd("marlc/forward");
-    e->dy0_ready = false;
+    e->dy0_owner = marlc_engine::Dy0Owner::none;
     cudaStream_t s = (cudaStream_t)stream;
     const marlc_config& c = e->cfg;
     const int M = e->M, T = c.T;
@@ -893,7 +895,7 @@ extern "C" int marlc_episode_forward(marlc_engine* e, const float* img, const in
 // msg[1], H[1], Cb[1], Hc[1], Cc[1].
 static int model_step_fwd(marlc_engine* e, const float* patch, const float* msg, const float* npos,
                           const float* const* hidden, cudaStream_t s) {
-    e->dy0_ready = false;
+    e->dy0_owner = marlc_engine::Dy0Owner::none;
     MARLC_TRY(refresh_lo(e, nullptr, nullptr, s));
     if (e->cfg.use_chains && e->cfg.use_tc) {
         MARLC_CUDA(cudaMemsetAsync(e->buf("enc_y1"), 0, sizeof(float) * (size_t)e->M * 2 * e->cfg.n_m, s));
@@ -1017,7 +1019,7 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
     const marlc_config& c = e->cfg;
     const int M = e->M, T = c.T, TM = e->TM, Kin = e->Kin, F = e->F;
     const int start = g_launch_count;
-    e->dy0_ready = false;  // until this backward runs to its end
+    e->dy0_owner = marlc_engine::Dy0Owner::none;  // until this backward runs to its end
     const float* d_probs = se ? se->d_out[0] : nullptr;
     const float* d_msg_out = se ? se->d_out[3] : nullptr;  // seeds the encoder backward of the last step
     const bool want_dh0 = se && (se->d_in[1] || se->d_in[3]);  // input gradients of step 0's recurrent states
@@ -1483,7 +1485,7 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
         MARLC_TRY(batched(0, T, s, e->side[1], e->side[0]));
     }
     if (par) MARLC_TRY(join_sides());  // dY0 included: the caller's stream is ordered after every side-stream launch
-    e->dy0_ready = se == nullptr;
+    e->dy0_owner = se ? marlc_engine::Dy0Owner::step : marlc_engine::Dy0Owner::episode;
     e->last_launches = g_launch_count - start;
     return 0;
 }
@@ -1543,7 +1545,7 @@ extern "C" int marlc_model_step_backward(marlc_engine* e, const float* patch, co
 extern "C" int marlc_episode_image_grad(marlc_engine* e, float* d_img, void* stream) {
     MARLC_CHECK(e && e->ws, "engine not bound");
     MARLC_CHECK(d_img, "episode_image_grad: null output");
-    MARLC_CHECK(e->dy0_ready,
+    MARLC_CHECK(e->dy0_owner == marlc_engine::Dy0Owner::episode,
                 "episode_image_grad: no complete marlc_episode_backward of the engine's last rollout (none since the "
                 "last forward / model step, a step-wise backward, or a backward cut short by marlc_engine_debug_stop)");
     const marlc_config& c = e->cfg;
@@ -1558,6 +1560,33 @@ extern "C" int marlc_episode_image_grad(marlc_engine* e, float* d_img, void* str
     return cnn_image_grad(a, (cudaStream_t)stream);
 }
 
+// d patch / d npos of the last marlc_model_step_backward from cnn_dY0 / d_pos_y (see include/marlc.h).  The
+// first conv layer's and map_pos.0's weights are read as they are now: call it before the parameters change.
+extern "C" int marlc_model_step_input_grad(marlc_engine* e, float* d_patch, float* d_npos, void* stream) {
+    MARLC_CHECK(e, "model_step_input_grad: null engine");
+    MARLC_CHECK(d_patch || d_npos, "model_step_input_grad: both outputs are null");
+    MARLC_CHECK(e->ws, "engine not bound");
+    MARLC_CHECK(e->dy0_owner == marlc_engine::Dy0Owner::step,
+                "model_step_input_grad: no complete marlc_model_step_backward since the last forward / model step / "
+                "episode backward (or a backward cut short by marlc_engine_debug_stop)");
+    const marlc_config& c = e->cfg;
+    cudaStream_t s = (cudaStream_t)stream;
+    NvtxRange nvtx("marlc/model_step_input_grad");
+    if (d_patch) {
+        PatchGradArgs a;
+        a.dY0 = e->buf("cnn_dY0");
+        a.w0 = e->cnn.w[0];
+        a.d_patch = d_patch;
+        a.M = e->M; a.C = c.C; a.f = c.f;
+        a.cin = e->cnn.cin[0]; a.cout = e->cnn.cout[0]; a.ho = e->cnn.hout[0];
+        MARLC_TRY(cnn_patch_grad(a, s));
+    }
+    // map_pos.0 is Linear(2, n_d): d npos[M,2] = d_pos_y[M,n_d] . W[n_d,2] (pitch 2: the FFMA back end)
+    if (d_npos)
+        MARLC_TRY(G_nn(e, e->buf("d_pos_y"), c.n_d, e->prm("map_pos.0.weight"), 2, d_npos, 2, e->M, c.n_d, 2, 0, s));
+    return 0;
+}
+
 extern "C" int marlc_engine_last_launches(const marlc_engine* e) { return e->last_launches; }
 extern "C" long marlc_gemm_launch_count(int ffma) { return ffma ? marlc::g_simt_gemm_launches : marlc::g_tc_gemm_launches; }
 
@@ -1566,6 +1595,11 @@ extern "C" int marlc_patch_gather(const float* img, const int64_t* pos, float* o
                                   int f, void* stream) {
     MARLC_CHECK(img && pos && obs, "patch_gather: null pointer");
     return patch_gather_i64(img, pos, obs, Na, B, C, H, W, f, (cudaStream_t)stream);
+}
+extern "C" int marlc_patch_gather_backward(const float* d_obs, const int64_t* pos, float* d_img, int Na, int B, int C,
+                                           int H, int W, int f, void* stream) {
+    MARLC_CHECK(d_obs && pos && d_img, "patch_gather_backward: null pointer");
+    return patch_gather_backward_i64(d_obs, pos, d_img, Na, B, C, H, W, f, (cudaStream_t)stream);
 }
 extern "C" int marlc_transition(int64_t* pos, const int64_t* act, const int64_t* table, int nA, int M, int f, int H,
                                 int W, float* norm_pos, int* err_flag, void* stream) {

@@ -87,6 +87,121 @@ int patch_gather_i32(const float* img, const int* pos, float* obs, int Na, int B
     return patch_gather_t<int>(img, pos, obs, Na, B, C, H, W, f, s);
 }
 
+// K1' adjoint of the patch gather (the backward of Environment.observe):
+//   d_img[b,c,y,x] = sum over agents a = 0..Na-1 whose window covers (y,x), in that order, of
+//                    d_obs[a,b,c,y-pos[a,b,0],x-pos[a,b,1]]
+// One CTA per (image, 32x16 pixel tile); a warp owns 32 consecutive columns of two rows, so every store of
+// d_img (mostly zeros: most pixels are under no window) is one 128-byte line.  The image's windows are tested
+// against the tile GB_THREADS at a time and each chunk's overlapping windows are compacted in agent order
+// (tile_window_list), so the list cannot overflow whatever Na is.  Each pixel
+// sums in registers from 0.0f in agent order: no atomics, and the result is the same bits as a sequential fp32
+// loop over the agents.
+constexpr int GB_TW = 32, GB_TH = 16, GB_THREADS = 256;
+constexpr int GB_PX = GB_TH * GB_TW / GB_THREADS;  // pixels (rows) per thread
+constexpr int GB_CB = 4;                            // channels per accumulation pass
+
+// The windows of image b that overlap the pixel tile, in agent order.  Each of the NT threads of the CTA brings
+// one candidate window (observation row m, corner wy, wx; valid = false past the last agent); those overlapping
+// the TH x TW tile at (y0, x0) are written in thread order to list_m / list_y / list_x, and their number is
+// returned to every thread.  At most NT candidates per call, so the list cannot overflow.  Starts with a block
+// barrier (the previous chunk's list may be read until then); the caller needs one more before it reads the new
+// list.  This is phase 1 of cnn_image_grad_kernel (cnn_bwd2.cu), which keeps its own copy: compiled into that
+// kernel, the helper costs an 8-byte spill at its 80-register budget.
+template <int NT, int TH, int TW>
+__device__ __forceinline__ int tile_window_list(bool valid, int m, int wy, int wx, int f, int y0, int x0, int* list_m,
+                                                int* list_y, int* list_x, int* warp_n) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const bool hit = valid && wy < y0 + TH && wy + f > y0 && wx < x0 + TW && wx + f > x0;
+    const unsigned bal = __ballot_sync(0xffffffffu, hit);
+    __syncthreads();  // the previous chunk's list is consumed
+    if (lane == 0) warp_n[warp] = __popc(bal);
+    __syncthreads();
+    int off = 0, n = 0;
+#pragma unroll
+    for (int k = 0; k < NT / 32; ++k) {
+        const int v = warp_n[k];
+        off += k < warp ? v : 0;
+        n += v;
+    }
+    if (hit) {
+        const int slot = off + __popc(bal & ((1u << lane) - 1u));
+        list_m[slot] = m;
+        list_y[slot] = wy;
+        list_x[slot] = wx;
+    }
+    return n;
+}
+
+__global__ void __launch_bounds__(GB_THREADS) patch_gather_backward_kernel(const float* __restrict__ d_obs,
+                                                                           const int64_t* __restrict__ pos,
+                                                                           float* __restrict__ d_img, int Na, int B,
+                                                                           int C, int H, int W, int f) {
+    __shared__ int list_m[GB_THREADS], list_y[GB_THREADS], list_x[GB_THREADS];
+    __shared__ int warp_n[GB_THREADS / 32];
+    const int tid = threadIdx.x;
+    const int b = blockIdx.z, y0 = blockIdx.y * GB_TH, x0 = blockIdx.x * GB_TW;
+    const int px = x0 + (tid & 31);
+    int py[GB_PX];
+#pragma unroll
+    for (int k = 0; k < GB_PX; ++k) py[k] = y0 + (tid >> 5) + k * (GB_THREADS / 32);
+    const int ff = f * f, plane = H * W;  // offsets inside one image fit 32 bits (host-checked)
+    float* out = d_img + (long)b * C * plane;
+    for (int c0 = 0; c0 < C; c0 += GB_CB) {
+        float acc[GB_PX][GB_CB];
+#pragma unroll
+        for (int k = 0; k < GB_PX; ++k)
+#pragma unroll
+            for (int u = 0; u < GB_CB; ++u) acc[k][u] = 0.f;
+        for (int a0 = 0; a0 < Na; a0 += GB_THREADS) {
+            const int ag = a0 + tid;
+            int m = 0, wy = 0, wx = 0;
+            if (ag < Na) {
+                m = ag * B + b;  // observation row m = a*B + b
+                wy = (int)pos[2 * (long)m];
+                wx = (int)pos[2 * (long)m + 1];
+            }
+            const int n = tile_window_list<GB_THREADS, GB_TH, GB_TW>(ag < Na, m, wy, wx, f, y0, x0, list_m, list_y,
+                                                                      list_x, warp_n);
+            __syncthreads();  // the list is written
+            for (int j = 0; j < n; ++j) {
+                const int lx = px - list_x[j];
+                if ((unsigned)lx >= (unsigned)f) continue;
+                const float* src = d_obs + (long)list_m[j] * C * ff + c0 * ff + lx;
+#pragma unroll
+                for (int k = 0; k < GB_PX; ++k) {
+                    const int ly = py[k] - list_y[j];
+                    if ((unsigned)ly >= (unsigned)f) continue;
+#pragma unroll
+                    for (int u = 0; u < GB_CB; ++u)
+                        if (c0 + u < C) acc[k][u] += __ldg(src + u * ff + ly * f);
+                }
+            }
+        }
+        if (px < W)
+#pragma unroll
+            for (int k = 0; k < GB_PX; ++k)
+                if (py[k] < H)
+#pragma unroll
+                    for (int u = 0; u < GB_CB; ++u)
+                        if (c0 + u < C) out[(c0 + u) * plane + py[k] * W + px] = acc[k][u];
+    }
+}
+
+int patch_gather_backward_i64(const float* d_obs, const int64_t* pos, float* d_img, int Na, int B, int C, int H, int W,
+                              int f, cudaStream_t s) {
+    MARLC_CHECK(f >= 1 && f <= H && f <= W, "patch_gather_backward: window f=%d does not fit %dx%d", f, H, W);
+    MARLC_CHECK(Na >= 0 && B >= 0 && C >= 1, "patch_gather_backward: bad shape (Na=%d, B=%d, C=%d)", Na, B, C);
+    MARLC_CHECK((long)C * H * W < 0x7fffffffl, "patch_gather_backward: one image must hold fewer than 2^31 elements");
+    MARLC_CHECK((long)Na * B < 0x7fffffffl, "patch_gather_backward: %d x %d windows", Na, B);
+    if (B == 0) return 0;
+    const unsigned tx = (W + GB_TW - 1) / GB_TW, ty = (H + GB_TH - 1) / GB_TH;
+    MARLC_CHECK(ty <= 65535 && B <= 65535, "patch_gather_backward: image batch %d x %d rows too large for the grid", B,
+                H);
+    patch_gather_backward_kernel<<<dim3(tx, ty, (unsigned)B), GB_THREADS, 0, s>>>(d_obs, pos, d_img, Na, B, C, H, W, f);
+    MARLC_LAUNCH_CHECK();
+    return 0;
+}
+
 // ---------------------------------------------------------------------------
 // K2 transition (environment.py:56-66, 128-150) in pure integer arithmetic:
 // the move is applied only if every dim stays inside (0 <= p+m, p+m+f < S).

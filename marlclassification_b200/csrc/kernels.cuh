@@ -12,6 +12,10 @@ int patch_gather_i32(const float* img, const int* pos, float* obs, int Na, int B
 int transition_i64(int64_t* pos, const int64_t* act, const int64_t* table, int nA, int M, int f, int H, int W,
                    float* npos, int* err, cudaStream_t s);
 int normalized_positions_i64(const int64_t* pos, float* out, int M, int H, int W, cudaStream_t s);
+// Adjoint of patch_gather_i64: d_img[b,c,y,x] = sum over a = 0..Na-1 whose window covers (y,x), in that order, of
+// d_obs[a,b,c,y-pos_y,x-pos_x]; every element of d_img written.
+int patch_gather_backward_i64(const float* d_obs, const int64_t* pos, float* d_img, int Na, int B, int C, int H, int W,
+                              int f, cudaStream_t s);
 
 struct EpisodeInitArgs {
     const int64_t* pos0;       // nullable: injected initial positions [M,2]
@@ -135,6 +139,15 @@ struct ImageGradArgs {
     int T, Na, B, C, H, W, f, cin, cout, ho;
 };
 int cnn_image_grad(const ImageGradArgs& a, cudaStream_t s);
+// Gradient on the M windows of one stand-alone step from their first-layer conv-output gradients: the
+// transposed convolution with W_0, window by window (no gather).
+struct PatchGradArgs {
+    const float* dY0;  // [M windows][ho*ho][cout] (cnn_dY0 of a T = 1 engine)
+    const float* w0;   // [cout][cin][3][3]
+    float* d_patch;    // out [M][C][f][f], every element written (0 in the channels c >= cin)
+    int M, C, f, cin, cout, ho;
+};
+int cnn_patch_grad(const PatchGradArgs& a, cudaStream_t s);
 
 // ---- loss.cu ------------------------------------------------------------------
 struct LossArgs {

@@ -238,6 +238,17 @@ class EpisodeEngine:
                                                      self._stream()))
         self.launches["backward"] = self._L.marlc_engine_last_launches(self._h)
 
+    def step_input_grad(self, d_patch: Optional[th.Tensor], d_npos: Optional[th.Tensor]) -> None:
+        """``marlc_model_step_input_grad``: the gradients the last ``model_step_backward`` leaves on its windows
+        (``d_patch`` f32 [na, nb, C, f, f]) and normalised positions (``d_npos`` f32 [na, nb, 2]), each None when
+        not wanted.  Call it right after ``model_step_backward`` and before the parameters change."""
+        f = self.cfg.f
+        for t, shape in ((d_patch, (self.na, self.nb, self.C, f, f)), (d_npos, (self.na, self.nb, 2))):
+            if t is not None and (tuple(t.shape) != shape or t.dtype != th.float32 or not t.is_contiguous()
+                                  or t.device != th.device(self.device)):
+                raise RuntimeError(f"step_input_grad: need a contiguous float32 {shape} tensor on {self.device}")
+        _lib.check(self._L.marlc_model_step_input_grad(self._h, _lib.ptr(d_patch), _lib.ptr(d_npos), self._stream()))
+
 
 def C_void_p():
     return ct.c_void_p()
@@ -348,7 +359,8 @@ class _StepFn(th.autograd.Function):
     backward = marlc_model_step_backward, which re-runs the step from the saved inputs (the next step-wise call
     of the geometry overwrites the workspace, so nothing but the inputs is kept) and then runs the engine's
     BPTT at T = 1 with the output gradients as its outer end.  Parameter gradients land in a fresh flat buffer
-    per call, handed to autograd as one view per parameter."""
+    per call, handed to autograd as one view per parameter.  With ``model.differentiable_step_inputs`` the
+    windows and positions may require grad too: their gradients come from ``marlc_model_step_input_grad``."""
 
     @staticmethod
     def forward(ctx, eng: EpisodeEngine, model, patch, msg, npos, h, c, hc, cc, *params):
@@ -375,6 +387,10 @@ class _StepFn(th.autograd.Function):
         flat = model.flat_params
         grads = th.empty_like(flat)
         eng.model_step_backward(patch, msg, npos, (h, c, hc, cc), d_out, d_in, grads)
+        d_patch = th.empty_like(patch) if need[2] else None
+        d_npos = th.empty_like(npos) if need[4] else None
+        if need[2] or need[4]:
+            eng.step_input_grad(d_patch, d_npos)
         # autograd adds each parameter gradient into param.grad in place: make sure param.grad is the parameter's
         # slot of model.flat_grads, so the bucket the fused Adam reads and param.grad stay one tensor.  After
         # zero_grad(set_to_none=True) param.grad is None: the slot starts from zero.  A gradient held outside
@@ -394,7 +410,7 @@ class _StepFn(th.autograd.Function):
                     slot.copy_(p.grad)
                 p.grad = slot
             out.append(grads[off: off + p.numel()].view(p.shape))
-        return (None, None, None, d_in[0], None, *d_in[1:], *out)
+        return (None, None, d_patch, d_in[0], d_npos, *d_in[1:], *out)
 
 
 def model_step(model, img_patch, msg_t, norm_pos, hidden):
@@ -412,10 +428,12 @@ def model_step(model, img_patch, msg_t, norm_pos, hidden):
         raise RuntimeError(f"img_patch window {f}x{f2} != model window {model.feature_extractor.cnn_spec[0]}")
     eng = get_engine(model, na=na, nb=nb, T=1, C=Cc, H=f + 1, W=f + 1, actions=[[0, 0]] * d["nb_action"], gamma=1.0)
     if th.is_grad_enabled() and getattr(model, "differentiable_steps", False):
-        for t, name in ((img_patch, "img_patch"), (norm_pos, "norm_pos")):
-            if t.requires_grad:
-                raise RuntimeError(f"ModelsWrapper.forward: {name} requires grad, but the step-wise backward computes "
-                                   f"no gradient for it; pass {name}.detach()")
+        if not getattr(model, "differentiable_step_inputs", False):
+            for t, name in ((img_patch, "img_patch"), (norm_pos, "norm_pos")):
+                if t.requires_grad:
+                    raise RuntimeError(f"ModelsWrapper.forward: {name} requires grad, but the step-wise backward "
+                                       f"computes no gradient for it; pass {name}.detach(), or set "
+                                       "model.differentiable_step_inputs = True to backpropagate into it")
         o = _StepFn.apply(eng, model, patch, msg, npos, *hid, *model.parameters())
         return ModelOutput(*o[:4]), RecurrentOutput(*o[4:])
     eng.model_step(patch, msg, npos, hid)

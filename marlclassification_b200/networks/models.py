@@ -92,6 +92,9 @@ class ModelsWrapper(nn.Module):
         # True: forward() / MultiAgent.act in grad mode carry a backward (engine.model_step); False: they are
         # forward-only and a backward() reaching them raises
         self.differentiable_steps = False
+        # True (with differentiable_steps): the step-wise backward also gives gradients to img_patch / norm_pos that
+        # require grad (pixel attribution, input optimisation with a hand-written loop); False: such inputs raise
+        self.differentiable_step_inputs = False
         self._param_updates = 0  # parameter writes torch cannot see (the fused Adam): see param_generation
 
     # ---- reference surface ------------------------------------------------------
@@ -117,9 +120,10 @@ class ModelsWrapper(nn.Module):
         self, img_patch: th.Tensor, msg_t: th.Tensor, norm_pos: th.Tensor, recurrent_hidden: RecurrentOutput
     ) -> tuple[ModelOutput, RecurrentOutput]:
         """One step of every network (models.py:78-138) on CUDA.  With ``differentiable_steps`` set, the
-        outputs carry a backward to every parameter, ``msg_t`` and ``recurrent_hidden`` (not to
-        ``img_patch`` / ``norm_pos``); otherwise this is forward-only and training goes through
-        EpisodeSampler.run_episode, whose outputs carry the hand-written BPTT backward."""
+        outputs carry a backward to every parameter, ``msg_t`` and ``recurrent_hidden``, and, with
+        ``differentiable_step_inputs`` set as well, to ``img_patch`` / ``norm_pos``; otherwise this is
+        forward-only and training goes through EpisodeSampler.run_episode, whose outputs carry the hand-written
+        BPTT backward."""
         from ..engine import model_step
 
         return model_step(self, img_patch, msg_t, norm_pos, recurrent_hidden)
