@@ -271,14 +271,9 @@ static int staged_floats(int maxw, int n1, int p1, int n2, int p2) {
     const size_t w = (size_t)n1 * p1 + (size_t)n2 * p2;
     return (chain_smem_bytes(maxw) + sizeof(float) * w <= CHAIN_SMEM_LIMIT) ? (int)w : 0;
 }
-// Weights resident in shared memory make ONE row block fast (no L2 round trips inside its dependent chain) but
-// cost 80-190 KB per CTA: one CTA = 4 rows per SM at a time.  With many row blocks per SM (sharded-batch
-// configurations: 1024 row blocks at 4096 rows) the latency of each chain is better hidden by running several
-// small CTAs per SM that read the weights through L1/L2.  Threshold in row blocks: MARLC_CHAIN_STAGE_MAX_RB.
-static bool stage_weights_for(int M) {
-    static const int max_rb = getenv("MARLC_CHAIN_STAGE_MAX_RB") ? atoi(getenv("MARLC_CHAIN_STAGE_MAX_RB")) : (1 << 30);
-    return (M + RB - 1) / RB <= max_rb;
-}
+// Weights are staged whenever they fit: resident in shared memory they make ONE row block fast (no L2 round trips
+// inside its dependent chain), at 80-190 KB per CTA (one CTA = 4 rows per SM at a time).  Wider layers read them
+// through L1/L2.
 static int maxw_of(std::initializer_list<int> v) {
     int m = 4;
     for (int x : v) m = max(m, x);
@@ -288,17 +283,17 @@ ChainStage step_pre_stage(int n_m, int n1, int n2, int nd) {
     const int maxw = maxw_of({n_m, n1, n2, nd});
     return {maxw, staged_floats(maxw, n1, odd_pitch(n_m), n2, odd_pitch(n1))};
 }
-ChainStage step_post_stage(int M, int n1, int n2) {
+ChainStage step_post_stage(int n1, int n2) {
     const int maxw = maxw_of({n1, n2});
-    return {maxw, stage_weights_for(M) ? staged_floats(maxw, n2, odd_pitch(n1), 0, 0) : 0};
+    return {maxw, staged_floats(maxw, n2, odd_pitch(n1), 0, 0)};
 }
-ChainStage bwd_pre_stage(int M, int n_m, int n1, int nb) {
+ChainStage bwd_pre_stage(int n_m, int n1, int nb) {
     const int maxw = maxw_of({n_m, n1, nb});
-    return {maxw, stage_weights_for(M) ? staged_floats(maxw, n_m, n1, n1, nb) : 0};
+    return {maxw, staged_floats(maxw, n_m, n1, n1, nb)};
 }
-ChainStage bwd_post_stage(int M, int n_m, int n1, int n2) {
+ChainStage bwd_post_stage(int n_m, int n1, int n2) {
     const int maxw = maxw_of({n_m, n1, n2});
-    return {maxw, stage_weights_for(M) ? staged_floats(maxw, n2, n1, n1, n_m) : 0};
+    return {maxw, staged_floats(maxw, n2, n1, n1, n_m)};
 }
 
 // ---------------------------------------------------------------------------------
@@ -431,23 +426,18 @@ static int persistent_blocks(int nrb, size_t smem_bytes, int waves = 1) {
 
 static int step_pre_small(const StepPreArgs& a, cudaStream_t s);
 
+constexpr int CNN_WIDE_MIN = 256;
 StepPrePlan step_pre_plan(const CnnDesc& d, bool have_img, bool have_wT, int M, CnnWidePlan* wide) {
     // feature extractor: one CTA per window while a step has few windows (latency-bound, every SM gets one:
-    // step_pre_kernel); from MARLC_CNN_WIDE_MIN windows on, persistent CTAs with stationary weights, 8 windows
+    // step_pre_kernel); from CNN_WIDE_MIN windows on, persistent CTAs with stationary weights, CW_NW windows
     // per pass, next to persistent decoder CTAs (step_pre_wide_kernel)
-    static const int wide_min = getenv("MARLC_CNN_WIDE_MIN") ? atoi(getenv("MARLC_CNN_WIDE_MIN")) : 256;
-    // 8 windows per pass; 4 (MARLC_CNN_WIDE_NW=4: twice the CTAs while 8 leave SMs idle) measured slower at
-    // 512 and 1024 windows (476 vs 438 us, 795 vs 745 us per 16 steps): a pass is bound by the latency of its
-    // phases, not by its FMA count
-    static const int nw_env = getenv("MARLC_CNN_WIDE_NW") ? atoi(getenv("MARLC_CNN_WIDE_NW")) : 0;
-    const int nw = nw_env ? nw_env : CW_NW;
     CnnWidePlan w;
     memset(&w, 0, sizeof(w));
-    if (M >= wide_min) w = cnn_wide_plan(d, have_img, have_wT, nw);
+    if (M >= CNN_WIDE_MIN) w = cnn_wide_plan(d, have_img, have_wT);
     if (wide) *wide = w;
     StepPrePlan p;
-    p.nw = w.ok ? nw : 1;
-    p.cnn_blocks = w.ok ? min((M + nw - 1) / nw, MARLC_SMS) : 0;
+    p.nw = w.ok ? CW_NW : 1;
+    p.cnn_blocks = w.ok ? min((M + CW_NW - 1) / CW_NW, MARLC_SMS) : 0;
     return p;
 }
 
@@ -474,10 +464,7 @@ int step_pre(const StepPreArgs& a, cudaStream_t s) {
     // (the launch's shared memory is the larger role's: one CTA per SM, so the decoder CTAs share the SMs with the
     //  feature extractor's in time; one wave of them)
     ka.dec_blocks = persistent_blocks((a.M + RB - 1) / RB, smem);
-    // profiling aid (WRONG results): time the feature-extractor role alone (1) / the decoder role alone (2)
-    static const int prof = getenv("MARLC_PROFILE_PRE_ROLE") ? atoi(getenv("MARLC_PROFILE_PRE_ROLE")) : 0;
-    if (prof == 2) ka.cnn_blocks = 0;
-    const int grid = ka.cnn_blocks + (prof == 1 ? 0 : ka.dec_blocks);
+    const int grid = ka.cnn_blocks + ka.dec_blocks;
     ka.trig = pdl_trigger_early();
     MARLC_CUDA(launch_pdl(step_pre_wide_kernel, dim3(grid), dim3(CT), smem, s, ka));
     MARLC_LAUNCH_CHECK();
@@ -799,7 +786,7 @@ int step_post(const StepPostArgs& a, cudaStream_t s) {
     MARLC_CHECK(a.act.nA <= MAX_ACT, "step_post: nb_action=%d > %d", a.act.nA, MAX_ACT);
     StepPostKernelArgs ka;
     ka.a = a;
-    const ChainStage st = step_post_stage(a.M, a.e3.n_in, a.e3.n_out);
+    const ChainStage st = step_post_stage(a.e3.n_in, a.e3.n_out);
     ka.maxw = st.maxw;
     ka.pol_blocks = (a.M + CT / 32 - 1) / (CT / 32);
     const int wfl = st.wfl;
@@ -1078,7 +1065,7 @@ int bwd_pre(const BwdPreArgs& a, cudaStream_t s) {
     if (a.M <= 0) return 0;
     BwdPreKernelArgs ka;
     ka.a = a;
-    const ChainStage st = bwd_pre_stage(a.M, a.n_m, a.e0.n_out, a.n[0]);
+    const ChainStage st = bwd_pre_stage(a.n_m, a.e0.n_out, a.n[0]);
     ka.maxw = st.maxw;
     const int wfl = st.wfl;
     ka.staged = wfl > 0;
@@ -1200,7 +1187,7 @@ int bwd_post(const BwdPostArgs& a, cudaStream_t s) {
     if (a.M <= 0) return 0;
     BwdPostKernelArgs ka;
     ka.a = a;
-    const ChainStage st = bwd_post_stage(a.M, a.n_m, a.d0.n_out, a.n_m_o);
+    const ChainStage st = bwd_post_stage(a.n_m, a.d0.n_out, a.n_m_o);
     ka.maxw = st.maxw;
     const int wfl = st.wfl;
     ka.staged = wfl > 0;

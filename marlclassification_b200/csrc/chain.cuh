@@ -108,8 +108,8 @@ StepPrePlan step_pre_plan(const CnnDesc& d, bool have_img, bool have_wT, int M, 
 // read through L1 / L2).
 struct ChainStage { int maxw, wfl; };
 ChainStage step_pre_stage(int n_m, int n1, int n2, int nd);
-ChainStage step_post_stage(int M, int n1, int n2);
-ChainStage bwd_pre_stage(int M, int n_m, int n1, int nb);
-ChainStage bwd_post_stage(int M, int n_m, int n1, int n2);
+ChainStage step_post_stage(int n1, int n2);
+ChainStage bwd_pre_stage(int n_m, int n1, int nb);
+ChainStage bwd_post_stage(int n_m, int n1, int n2);
 
 }  // namespace marlc

@@ -26,11 +26,7 @@ struct CnnBwdLayerKernelArgs {
     FastDiv d_npos, d_ho, d_co, d_kk, d_hon;  // index decompositions without runtime division
 };
 
-// MARLC_CNNBWD_DIV=1 selects the runtime-division instantiation (A/B timing only).
-static bool cnn_bwd_use_div() {
-    const char* e = getenv("MARLC_CNNBWD_DIV");
-    return e && e[0] == '1';
-}
+// FAST = false: runtime divisions, for sizes where FastDiv is not exact.
 #define MARLC_DIV(n, fd, d) (FAST ? (fd).div(n) : (n) / (d))
 
 template <bool FAST>
@@ -204,7 +200,7 @@ int cnn_bwd_layer(const CnnBwdLayerArgs& a, cudaStream_t s) {
     ka.d_hon = FastDiv((unsigned)std::max(a.ho_next, 1));
     // FastDiv exactness: the largest dividends are total (/ npos, / cout) and npn * kk (/ kk)
     const long nmax = std::max((long)ka.total, (long)ka.npn * a.cout * 9);
-    const bool fast = FastDiv::exact_up_to(nmax, std::max(std::max(ka.npos, a.cout * 9), 1)) && !cnn_bwd_use_div();
+    const bool fast = FastDiv::exact_up_to(nmax, std::max(std::max(ka.npos, a.cout * 9), 1));
     static size_t attr = 0;
     if (smem > 48 * 1024 && smem > attr) {
         MARLC_CUDA(cudaFuncSetAttribute(cnn_bwd_layer_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -245,7 +241,7 @@ int cnn_im2col_input(const CnnWindows& win, float* col, int P, int cin, int ho, 
     if (P <= 0) return 0;
     const int kkp = (cin * 9 + 3) & ~3;
     const FastDiv d_kk((unsigned)kkp), d_ho((unsigned)ho);
-    const bool fast = FastDiv::exact_up_to((long long)ho * ho * kkp, kkp) && !cnn_bwd_use_div();
+    const bool fast = FastDiv::exact_up_to((long long)ho * ho * kkp, kkp);
     const unsigned grid = (P * 32 + 255) / 256;
     if (win.patch) {
         if (fast) cnn_im2col_input_kernel<true, true><<<grid, 256, 0, s>>>(win, col, P, cin, ho, d_kk, d_ho);

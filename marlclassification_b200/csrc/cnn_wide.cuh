@@ -24,14 +24,15 @@
 
 namespace marlc {
 
-constexpr int CW_NW = 8;        // windows per pass (template parameter NW: 8; 4 exists for A/B runs, slower)
+// Windows per pass.  4 (twice the CTAs while 8 leave SMs idle) measured slower at 512 and 1024 windows (476 vs
+// 438 us, 795 vs 745 us per 16 steps): a pass is bound by the latency of its phases, not by its FMA count.
+constexpr int CW_NW = 8;
 constexpr int CW_THREADS = 256;  // = the chain kernels' CTA (step_pre hosts this role); 512 threads as a separate launch
                                  // measured no faster per batch and cost a fork / join per step
 constexpr int CW_MAX_KS = 8;
 
 struct CnnWidePlan {
     int ok;                          // 0: shapes not supported (caller uses the per-window block)
-    int nw;                          // windows per pass: 8 or 4
     int w_off[MAX_CNN_LAYERS];       // floats: transposed weights of layer l
     int p_off[MAX_CNN_LAYERS];       // bias | gamma | beta (3 * cout)
     int lut_off[MAX_CNN_LAYERS];     // per output element e = c * npos + pos: (c << 16) | position in the next layer's input
@@ -44,15 +45,11 @@ struct CnnWidePlan {
 
 // have_wT: the engine keeps transposed conv weights (d.wT, one buffer per layer; with the chain kernels).  A flag
 // rather than a test of d.wT[0], which is only set at bind, so that an engine's plan can be queried before.
-inline CnnWidePlan cnn_wide_plan(const CnnDesc& d, bool have_img, bool have_wT, int nw = CW_NW) {
+inline CnnWidePlan cnn_wide_plan(const CnnDesc& d, bool have_img, bool have_wT) {
+    constexpr int nw = CW_NW;
     CnnWidePlan p;
     memset(&p, 0, sizeof(p));
-    p.nw = nw;
-#ifdef MARLC_CW_NW4
-    if (!have_img || !have_wT || (nw != 8 && nw != 4)) return p;
-#else
-    if (!have_img || !have_wT || nw != 8) return p;
-#endif
+    if (!have_img || !have_wT) return p;
     int off = 0;
     for (int l = 0; l < d.L; ++l) {
         if ((d.cout[l] & 3) || d.groups[l] > 32 || d.cout[l] % d.groups[l]) return p;
@@ -442,11 +439,7 @@ __device__ __forceinline__ void cnn_fwd_wide_t(const CnnFwdArgs& a, const CnnWid
 // All CW_THREADS threads of CTA `cta` (of `n_cta` cooperating CTAs) must call.
 __device__ __forceinline__ void cnn_fwd_wide(const CnnFwdArgs& a, const CnnWidePlan& pl, const int cta, const int n_cta,
                                              float* sm) {
-#ifdef MARLC_CW_NW4  // A/B build: 4 windows per pass (measured slower); not compiled by default -- the second
-                     // instantiation doubles the role's code, and the kernel already runs close to the instruction cache
-    if (pl.nw == 4) { cnn_fwd_wide_t<4>(a, pl, cta, n_cta, sm); return; }
-#endif
-    cnn_fwd_wide_t<8>(a, pl, cta, n_cta, sm);
+    cnn_fwd_wide_t<CW_NW>(a, pl, cta, n_cta, sm);
 }
 
 }  // namespace marlc

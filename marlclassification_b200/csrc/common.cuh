@@ -53,7 +53,7 @@ extern long g_simt_gemm_launches, g_tc_gemm_launches;  // per GEMM back end (mar
 // of the current iteration) is read, and no global memory is written, before pdl_wait(); pdl_trigger() at
 // entry lets the NEXT kernel of the chain do the same.  g_pdl is set by the engine (PdlScope) only around
 // launches whose predecessor in the stream is a kernel of the same chain; everywhere else the launch is an
-// ordinary one and pdl_wait() returns immediately.  MARLC_PDL=0 switches the attribute off (A/B runs).
+// ordinary one and pdl_wait() returns immediately.  MARLC_PDL=0 switches the attribute off (to bisect a suspected ordering race).
 extern thread_local int g_pdl, g_pdl_trig;
 struct PdlScope {  // on: the launches inside are programmatic dependents; trig: they trigger THEIR dependents at entry
     int prev, prev_trig;
@@ -67,13 +67,9 @@ bool pdl_enabled();
 //   * BPTT sweep: an entry trigger makes every edge slower (+44 us for bwd_pre alone: the next kernel's CTAs pile
 //     onto the SMs the running kernel leaves free and start unevenly); without an explicit trigger (dependents
 //     launch when the last CTA exits, skipping only the drain) the three edges gain 26 us.
-// A/B switches: MARLC_PDL_MASK selects the edges (bit per consumer kernel: 1 step_pre, 2 LSTM pair, 4 block-0 GEMMs,
-// 8 step_post, 16 bwd_pre, 32 input-gradient GEMMs, 64 bwd_post; default 125); MARLC_PDL_TRIG: bit 0 = entry
-// trigger in the forward chain, bit 1 = in the sweep (default 1).
-enum { PDL_STEP_PRE = 1, PDL_LSTM = 2, PDL_G0 = 4, PDL_STEP_POST = 8, PDL_BWD_PRE = 16, PDL_DX = 32, PDL_BWD_POST = 64 };
-int pdl_edge(int bit);   // 1 if that edge is enabled
+// So every PdlScope of the engine makes its launches dependents except the LSTM pair's, and only the forward chain's
+// scopes set the entry trigger.
 int pdl_trigger_early(); // value for the kernels' `trig` argument (from the enclosing PdlScope)
-int pdl_trig_mode(int bwd);  // MARLC_PDL_TRIG bit for the forward chain (0) / the sweep (1)
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 // Launch `kern(arg)`; with g_pdl set (and PDL enabled) as a programmatic dependent of the previous kernel in `s`.

@@ -27,19 +27,11 @@ void set_error(const char* fmt, ...) {
     vsnprintf(g_err, sizeof(g_err), fmt, ap);
     va_end(ap);
 }
-// programmatic dependent launch: state and A/B switches (common.cuh)
+// programmatic dependent launch: state and the MARLC_PDL switch (common.cuh)
 thread_local int g_pdl = 0, g_pdl_trig = 0;
 bool pdl_enabled() {
     static const bool on = !(getenv("MARLC_PDL") && atoi(getenv("MARLC_PDL")) == 0);
     return on;
-}
-int pdl_edge(int bit) {
-    static const int mask = getenv("MARLC_PDL_MASK") ? atoi(getenv("MARLC_PDL_MASK")) : 125;
-    return (mask & bit) ? 1 : 0;
-}
-int pdl_trig_mode(int bwd) {
-    static const int t = getenv("MARLC_PDL_TRIG") ? atoi(getenv("MARLC_PDL_TRIG")) : 1;
-    return (t >> (bwd ? 1 : 0)) & 1;
 }
 int pdl_trigger_early() { return g_pdl_trig; }
 
@@ -86,11 +78,7 @@ struct marlc_engine {
     int debug_stop = 0;
     // fork/join plumbing for independent branches (works eagerly and under stream capture)
     cudaStream_t side[2] = {nullptr, nullptr};
-    cudaStream_t hp = nullptr;  // highest priority: the latency-bound BPTT sweep, while batched gradients fill the GPU
-    // time-step chunks of the batched gradients; chunks > 1 overlap the sweep (MARLC_BWD_CHUNKS).  Measured at C2:
-    // 1, 2 and 4 chunks take the same time (the overlapped launches delay the sweep as much as they save), 8 is
-    // slower, so the default is one chunk after the sweep.
-    int bwd_chunks = 1;
+    cudaStream_t hp = nullptr;  // highest priority: the latency-bound BPTT sweep
     // Whose first-layer conv-output gradients cnn_dY0 holds: those of the last rollout after a complete
     // marlc_episode_backward (read by marlc_episode_image_grad), those of a stand-alone step after a complete
     // marlc_model_step_backward (read by marlc_model_step_input_grad), or neither: every forward, model step and
@@ -409,7 +397,6 @@ extern "C" int marlc_engine_bind(marlc_engine* e, void* workspace, float* params
         int least = 0, greatest = 0;
         MARLC_CUDA(cudaDeviceGetStreamPriorityRange(&least, &greatest));
         MARLC_CUDA(cudaStreamCreateWithPriority(&e->hp, cudaStreamNonBlocking, greatest));
-        if (const char* env = getenv("MARLC_BWD_CHUNKS")) e->bwd_chunks = std::max(1, atoi(env));
         for (int i = 0; i < 64; ++i) {
             MARLC_CUDA(cudaEventCreateWithFlags(&e->ev[i], cudaEventDisableTiming));
             e->n_ev = i + 1;
@@ -486,11 +473,9 @@ static bool lstm_on_tc(const marlc_engine* e) {
 // Fused chain kernels for the sweep while a step has fewer than 4096 rows (latency-bound: 3 launches per step).
 // From 4096 rows per step on (config 4 on ONE GPU) the one-kernel-per-op sweep with its products on the
 // tensor cores wins: the chains run 4 rows per CTA, one CTA per SM.  Measured (sweep of 16 steps): 4096 rows
-// 2.72 vs 3.01 ms, 2048 rows 2.91 vs 2.48 ms -- hence the threshold (MARLC_SWEEP_UNFUSED_MIN_M).
-static bool sweep_chained(const marlc_engine* e) {
-    static const int unfused_min_m = getenv("MARLC_SWEEP_UNFUSED_MIN_M") ? atoi(getenv("MARLC_SWEEP_UNFUSED_MIN_M")) : 4096;
-    return e->cfg.use_chains && e->M < unfused_min_m;
-}
+// 2.72 vs 3.01 ms, 2048 rows 2.91 vs 2.48 ms -- hence the threshold.
+constexpr int SWEEP_UNFUSED_MIN_M = 4096;
+static bool sweep_chained(const marlc_engine* e) { return e->cfg.use_chains && e->M < SWEEP_UNFUSED_MIN_M; }
 
 extern "C" int marlc_engine_plan(const marlc_engine* e, marlc_plan* out) {
     MARLC_CHECK(e && out, "plan: null argument");
@@ -515,11 +500,11 @@ extern "C" int marlc_engine_plan(const marlc_engine* e, marlc_plan* out) {
     p.sweep_chained = sweep_chained(e);
     if (c.use_chains) {
         p.staged_step_pre = step_pre_stage(c.n_m, 2 * c.n_m, c.n_m_o, c.n_d).wfl > 0;
-        p.staged_step_post = step_post_stage(M, 2 * c.n_m, c.n_m).wfl > 0;
+        p.staged_step_post = step_post_stage(2 * c.n_m, c.n_m).wfl > 0;
     }
     if (p.sweep_chained) {
-        p.staged_bwd_pre = bwd_pre_stage(M, c.n_m, 2 * c.n_m, c.n_b).wfl > 0;
-        p.staged_bwd_post = bwd_post_stage(M, c.n_m, 2 * c.n_m, c.n_m_o).wfl > 0;
+        p.staged_bwd_pre = bwd_pre_stage(c.n_m, 2 * c.n_m, c.n_b).wfl > 0;
+        p.staged_bwd_post = bwd_post_stage(c.n_m, 2 * c.n_m, c.n_m_o).wfl > 0;
     }
     *out = p;
     return 0;
@@ -648,7 +633,7 @@ static int step_networks(marlc_engine* e, int t, const float* img, const int* po
         pa.pos_y = e->buf("pos_y") + (size_t)t * M * c.n_d;
         pa.U = Ut; pa.ldu = Kin; pa.F = F; pa.Na = c.na; pa.Nb = c.nb; pa.M = M;
         {
-            PdlScope pdl_first(pdl >= 2 && pdl_edge(PDL_STEP_PRE), pdl >= 1 && pdl_trig_mode(0));
+            PdlScope pdl_first(pdl >= 2, pdl >= 1);
             MARLC_TRY(step_pre(pa, s));
         }
         if (e->debug_stop == 11) return 0;
@@ -698,12 +683,10 @@ static int step_networks(marlc_engine* e, int t, const float* img, const int* po
                 TcLstmArgs& a = la[k];
                 a.U.lo = e->lo_on ? e->buf("U_lo") : nullptr;
                 a.Hprev.lo = e->lo_of(a.Hprev.ptr);
-                static const int a_lo = getenv("MARLC_LSTM_A_LO") ? atoi(getenv("MARLC_LSTM_A_LO")) : 1;  // A/B toggle
-                if (!a_lo) { a.U.lo = nullptr; a.Hprev.lo = nullptr; }  // activations' lo part split in-kernel
                 a.Wih_lo = e->lo_of(a.Wih); a.Whh_lo = e->lo_of(a.Whh);
                 a.h_new_lo = const_cast<float*>(e->lo_of(a.h_new));
             }
-            PdlScope pdl_lstm(pdl_rest && pdl_edge(PDL_LSTM), pdl_rest && pdl_trig_mode(0));
+            PdlScope pdl_lstm(0, pdl_rest);  // an ordinary launch: as a dependent it was slower (common.cuh)
             MARLC_TRY(tc_lstm_pair(la[0], la[1], s));
         }
     }
@@ -749,7 +732,7 @@ static int step_networks(marlc_engine* e, int t, const float* img, const int* po
             g[0].allow_split = g[1].allow_split = 2;
             g[0].c_zeroed = g[1].c_zeroed = 1;
             if (tc_operand_ok(g[0].A) && tc_operand_ok(g[0].B) && tc_operand_ok(g[1].A) && tc_operand_ok(g[1].B)) {
-                PdlScope pdl_g0(pdl_rest && pdl_edge(PDL_G0), pdl_rest && pdl_trig_mode(0));
+                PdlScope pdl_g0(pdl_rest, pdl_rest);
                 MARLC_TRY(tc_gemm_group(g, 2, s));
                 grouped = true;
             }
@@ -877,7 +860,7 @@ extern "C" int marlc_episode_forward(marlc_engine* e, const float* img, const in
                                 npos + (size_t)t * M * 2, H + (size_t)t * M * c.n_b, Cb + (size_t)t * M * c.n_b,
                                 Hc + (size_t)t * M * c.n_a, Cc + (size_t)t * M * c.n_a, s, t > 0 ? 2 : 1));
         if (e->debug_stop >= 11 && e->debug_stop <= 13) continue;  // profiling: skip the tail
-        PdlScope pdl_post(c.use_chains && pdl_edge(PDL_STEP_POST), c.use_chains && pdl_trig_mode(0));
+        PdlScope pdl_post(c.use_chains, c.use_chains);
         MARLC_TRY(step_act(e, t, actions ? actions + (size_t)t * M : nullptr, s));
     }
     if (e->debug_stop >= 11 && e->debug_stop <= 14) { e->last_launches = g_launch_count - start; return 0; }
@@ -1097,9 +1080,10 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
     if (e->debug_stop == 1) { MARLC_TRY(join_sides()); e->last_launches = g_launch_count - start; return 0; }
     // ---- weight gradients of steps [t0, t1), batched over their (t1-t0)*M rows (the reduction
     //      dimension).  Three independent branches on three streams: LSTM (sL) | encoder / decoder /
-    //      position features (s1) | feature extractor (s0).  Nothing here feeds the sweep, so with the
-    //      fused chains the sweep runs on the high-priority stream and these launches fill the GPU
-    //      underneath it, one chunk of time steps behind.
+    //      position features (s1) | feature extractor (s0).  With the fused chains they run once the
+    //      sweep (high-priority stream) is done.  Overlapping them with the sweep in chunks of time steps
+    //      was measured at C2: 2 and 4 chunks take the same time (the overlapped launches delay the sweep
+    //      as much as they save), 8 are slower.
     const bool par = c.use_chains != 0;
     auto batched = [&](int t0, int t1, cudaStream_t sL, cudaStream_t s1, cudaStream_t s0) -> int {
         NvtxRange nvtx_batched("marlc/backward/batched_grads");
@@ -1241,10 +1225,8 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
         MARLC_CUDA(cudaMemsetAsync(dhc_hist, 0, sizeof(float) * (size_t)TM * c.n_a, s));
         // the sweep moves to the high-priority stream; the caller's stream becomes the LSTM branch
         const bool profiling_stop = e->debug_stop == 2 || e->debug_stop == 21 || e->debug_stop == 22;
-        const int nch = profiling_stop ? 0 : std::max(1, std::min(e->bwd_chunks, T));
         cudaStream_t sw = e->hp, s0 = e->side[0], s1 = e->side[1];
         MARLC_TRY(e->chain(s, sw));
-        int chunk_hi = T, next_chunk = nch - 1;  // chunk k covers steps [k*T/nch, (k+1)*T/nch)
         for (int t = T - 1; t >= 0; --t) {
             float* dgb = e->buf("dgates_b") + (size_t)t * M * 4 * c.n_b;
             float* dga = e->buf("dgates_a") + (size_t)t * M * 4 * c.n_a;
@@ -1279,7 +1261,7 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
             bp.n[0] = c.n_b; bp.n[1] = c.n_a;
             bp.Na = c.na; bp.Nb = c.nb; bp.M = M; bp.n_m = c.n_m;
             {
-                PdlScope pdl(t < T - 1 && pdl_edge(PDL_BWD_PRE), pdl_trig_mode(1));  // predecessor in `sw`: bwd_post of step t+1 (an event wait at t = T-1)
+                PdlScope pdl(t < T - 1);  // predecessor in `sw`: bwd_post of step t+1 (an event wait at t = T-1)
                 MARLC_TRY(bwd_pre(bp, sw));
             }
             cur ^= 1;
@@ -1305,7 +1287,7 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
                 }
                 ok = ok && tc_operand_ok(g[0].A2) && tc_operand_ok(g[0].B2);
                 if (ok) {
-                    PdlScope pdl(pdl_edge(PDL_DX), pdl_trig_mode(1));
+                    PdlScope pdl(1);
                     MARLC_TRY(tc_gemm_group(g, t > 0 || want_dh0 ? 3 : 1, sw));  // at t == 0 only a step's caller consumes dh / dh^
                     tc_dx = true;
                 }
@@ -1353,19 +1335,17 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
             bq.dcoll = (t > 0 || want_dmsg0) ? dcoll : nullptr;
             bq.M = M; bq.n_m = c.n_m; bq.n_m_o = c.n_m_o;
             {
-                PdlScope pdl(pdl_edge(PDL_BWD_POST), pdl_trig_mode(1));
+                PdlScope pdl(1);
                 MARLC_TRY(bwd_post(bq, sw));
             }
-            if (next_chunk >= 0 && t == (int)((long)next_chunk * T / nch)) {  // steps [t, chunk_hi) are final
-                cudaEvent_t done = e->next_event();
-                MARLC_CUDA(cudaEventRecord(done, sw));
-                MARLC_CUDA(cudaStreamWaitEvent(s, done, 0));
-                MARLC_CUDA(cudaStreamWaitEvent(s0, done, 0));
-                MARLC_CUDA(cudaStreamWaitEvent(s1, done, 0));
-                MARLC_TRY(batched(t, chunk_hi, s, s1, s0));
-                chunk_hi = t;
-                --next_chunk;
-            }
+        }
+        if (!profiling_stop) {  // every step's gradients are final
+            cudaEvent_t done = e->next_event();
+            MARLC_CUDA(cudaEventRecord(done, sw));
+            MARLC_CUDA(cudaStreamWaitEvent(s, done, 0));
+            MARLC_CUDA(cudaStreamWaitEvent(s0, done, 0));
+            MARLC_CUDA(cudaStreamWaitEvent(s1, done, 0));
+            MARLC_TRY(batched(0, T, s, s1, s0));
         }
         MARLC_TRY(e->chain(sw, s));
     } else

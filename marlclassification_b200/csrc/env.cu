@@ -53,12 +53,6 @@ patch_gather_kernel(const float* __restrict__ img, const PosT* __restrict__ pos,
     }
 }
 
-// MARLC_GATHER_DIV=1 selects the runtime-division body (kept for A/B timing, scripts/gather_ab.py).
-static bool gather_use_div() {
-    const char* e = getenv("MARLC_GATHER_DIV");
-    return e && e[0] == '1';
-}
-
 template <typename PosT>
 static int patch_gather_t(const float* img, const PosT* pos, float* obs, int Na, int B, int C, int H, int W, int f,
                           cudaStream_t s) {
@@ -68,7 +62,7 @@ static int patch_gather_t(const float* img, const PosT* pos, float* obs, int Na,
     const int blocks = (M + 7) / 8;  // 8 warps = 8 windows per CTA
     const long ff = (long)f * f, total = (long)C * ff;
     MARLC_CHECK((long)C * H * W < 0x7fffffffl, "patch_gather: one image must hold fewer than 2^31 elements");
-    const bool fast = f >= 2 && FastDiv::exact_up_to(total, ff) && !gather_use_div();
+    const bool fast = f >= 2 && FastDiv::exact_up_to(total, ff);
     const FastDiv dff((unsigned)max(ff, 2l)), df((unsigned)max(f, 2));
 #define MARLC_GATHER_LAUNCH(U, F) \
     patch_gather_kernel<PosT, U, F><<<blocks, 256, 0, s>>>(img, pos, obs, Na, B, C, H, W, f, dff, df)

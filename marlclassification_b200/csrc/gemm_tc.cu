@@ -119,26 +119,6 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, u
         ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
         : "memory");
 }
-__device__ __forceinline__ void tma_load_3d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2,
-                                               uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5}], [%2], %6;"
-        ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(mask)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                     smem_u32(bar)), "h"(mask) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_rank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                  : "memory");
@@ -208,8 +188,6 @@ struct TcKernelParams {
     CUtensorMap a1l, b1l, a2l, b2l;
     CUtensorMap cmap;            // EPI_STORE: C as [M rows][N cols], box 32 x 32, 128B swizzle (TMA store / reduce)
     int c_tma;                   // 1: cmap is valid (C 16-byte aligned, ldc % 4 == 0)
-    int cluster;                 // EPI_LSTM: CTAs along x that share the A tile through TMA multicast (1 = off);
-                                 // the A maps then have box rows BM / cluster
     int ksplit;                  // EPI_LSTM: 2 = a pair of CTAs (cluster of 2 along x) splits K; the odd CTA ships its
                                  // partial accumulators into the even CTA's shared memory (DSMEM) before the cell
     int a_lo_g, b_lo_g;          // 1: the lo part of A / B comes from global memory
@@ -229,7 +207,6 @@ struct TcKernelParams {
     float* h_new_lo;  // optional: lo part of h_new for the next consumer's pre-split A operand
     float* gates;
     int n_hidden;
-    int epi_staged;   // EPI_LSTM: cell outputs leave through a shared-memory transpose (row-coalesced stores)
 };
 constexpr int TC_MAX_GROUP = 3;
 struct TcKernelGroup {  // up to 3 independent problems in one launch; blockIdx.z -> (problem, K split)
@@ -280,9 +257,6 @@ __device__ __forceinline__ void tc_gemm_body(const TcKernelGroup& pp, const int 
 
     const TcKernelParams& p = pp.p[PI];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int cl = (EPI == EPI_LSTM && p.cluster > 1) ? p.cluster : 1;
-    const uint16_t cl_mask = (uint16_t)((1u << cl) - 1u);
-    const uint32_t cl_rank = cl > 1 ? cluster_rank() : 0u;
 #ifdef MARLC_TC_TRACE  // in-kernel timeline of CTA (0,0,0): cycles since entry at each pipeline event
     __shared__ long long trace[12];
     const bool tr = blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0;
@@ -322,9 +296,7 @@ __device__ __forceinline__ void tc_gemm_body(const TcKernelGroup& pp, const int 
     }
     if (threadIdx.x == 32) {
         for (int s = 0; s < stages; ++s) {
-            // with A multicast a slot is refilled by every CTA of the cluster, so it is free only when
-            // ALL of them have consumed it: every MMA warp arrives on every CTA's empty barrier
-            mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], cl);
+            mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1);
             mbar_init(&split_bar[s], TC_SPLITTERS / TC_SPLIT_GROUPS(STAGES));  // one splitter group per slot
         }
         mbar_init(&tmem_full_bar, 1);
@@ -337,7 +309,6 @@ __device__ __forceinline__ void tc_gemm_body(const TcKernelGroup& pp, const int 
     }
     tc_fence_before();
     __syncthreads();
-    if (cl > 1) cluster_sync_all();  // every CTA's barriers exist before any peer multicasts into them
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_smem;
     // Everything above touched only the kernel parameters and this CTA's shared memory / TMEM.  From here on the
@@ -379,10 +350,7 @@ __device__ __forceinline__ void tc_gemm_body(const TcKernelGroup& pp, const int 
                     uint8_t* a_dst = sA + s * S::A_BYTES + sub * S::A_SUB + hl * LO_OFF;
                     uint8_t* b_dst = sB + s * S::B_BYTES + sub * S::B_SUB + hl * LO_OFF;
                     if (do_a) {
-                        if (!A_MN && cl > 1) {  // this CTA fetches rows [rank*BM/cl, +BM/cl) for the whole cluster
-                            const int rows = BM / cl;
-                            tma_load_3d_mc(a_dst + cl_rank * rows * 128, ma, &full_bar[s], k0, m0 + (int)cl_rank * rows, za, cl_mask);
-                        } else if (!A_MN) tma_load_3d(a_dst, ma, &full_bar[s], k0, m0, za);
+                        if (!A_MN) tma_load_3d(a_dst, ma, &full_bar[s], k0, m0, za);
                         else
                             for (int j = 0; j < BM / 32; ++j) tma_load_3d(a_dst + j * 4096, ma, &full_bar[s], m0 + 32 * j, k0, za);
                     }
@@ -434,8 +402,7 @@ __device__ __forceinline__ void tc_gemm_body(const TcKernelGroup& pp, const int 
                     }
                 }
                 }
-                if (cl > 1) umma_commit_mc(&empty_bar[s], cl_mask);
-                else umma_commit(&empty_bar[s]);  // frees the smem slot once these MMAs retire
+                umma_commit(&empty_bar[s]);  // frees the smem slot once these MMAs retire
             }
             umma_commit(&tmem_full_bar);
             TC_TRACE(3);  // last MMA issued
@@ -454,7 +421,7 @@ __device__ __forceinline__ void tc_gemm_body(const TcKernelGroup& pp, const int 
         // of 8 units take ~1 750 cycles for a warp that runs alone on its scheduler (dependent MUFU chains: in-kernel
         // trace, round 2) -- 14 000 of the 22 500-cycle epilogue of a 128 x 256 tile; two warps per scheduler overlap them.
         constexpr int HU_E = BN / 4;
-        const bool epi8 = EPI == EPI_LSTM && X3 && HU_E >= 32 && ksp == 1 && p.a_lo_g && p.b_lo_g && p.epi_staged != 0;
+        const bool epi8 = EPI == EPI_LSTM && X3 && HU_E >= 32 && ksp == 1 && p.a_lo_g && p.b_lo_g;
         const bool epi_warp = warp < 6 || epi8;
         const int jb_begin = (epi8 && warp >= 6) ? HU_E / 2 : 0;
         const int jb_end = epi8 ? (warp >= 6 ? HU_E : HU_E / 2) : HU_E;
@@ -708,7 +675,7 @@ __device__ __forceinline__ void tc_gemm_body(const TcKernelGroup& pp, const int 
             constexpr int SP = CH + 4;             // staging row pitch: conflict-free 128-bit row-per-lane writes
             constexpr int LPR = CH / 4, RPI = 32 / LPR;  // lanes per row / rows per store instruction on the way out
             static_assert(EPI != EPI_LSTM || NEW * 7 * 32 * SP * 4 <= S::BYTES - 1024, "cell staging does not fit in the ring");
-            const bool staged = ksp == 1 && p.epi_staged != 0;
+            const bool staged = ksp == 1;
             float* stg = reinterpret_cast<float*>(smem) + (warp - 2) * (7 * 32 * SP);  // [7 arrays][32 rows][SP] of this warp
             if (ksp == 1 || kslice == 0) {
 #pragma unroll 1
@@ -833,7 +800,6 @@ __device__ __forceinline__ void tc_gemm_body(const TcKernelGroup& pp, const int 
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS));
     }
-    if (cl > 1) cluster_sync_all();  // no CTA may exit while a peer can still signal its barriers
 }
 
 template <int BN, bool A_MN, bool B_MN, int EPI, int STAGES, bool X3, int KS>
@@ -858,7 +824,7 @@ template <int BN, bool A_MN, bool B_MN, bool X3, int KS>
 static int launch_store(TcKernelGroup& kp, int gx, int gy, int gz, int max_kb, cudaStream_t s) {
     (void)max_kb;
     // KS == 1: <= 96 KB per CTA, two CTAs per SM (epilogue / main loop overlap); fat stages: 2-deep ring
-    constexpr int STAGES = BN >= 256 ? (X3 ? 2 : 4) : (KS > 1 ? 2 : (BN >= 128 ? 3 : 4));
+    constexpr int STAGES = KS > 1 ? 2 : (BN >= 128 ? 3 : 4);
     using S = TcSmem<BN, STAGES, X3, KS>;
     static_assert(S::BYTES <= 227 * 1024, "tile configuration exceeds shared memory");
     auto kern = tc_gemm_kernel<BN, A_MN, B_MN, EPI_STORE, STAGES, X3, KS>;
@@ -877,9 +843,16 @@ static int launch_store(TcKernelGroup& kp, int gx, int gy, int gz, int max_kb, c
 // Tile width for a launch of `count` problems: narrow tiles keep small launches spread over the SMs,
 // 128-wide tiles halve the operand bytes per flop once there is a wave of CTAs anyway.  K splits count as
 // CTAs (weight gradients: few output tiles, reductions of 10^4..10^6 rows cut into TC_MAX_CHAIN chains).
+// The per-step input-gradient group (du | dh | dh^) is bound by the chip-wide L2 -> SM throughput: every tile
+// re-streams its K range, so 128-wide tiles (split-K restores the CTA count) move a third fewer bytes.  Measured
+// per 16 steps: 512 rows 320 -> 238 us, 1024 rows 590 -> 418 us, 128 rows 180 -> 181 us (kept at 64 there).
+constexpr int TC_DX128_MIN_CTAS = 16;
+// Weight gradients (MN-major x MN-major, reductions of 10^4.. rows cut into chains) stay at 128 wide.  128 x 256
+// tiles would read A once per 256 output columns instead of once per 128 (dW_ih at 65 536 rows: 1.58 -> 1.31 GB per
+// cell), but MEASURED SLOWER (backward at c4: 8.14 vs 7.99 ms): the 96 KB stages leave room for a 2-deep ring only.
+// (The 128-wide MN/MN variant once exposed a phase-aliasing bug of the operand splitter with odd ring depths --
+//  fixed in tc_gemm_body, see the comment there.)
 static int pick_bn(const TcGemmArgs* args, int count) {
-    // (measured per iteration with / without: 512 rows per step 2415 vs 2515 us, 1024 rows 4002 vs 4068, 128 rows 1563 vs 1576)
-    static const int dw_split_potential = getenv("MARLC_TC_DW_SPLIT_POTENTIAL") ? atoi(getenv("MARLC_TC_DW_SPLIT_POTENTIAL")) : 1;
     int max_n = 0;
     long ctas128 = 0;
     for (int i = 0; i < count; ++i) {
@@ -887,38 +860,13 @@ static int pick_bn(const TcGemmArgs* args, int count) {
         max_n = max(max_n, a.N);
         long chains = a.allow_split ? max(1L, ((long)a.K + a.K2 + TC_MAX_CHAIN - 1) / TC_MAX_CHAIN) : 1L;
         // weight gradients: split-K (>= 4 K blocks of 32 per split) restores the CTA count of wide tiles
-        if (dw_split_potential && a.allow_split == 1 && a.A.mn_major && a.B.mn_major) chains = max(chains, ((long)a.K + a.K2) / 128);
+        // (measured per iteration with / without: 512 rows per step 2415 vs 2515 us, 1024 rows 4002 vs 4068, 128 rows 1563 vs 1576)
+        if (a.allow_split == 1 && a.A.mn_major && a.B.mn_major) chains = max(chains, ((long)a.K + a.K2) / 128);
         ctas128 += (long)((a.M + BM - 1) / BM) * ((a.N + 127) / 128) * chains;
     }
-    static const int bn_cap = getenv("MARLC_TC_BN_MAX") ? atoi(getenv("MARLC_TC_BN_MAX")) : 128;  // A/B toggles
-    // (A/B toggles.  The 128-wide MN/MN weight-gradient variant exposed a phase-aliasing bug of the operand
-    //  splitter with odd ring depths -- fixed in tc_gemm_body, see the comment there.)
-    static const int dw128 = getenv("MARLC_TC_BN128_DW") ? atoi(getenv("MARLC_TC_BN128_DW")) : 1;
-    static const int dx128 = getenv("MARLC_TC_BN128_DX") ? atoi(getenv("MARLC_TC_BN128_DX")) : 1;
-    // The per-step input-gradient group (du | dh | dh^) is bound by the chip-wide L2 -> SM throughput: every tile
-    // re-streams its K range, so 128-wide tiles (split-K restores the CTA count) move a third fewer bytes.  Measured
-    // per 16 steps: 512 rows 320 -> 238 us, 1024 rows 590 -> 418 us, 128 rows 180 -> 181 us (kept at 64 there).
-    static const int dx_min_ctas = getenv("MARLC_TC_DX128_MIN_CTAS") ? atoi(getenv("MARLC_TC_DX128_MIN_CTAS")) : 16;
     if (max_n <= 32) return 32;
     const bool dx_group = !args[0].A.mn_major && args[0].B.mn_major && count > 1;  // per-step input-gradient group
-    if (max_n <= 64 || ctas128 < (dx_group ? dx_min_ctas : MARLC_SMS / 2) || bn_cap < 128) return 64;
-    if (!dw128 && args[0].A.mn_major && args[0].B.mn_major) return 64;
-    if (!dx128 && !args[0].A.mn_major && args[0].B.mn_major && count > 1) return 64;
-    // Weight gradients (MN-major x MN-major, reductions of 10^4.. rows cut into chains): the launch is bound by the
-    // chip-wide L2 -> SM throughput (~6300 B/clk), every output tile re-streams its K range of both operands --
-    // 128 x 256 tiles read A once per 256 output columns instead of once per 128 (dW_ih at 65 536 rows: 1.58 ->
-    // 1.31 GB per cell).  MEASURED SLOWER (backward at c4: 8.14 vs 7.99 ms): the 96 KB stages leave room for a
-    // 2-deep ring only.  Off; MARLC_TC_BN256_DW=1 selects it.
-    static const int dw256 = getenv("MARLC_TC_BN256_DW") ? atoi(getenv("MARLC_TC_BN256_DW")) : 0;
-    if (dw256 && args[0].A.mn_major && args[0].B.mn_major && max_n > 128) {
-        long ctas256 = 0;
-        for (int i = 0; i < count; ++i) {
-            const TcGemmArgs& a = args[i];
-            const long chains = a.allow_split ? max(1L, ((long)a.K + a.K2 + TC_MAX_CHAIN - 1) / TC_MAX_CHAIN) : 1L;
-            ctas256 += (long)((a.M + BM - 1) / BM) * ((a.N + 255) / 256) * chains;
-        }
-        if (ctas256 >= MARLC_SMS) return 256;
-    }
+    if (max_n <= 64 || ctas128 < (dx_group ? TC_DX128_MIN_CTAS : MARLC_SMS / 2)) return 64;
     return 128;
 }
 
@@ -969,8 +917,7 @@ int tc_gemm_group(const TcGemmArgs* args, int count, cudaStream_t s) {
         }
         p.M = a.M; p.N = a.N; p.C = a.C; p.ldc = a.ldc; p.bias = a.bias; p.bias2 = a.bias2;
         p.accumulate = a.accumulate;
-        static const int no_ctma = getenv("MARLC_TC_NO_CTMA") ? atoi(getenv("MARLC_TC_NO_CTMA")) : 0;  // A/B toggle
-        p.c_tma = (!no_ctma && (a.ldc & 3) == 0 && ((uintptr_t)a.C & 15) == 0) ? 1 : 0;
+        p.c_tma = ((a.ldc & 3) == 0 && ((uintptr_t)a.C & 15) == 0) ? 1 : 0;
         if (p.c_tma) MARLC_TRY(make_map_c(&p.cmap, a.C, a.M, a.N, a.ldc));
         const int mt = (a.M + BM - 1) / BM, nt = (a.N + BN - 1) / BN, nkb = p.nk1 + p.nk2;
         int splits = 1;
@@ -1024,10 +971,6 @@ int tc_gemm_group(const TcGemmArgs* args, int count, cudaStream_t s) {
     else { DISPATCH3(BNv, false, KSv) }
     if (BN == 32) { if (KS == 2) { DISPATCH(32, 2) } DISPATCH(32, 1) }
     if (BN == 64) { if (KS == 2) { DISPATCH(64, 2) } DISPATCH(64, 1) }
-    if (BN == 256) {  // weight gradients only (pick_bn)
-        if (x3) return launch_store<256, true, true, true, 1>(kp, gx, gy, gz, max_kb, s);
-        return launch_store<256, true, true, false, 1>(kp, gx, gy, gz, max_kb, s);
-    }
     DISPATCH(128, 1)
 #undef DISPATCH
 #undef DISPATCH3
@@ -1047,8 +990,7 @@ static int launch_lstm(TcKernelGroup& kp, int gx, int gy, int nkb, cudaStream_t 
         MARLC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::BYTES));
         attr_done = true;
     }
-    const int ksp = kp.p[0].ksplit > 1 ? kp.p[0].ksplit : 1;
-    const int cl = ksp > 1 ? ksp : kp.p[0].cluster;
+    const int ksp = kp.p[0].ksplit > 1 ? kp.p[0].ksplit : 1;  // a K-split pair runs as a cluster of ksp CTAs
     const size_t smem_bytes = S::BYTES + (ksp > 1 ? (size_t)BM * (BN + 4) * 4 : 0);
     MARLC_CHECK(smem_bytes <= 227 * 1024, "tc_lstm_pair: K-split staging does not fit in shared memory");
     static size_t attr_sz = 0;
@@ -1057,8 +999,7 @@ static int launch_lstm(TcKernelGroup& kp, int gx, int gy, int nkb, cudaStream_t 
         attr_sz = smem_bytes;
     }
     kp.trig = pdl_trigger_early();
-    MARLC_CUDA(launch_pdl(kern, dim3(gx * ksp, gy, 2), dim3(X3 ? TC_THREADS_X3 : TC_THREADS), cl > 1 ? smem_bytes : (size_t)S::BYTES,
-                          s, kp, cl > 1 ? cl : 1));
+    MARLC_CUDA(launch_pdl(kern, dim3(gx * ksp, gy, 2), dim3(X3 ? TC_THREADS_X3 : TC_THREADS), smem_bytes, s, kp, ksp));
     ++g_tc_gemm_launches;
     MARLC_LAUNCH_CHECK();
     return 0;
@@ -1079,31 +1020,21 @@ TcLstmPlan tc_lstm_plan(int M, int n0, int n1, bool x3) {
     // 128 x 256 tiles (64 hidden units x 4 gates) once they still fill the machine: a kind::tf32 MMA reads its
     // operands from shared memory at 128 B/clk for a 128 x 128 tile (the whole shared-memory bandwidth of the
     // SM, before the TMA writes and the 3xTF32 low-order tiles), 96 B/clk for 128 x 256 -- and the tile streams
-    // 25 % fewer operand bytes per flop (MARLC_LSTM_HU64=0 switches it off)
-    static const int hu64 = getenv("MARLC_LSTM_HU64") ? atoi(getenv("MARLC_LSTM_HU64")) : 1;
+    // 25 % fewer operand bytes per flop
     // (measured, 16 steps at n = 256: M = 2048 -> 796 us with 64 units per tile vs 858 with 32; M = 1024 -> 673 vs 439)
-    if (hu64 && n0 % 64 == 0 && n1 % 64 == 0 && 2 * mt * (n0 / 64) >= 120) HU = 64;
-    static const int hu_force = getenv("MARLC_LSTM_HU") ? atoi(getenv("MARLC_LSTM_HU")) : 0;  // A/B toggle
-    if (hu_force == 8 || hu_force == 16 || hu_force == 32 || hu_force == 64) HU = hu_force;
+    if (n0 % 64 == 0 && n1 % 64 == 0 && 2 * mt * (n0 / 64) >= 120) HU = 64;
     while (HU > 8 && (n0 % HU != 0 || n1 % HU != 0)) HU >>= 1;
     // few CTAs (small M): fat stages, KS sub-blocks of 32 floats per barrier round trip
     const bool fat = HU <= 16 && 2 * mt * (n0 / HU) <= MARLC_SMS;
     const int KSv = !fat ? 1 : (x3 ? 2 : (HU == 8 ? 4 : 2));
-    // A-tile multicast: the n/HU CTAs of one M tile all read the same 128 x K activations; in a cluster
-    // of `cl` of them each CTA requests 1/cl of every A tile and the TMA unit delivers it to all
-    // (the main loop is bound by what one SM's TMA engine can request, ~40-50 B/clk measured)
-    // (measured: no gain at M=128 - 14.4 vs 14.1 us - and slightly slower at M=4096: what binds is the
-    // bytes ARRIVING in each SM, not the requests its TMA engine issues; off unless MARLC_LSTM_CLUSTER)
-    int cl = 1;
-    if (const char* env = getenv("MARLC_LSTM_CLUSTER")) cl = atoi(env);
-    while (cl > 1 && ((n0 / HU) % cl != 0 || (BM / cl) % 8 != 0)) cl >>= 1;
-    if (cl < 1) cl = 1;
+    // (A-tile TMA multicast across the n/HU CTAs of one M tile was measured: no gain at M=128 - 14.4 vs 14.1 us -
+    // and slightly slower at M=4096: what binds is the bytes ARRIVING in each SM, not the requests its TMA engine
+    // issues.  Removed.)
     // K split over CTA pairs (DSMEM reduction): halves the bytes each SM streams; used when the launch is
     // small enough that twice the CTAs still fit in one wave
-    int ksplit = (fat && HU == 8 && cl == 1 && 2 * 2 * mt * (n0 / HU) <= MARLC_SMS) ? 2 : 1;
-    if (const char* env = getenv("MARLC_LSTM_KSPLIT")) ksplit = (atoi(env) == 2 && fat && HU == 8 && cl == 1) ? 2 : 1;
+    const int ksplit = (fat && HU == 8 && 2 * 2 * mt * (n0 / HU) <= MARLC_SMS) ? 2 : 1;
     TcLstmPlan p;
-    p.hu = HU; p.bn = 4 * HU; p.fat = fat ? 1 : 0; p.ks = KSv; p.ksplit = ksplit; p.cluster = cl;
+    p.hu = HU; p.bn = 4 * HU; p.fat = fat ? 1 : 0; p.ks = KSv; p.ksplit = ksplit;
     p.tail_rows = M - (mt - 1) * BM;
     return p;
 }
@@ -1113,7 +1044,7 @@ int tc_lstm_pair(const TcLstmArgs& c0, const TcLstmArgs& c1, cudaStream_t s) {
     MARLC_CHECK(c0.M == c1.M, "tc_lstm_pair: row counts differ");
     const int mt = (c0.M + BM - 1) / BM;
     const TcLstmPlan pl = tc_lstm_plan(c0.M, c0.n, c1.n, c0.x3 != 0);
-    const int HU = pl.hu, KSv = pl.ks, cl = pl.cluster, ksplit = pl.ksplit;
+    const int HU = pl.hu, KSv = pl.ks, ksplit = pl.ksplit;
     const bool fat = pl.fat != 0;
     MARLC_CHECK(c0.n % HU == 0 && c1.n % HU == 0, "tc_lstm_pair: hidden size not a multiple of %d", HU);
     TcKernelGroup kp;
@@ -1122,26 +1053,24 @@ int tc_lstm_pair(const TcLstmArgs& c0, const TcLstmArgs& c1, cudaStream_t s) {
     kp.zofs[0] = 0; kp.zofs[1] = 1; kp.zofs[2] = 2;
     const int BKS = BK * KSv;
     const TcLstmArgs* cs[2] = {&c0, &c1};
-    const int abox = BM / cl;
     int gx = 0;
     for (int k = 0; k < 2; ++k) {
         const TcLstmArgs& c = *cs[k];
         TcKernelParams& p = kp.p[k];
-        p.cluster = cl;
         p.ksplit = ksplit;
-        MARLC_TRY(make_map(&p.a1, c.U.ptr, c.Kin, c.M, c.U.slabs, c.U.ld, c.U.slab_stride, abox));
+        MARLC_TRY(make_map(&p.a1, c.U.ptr, c.Kin, c.M, c.U.slabs, c.U.ld, c.U.slab_stride, BM));
         // weights viewed as [gate][unit][K]: ONE box of HU units x 4 gates per K sub-block (the producer
         // thread is issue-bound: 4 separate gate boxes per sub-block made 20 TMA instructions per stage)
         MARLC_TRY(make_map(&p.b1, c.Wih, c.Kin, c.n, 4, c.Kin, (long)c.n * c.Kin, HU, false, 4));
-        MARLC_TRY(make_map(&p.a2, c.Hprev.ptr, c.n, c.M, c.Hprev.slabs, c.Hprev.ld, c.Hprev.slab_stride, abox));
+        MARLC_TRY(make_map(&p.a2, c.Hprev.ptr, c.n, c.M, c.Hprev.slabs, c.Hprev.ld, c.Hprev.slab_stride, BM));
         MARLC_TRY(make_map(&p.b2, c.Whh, c.n, c.n, 4, c.n, (long)c.n * c.n, HU, false, 4));
         p.nk1 = (c.Kin + BKS - 1) / BKS;
         p.nk2 = (c.n + BKS - 1) / BKS;
         p.a_lo_g = (c.x3 && c.U.lo && c.Hprev.lo) ? 1 : 0;
         p.b_lo_g = (c.x3 && c.Wih_lo && c.Whh_lo) ? 1 : 0;
         if (p.a_lo_g) {
-            MARLC_TRY(make_map(&p.a1l, c.U.lo, c.Kin, c.M, c.U.slabs, c.U.ld, c.U.slab_stride, abox));
-            MARLC_TRY(make_map(&p.a2l, c.Hprev.lo, c.n, c.M, c.Hprev.slabs, c.Hprev.ld, c.Hprev.slab_stride, abox));
+            MARLC_TRY(make_map(&p.a1l, c.U.lo, c.Kin, c.M, c.U.slabs, c.U.ld, c.U.slab_stride, BM));
+            MARLC_TRY(make_map(&p.a2l, c.Hprev.lo, c.n, c.M, c.Hprev.slabs, c.Hprev.ld, c.Hprev.slab_stride, BM));
         }
         if (p.b_lo_g) {
             MARLC_TRY(make_map(&p.b1l, c.Wih_lo, c.Kin, c.n, 4, c.Kin, (long)c.n * c.Kin, HU, false, 4));
@@ -1153,8 +1082,6 @@ int tc_lstm_pair(const TcLstmArgs& c0, const TcLstmArgs& c1, cudaStream_t s) {
         p.bias = c.bih; p.bias2 = c.bhh;
         p.c_prev = c.c_prev; p.c_new = c.c_new; p.h_new = c.h_new; p.gates = c.gates;
         p.n_hidden = c.n;
-        static const int staged_env = getenv("MARLC_LSTM_STAGED") ? atoi(getenv("MARLC_LSTM_STAGED")) : 1;  // A/B toggle
-        p.epi_staged = staged_env;
         p.splits = 1;
         gx = max(gx, c.n / HU);
     }

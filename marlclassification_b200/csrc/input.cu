@@ -13,36 +13,11 @@
 
 namespace marlc {
 
-// HWC uint8 -> CHW fp32.  One thread = 4 consecutive pixels of one row (needs W % 4 == 0 so the
-// 4*C source bytes start on a 4-byte boundary): C 32-bit loads, C float4 stores.
-template <int C>
-__global__ void __launch_bounds__(256) u8hwc_to_f32chw_kernel(const uint8_t* __restrict__ src, float* __restrict__ dst,
-                                                              long groups, int H, int W) {
-    const int w4 = W >> 2;
-    for (long g = blockIdx.x * (long)blockDim.x + threadIdx.x; g < groups; g += (long)gridDim.x * blockDim.x) {
-        const long row = g / w4;          // b * H + y
-        const int x0 = (int)(g - row * w4) << 2;
-        const long b = row / H;
-        const int y = (int)(row - b * H);
-        const uint32_t* s4 = reinterpret_cast<const uint32_t*>(src + (row * W + x0) * C);
-        uint32_t wds[C];
-#pragma unroll
-        for (int i = 0; i < C; ++i) wds[i] = __ldg(s4 + i);
-        float px[4 * C];
-#pragma unroll
-        for (int i = 0; i < 4 * C; ++i) px[i] = (float)((wds[i >> 2] >> (8 * (i & 3))) & 0xFFu) / 255.0f;
-#pragma unroll
-        for (int c = 0; c < C; ++c) {
-            float* d = dst + ((b * C + c) * H + y) * (long)W + x0;
-            __stcs(reinterpret_cast<float4*>(d), make_float4(px[c], px[C + c], px[2 * C + c], px[3 * C + c]));
-        }
-    }
-}
-
-// Same conversion, one image ROW per threadIdx.y: the row's (b, y) is one 32-bit division per
-// thread and the position inside the row needs none.  The 1-D kernel above pays two 64-bit
-// divisions (~200 instructions) per 4 pixels, which is more issue time than the 60 bytes it moves
-// cost in HBM time; kept behind MARLC_U8_ROWS=0 for the A/B in profiles/README.md.
+// HWC uint8 -> CHW fp32, one image ROW per threadIdx.y (needs W % 4 == 0 so the 4*C source bytes of
+// 4 pixels start on a 4-byte boundary): the row's (b, y) is one 32-bit division per thread and the
+// position inside the row needs none.  A 1-D grid over groups of 4 pixels pays two 64-bit divisions
+// (~200 instructions) per 4 pixels, more issue time than the 60 bytes they move cost in HBM time
+// (A/B in profiles/README.md).
 template <int C>
 __global__ void __launch_bounds__(256) u8hwc_to_f32chw_rows_kernel(const uint8_t* __restrict__ src,
                                                                    float* __restrict__ dst, int rows, int H, int W) {
@@ -107,11 +82,6 @@ static void launch_rows(const uint8_t* src, float* dst, int rows, int H, int W, 
     u8hwc_to_f32chw_rows_kernel<C><<<grid, dim3(tx, ty), 0, s>>>(src, dst, rows, H, W);
 }
 
-static bool u8_rows_enabled() {
-    const char* e = getenv("MARLC_U8_ROWS");
-    return !(e && e[0] == '0');
-}
-
 static int grid_for(long work_items) {
     const long blocks = (work_items + 255) / 256;
     return (int)std::max(1L, std::min(blocks, 148L * 16));  // grid-stride beyond 16 CTAs per SM
@@ -134,14 +104,10 @@ extern "C" int marlc_images_u8_to_f32(const uint8_t* src, float* dst, int B, int
         else u8hwc_to_f32chw_generic_kernel<<<grid_for(total), 256, 0, s>>>(src, dst, total, 1, 1, 1024);  // identity order
     } else {
         const bool vec = (W % 4 == 0) && (((uintptr_t)src & 3) == 0) && (((uintptr_t)dst & 15) == 0);
-        const long groups = (long)B * H * (W / 4);
-        const bool rows = vec && (long)B * H < 0x7fffffffL && u8_rows_enabled();
+        const bool rows = vec && (long)B * H < 0x7fffffffL;
         if (rows && C == 3) launch_rows<3>(src, dst, B * H, H, W, s);
         else if (rows && C == 4) launch_rows<4>(src, dst, B * H, H, W, s);
         else if (rows && C == 2) launch_rows<2>(src, dst, B * H, H, W, s);
-        else if (vec && C == 3) u8hwc_to_f32chw_kernel<3><<<grid_for(groups), 256, 0, s>>>(src, dst, groups, H, W);
-        else if (vec && C == 4) u8hwc_to_f32chw_kernel<4><<<grid_for(groups), 256, 0, s>>>(src, dst, groups, H, W);
-        else if (vec && C == 2) u8hwc_to_f32chw_kernel<2><<<grid_for(groups), 256, 0, s>>>(src, dst, groups, H, W);
         else u8hwc_to_f32chw_generic_kernel<<<grid_for(total), 256, 0, s>>>(src, dst, total, C, H, W);
     }
     MARLC_LAUNCH_CHECK();

@@ -125,8 +125,6 @@ int tn_skinny(const float* dY, long lddy, const float* X, long ldx, float* dW, l
               int accumulate, cudaStream_t s, bool* done) {
     *done = false;
     if (R <= 0 || N <= 0 || K <= 0) return 0;
-    static const bool off = getenv("MARLC_NO_SKINNY") != nullptr;  // A/B toggle
-    if (off) return 0;
     const bool tiny = N * K <= 32 && K <= 32;
     const bool small = N <= 8;
     if (!tiny && !small) return 0;

@@ -70,9 +70,8 @@ bool tc_lstm_shapes_ok(int Kin, int n);
 bool tc_lstm_supported(const TcLstmArgs& a);
 // The tile configuration tc_lstm_pair launches for M rows and hidden sizes n0 / n1 (host only; also
 // what marlc_engine_plan reports): HU hidden units x 4 gates = BN columns per CTA, fat stages of KS
-// 32-float K sub-blocks, K split over `ksplit` CTAs, A-tile multicast over `cluster` CTAs; `tail_rows` rows
-// in the last 128-row tile.
-struct TcLstmPlan { int hu, bn, fat, ks, ksplit, cluster, tail_rows; };
+// 32-float K sub-blocks, K split over `ksplit` CTAs (a cluster); `tail_rows` rows in the last 128-row tile.
+struct TcLstmPlan { int hu, bn, fat, ks, ksplit, tail_rows; };
 TcLstmPlan tc_lstm_plan(int M, int n0, int n1, bool x3);
 int tc_lstm_pair(const TcLstmArgs& belief, const TcLstmArgs& action, cudaStream_t s);
 

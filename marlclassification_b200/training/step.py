@@ -30,13 +30,10 @@ class TrainStep:
         self._graphs: dict = {False: None, True: None}
         self._warm = {False: 0, True: 0}
         self._inj: Optional[dict] = None  # static pos0 / hidden0 / actions (parity runs through the graph path)
-        import os
-
-        # Data parallel: three graphs with the two NCCL all-reduces issued eagerly between them (default), or ONE
-        # graph with the collectives captured inside it (MARLC_DP_ONE_GRAPH=1).  Measured on 2 B200 (round 2,
-        # config c4, 128 images per GPU): one graph 8.03 ms per iteration, three graphs 7.93 ms -- no gain -- and
-        # the one-graph form HUNG in tests/test_gpu_dp.py (small shapes, 6 steps), so it stays opt-in.
-        self.split_graphs = os.environ.get("MARLC_DP_ONE_GRAPH", "0") != "1"
+        # Data parallel: three graphs with the two NCCL all-reduces issued eagerly between them.  One graph with the
+        # collectives captured inside it was measured on 2 B200 (config c4, 128 images per GPU): 8.03 ms per
+        # iteration against 7.93 ms for three graphs, and it hung in tests/test_gpu_dp.py, so it was removed.
+        # Reported by bench.py: the collectives are never part of a captured graph.
         self.nccl_in_graph = False
 
     # ---- the segments between collectives -----------------------------------------
@@ -54,15 +51,6 @@ class TrainStep:
     def _seg_update(self) -> None:
         self.optim.step(1.0 / self.dp.world_size)
 
-    def _whole_step(self, injected: bool = False) -> None:
-        """The complete iteration, collectives included, in stream order."""
-        eng, dp = self.engine, self.dp
-        self._seg_forward(injected)
-        dp.all_reduce_stats(eng.loss_stats)          # no-op on one GPU
-        self._seg_backward()
-        dp.all_reduce_grads_sum(eng.model.flat_grads)
-        self._seg_update()
-
     def _segments(self, injected: bool = False):
         fwd = lambda: self._seg_forward(injected)  # noqa: E731
         if self.dp.enabled:
@@ -71,25 +59,7 @@ class TrainStep:
 
     def _capture(self, injected: bool) -> None:
         """Single GPU: ONE CUDA graph for the whole iteration.  Data parallel: the segments between the two
-        NCCL all-reduces (3 doubles of advantage statistics, the flat gradient bucket) are one graph each; with
-        MARLC_DP_ONE_GRAPH=1 the collectives are captured too and the iteration is one graph (experimental,
-        see __init__)."""
-        if self.dp.enabled and not self.split_graphs:
-            try:
-                th.cuda.synchronize()
-                g = th.cuda.CUDAGraph()
-                with th.cuda.graph(g):
-                    self._whole_step(injected)
-                self._graphs[injected] = [g]
-                self.nccl_in_graph = True
-                return
-            except Exception as exc:  # pragma: no cover - depends on the NCCL build
-                import warnings
-
-                warnings.warn(f"NCCL collectives could not be captured in the step graph ({exc!r}); "
-                              "using three graphs with eager collectives between them")
-                self.split_graphs = True
-                th.cuda.synchronize()
+        NCCL all-reduces (3 doubles of advantage statistics, the flat gradient bucket) are one graph each."""
         graphs = []
         for seg in self._segments(injected):
             g = th.cuda.CUDAGraph()
@@ -114,9 +84,7 @@ class TrainStep:
         else:
             segs = self._segments(injected)
             self._warm[injected] += 1
-        if len(segs) == 1 and dp.enabled:  # whole step, collectives captured inside
-            segs[0]()
-        elif dp.enabled:
+        if dp.enabled:
             segs[0]()
             dp.all_reduce_stats(eng.loss_stats)
             segs[1]()

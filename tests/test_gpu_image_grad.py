@@ -225,13 +225,10 @@ def test_geometry_image_grad(key, geometry_cache):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("key,mode", [("93", "fp32"), ("dense", "fp32"), ("93", "unfused"), ("odd_window", "unfused"),
-                                      ("1190", "chunks2"), ("many_windows", "chunks2")])
-def test_modes_image_grad(key, mode, geometry_cache, monkeypatch):
-    if mode == "chunks2":  # read when the engine is bound: set before the model (and its engines) exist
-        monkeypatch.setenv("MARLC_BWD_CHUNKS", "2")
+@pytest.mark.parametrize("key,mode", [("93", "fp32"), ("dense", "fp32"), ("93", "unfused"), ("odd_window", "unfused")])
+def test_modes_image_grad(key, mode, geometry_cache):
     d, ref, _ = geometry(key, geometry_cache)
-    got, _, _ = engine_grad(d, mode="tf32x3" if mode == "chunks2" else mode)
+    got, _, _ = engine_grad(d, mode=mode)
     rel, pix = img_errors(got, ref)
     print(f"\n{key} {mode}: image gradient rel-L2 {rel:.1e}, per-pixel {pix:.1e}")
     bound = BOUND_FP32 if mode == "fp32" else BOUND

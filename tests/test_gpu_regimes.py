@@ -17,23 +17,19 @@ that put a gradient on a few rows only.
 """
 import ctypes as ct
 import functools
-import json
-import os
-import subprocess
-import sys
 
 import pytest
 import torch
 
 from oracle import marl_oracle as O
-from tests.conftest import ROOT, oracle_config, rel_l2
+from tests.conftest import oracle_config, rel_l2
 from tests.test_gpu_configs import C2_NET, MOVES1, MOVES3, _graphed_iteration, _mc
 
 DEV = "cuda"
 MNIST_NET = _mc("mnist", 6, 64, 16, 24, 8, 96, 96, 10, MOVES1)  # n = 64, channel 0 of 3
 AID_NET = _mc("aid", 24, 256, 64, 96, 16, 320, 320, 30, MOVES3)  # 388 KB of conv weights: never wide
 
-# Expected plan columns, computed from the launchers' code at the default settings (no MARLC_* variable):
+# Expected plan columns, computed from the launchers' code:
 #   cnn  = None (one CTA per window) or (batches of 8 windows, CTAs, passes, windows in the last batch)
 #   lstm = (HU, fat, K split, rows in the last 128-row tile)    sweep = 1 chained / 0 unfused
 # HU: 8 for one 128-row tile, 16 from 2 tiles, 32 from 8, 64 once 2 * tiles * (n / 64) >= 120 (M >= 1793 at
@@ -104,12 +100,7 @@ def _plans():
 
 
 def test_plan_table():
-    # the thresholds are read once per process: query them in a fresh one without any MARLC_* override
-    env = {k: v for k, v in os.environ.items() if not k.startswith("MARLC_")}
-    code = "import json; from tests.test_gpu_regimes import _plans; print(json.dumps(_plans()))"
-    res = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=env, capture_output=True, text=True, timeout=900)
-    assert res.returncode == 0, res.stderr[-3000:]
-    plans = json.loads(res.stdout.strip().splitlines()[-1])
+    plans = _plans()
     for key, c in CASES.items():
         got, want = plans[key], _mplan(key)
         diff = {k: (got[k], v) for k, v in want.items() if got[k] != v}

@@ -175,16 +175,29 @@ def test_same_seed_gives_the_reference_initialisation(name):
 
 
 def test_every_environment_switch_is_documented():
-    """Every MARLC_* variable the library or the Python package reads is listed in INTEGRATION.md section 3."""
+    """Every MARLC_* variable the library or the Python package reads is listed in INTEGRATION.md section 3, and
+    every MARLC_* name in the first column of that table is still read by the code or tested by an #ifdef in csrc/."""
     import glob
     import re
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    names = set()
+    names, macros = set(), set()
     for path in glob.glob(os.path.join(root, "marlclassification_b200", "csrc", "*.cu*")):
-        names |= set(re.findall(r'getenv\("(MARLC_[A-Z0-9_]+)"\)', open(path).read()))
+        src = open(path).read()
+        names |= set(re.findall(r'getenv\("(MARLC_[A-Z0-9_]+)"\)', src))
+        macros |= set(re.findall(r"#\s*ifn?def\s+(MARLC_[A-Z0-9_]+)", src))
+        macros |= set(re.findall(r"defined\s*\(?\s*(MARLC_[A-Z0-9_]+)", src))
     for path in glob.glob(os.path.join(root, "marlclassification_b200", "**", "*.py"), recursive=True) + [os.path.join(root, "bench.py")]:
         names |= set(re.findall(r'environ(?:\.get)?[\(\[]"(MARLC_[A-Z0-9_]+)"', open(path).read()))
     doc = open(os.path.join(root, "INTEGRATION.md")).read()
     missing = sorted(n for n in names if n not in doc)
     assert names and not missing, f"undocumented switches: {missing}"
+    section = re.search(r"^## 3\..*?$(.*?)(?=^## |\Z)", doc, re.M | re.S)
+    assert section, "INTEGRATION.md has no section 3"
+    listed = set()
+    for line in section.group(1).splitlines():
+        if line.startswith("|"):
+            listed |= set(re.findall(r"MARLC_[A-Z0-9_]+", line.split("|")[1]))
+    assert listed, "no switches parsed from INTEGRATION.md section 3"
+    stale = sorted(listed - names - macros)
+    assert not stale, f"documented switches the code no longer reads: {stale}"
