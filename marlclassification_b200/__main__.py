@@ -66,7 +66,8 @@ def build_parser() -> argparse.ArgumentParser:
     train.add_argument("--batch-size", type=int, default=8, dest="batch_size",
                        help="images per optimisation step (the GLOBAL batch under torchrun)")
     train.add_argument("--lr", "--learning-rate", type=float, default=1e-3, dest="learning_rate", help="Adam step size")
-    train.add_argument("--gamma", type=float, default=0.99, help="discount of the returns")
+    train.add_argument("--gamma", type=float, default=0.99, help="discount of the returns (0: the returns are the rewards, where the "
+                       "original's closed form divides 0 by 0)")
     train.add_argument("--nb-epoch", type=int, default=10, dest="nb_epoch", help="passes over the training split")
     train.add_argument("--workers", type=int, default=6, help="DataLoader worker processes (train.py:95 uses 6)")
     train.add_argument("--resident", action="store_true",

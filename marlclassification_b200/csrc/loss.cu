@@ -75,7 +75,10 @@ __global__ void vote_kernel(const LossArgs a) {
     if (lane == 0) atomicAdd(&a.stats[5], (double)(lse - vote(y)));
 }
 
-// thread per m: G_t = r_t + gamma G_{t+1} (== functions.py:35-51), adv = G - V
+// thread per m: G_t = r_t + gamma G_{t+1} (== functions.py:35-51), adv = G - V.
+// Deliberate departure at gamma = 0: the reference's closed form (flip-cumsum-flip of r gamma^t, divided by gamma^t)
+// is 0/0 there from t = 1 on, so its returns, losses and gradients are NaN; this recursion gives G_t = r_t, the
+// returns that closed form stands for (tests/test_gpu_update.py pins both)
 __global__ void returns_kernel(const LossArgs a) {
     const int M = a.Na * a.Nb;
     const int m = blockIdx.x * blockDim.x + threadIdx.x;
@@ -139,7 +142,10 @@ __global__ void loss_b_kernel(const LossArgs a) {
         const double n = a.stats[2];
         const double mean = a.stats[0] / n;
         const double var = (a.stats[1] - n * mean * mean) / (n - 1.0);  // unbiased (torch.std default)
-        const float stdv = (float)sqrt(var > 0.0 ? var : 0.0);
+        // one advantage in the whole batch (T * Na * Nb == 1): torch.std of one element is NaN, and so is the
+        // reference's loss.  The clamp below used to turn that 0/0 into 0 and return a finite loss; the NaN is
+        // kept instead, like the bad-label NaN of loss_finalize_kernel (error and critic stay finite, as there)
+        const float stdv = n < 2.0 ? __int_as_float(0x7fc00000) : (float)sqrt(var > 0.0 ? var : 0.0);
         const float nadv = (a.adv[i] - (float)mean) / (stdv + 1e-8f);
         const float invM = 1.0f / (float)M;
         path = (double)(-a.logp[i] * nadv);

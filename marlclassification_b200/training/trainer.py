@@ -66,6 +66,11 @@ class Trainer:
         synchronising.  ``x`` / ``y`` may be host (pinned) or device tensors, or ``x`` a
         StagedBatch produced by :meth:`prefetch` (then ``y`` is ignored)."""
         eng = episode_sampler.engine_for(x, gamma=self.__gamma)
+        if eng.T * eng.na * eng.nb * self.__dp.world_size < 2:
+            # the fused loss would be NaN (the standard deviation of one advantage, as in the reference) and its
+            # NaN gradients would reach every parameter through Adam: refuse before anything is updated
+            raise RuntimeError("the batch holds a single advantage (nb_step * nb_agents * images == 1), whose "
+                               "standard deviation is undefined: use more steps, agents or images per batch")
         step = self.__steps.get(id(eng))
         if step is None:
             step = TrainStep(eng, self.__optim, self.__dp, use_graph=self.__cuda_graph)

@@ -323,7 +323,8 @@ def classification_rewards(step_preds: torch.Tensor, targets: torch.Tensor) -> t
 
 
 def discounted_returns(rewards: torch.Tensor, gamma: float) -> torch.Tensor:
-    """functions.py:35-51: flip-cumsum-flip of r*gamma^t, divided by gamma^t."""
+    """functions.py:35-51: flip-cumsum-flip of r*gamma^t, divided by gamma^t (0/0 = NaN from t = 1 on at
+    gamma = 0, as in the reference)."""
     T = rewards.shape[0]
     g = (gamma ** torch.arange(T, dtype=rewards.dtype, device=rewards.device)).view(T, *([1] * (rewards.dim() - 1)))
     return (rewards * g).flip(0).cumsum(0).flip(0) / g
@@ -370,10 +371,11 @@ def loss_and_grads(p, cfg, img, targets, pos0, hidden0, actions, nb_step, gamma)
     return ro, parts, {k: (g if g is not None else torch.zeros_like(leaf[k])) for k, g in zip(names, grads)}
 
 
-def train_steps(p, cfg, img, targets, pos0, hidden0, actions, nb_step, gamma, lr, n_steps):
+def train_steps(p, cfg, img, targets, pos0, hidden0, actions, nb_step, gamma, lr, n_steps, parts_out=None):
     """``n_steps`` optimisation steps of trainer.py:66-116 on ONE batch with the same injected draws
     every step: rollout -> loss -> ``backward`` -> ``th.optim.Adam(lr)`` (trainer.py:33 defaults:
-    betas (0.9, 0.999), eps 1e-8).  Returns (final params, [loss per step])."""
+    betas (0.9, 0.999), eps 1e-8).  Returns (final params, [loss per step]); a list ``parts_out``
+    receives each step's [loss, path, error, actor, critic]."""
     leaf = {k: v.detach().clone().requires_grad_(True) for k, v in p.items()}
     opt = torch.optim.Adam(list(leaf.values()), lr=lr)
     losses = []
@@ -384,6 +386,8 @@ def train_steps(p, cfg, img, targets, pos0, hidden0, actions, nb_step, gamma, lr
         parts.loss.backward()
         opt.step()
         losses.append(float(parts.loss.detach()))
+        if parts_out is not None:
+            parts_out.append([float(getattr(parts, k).detach()) for k in ("loss", "path", "error", "actor", "critic")])
     return {k: v.detach() for k, v in leaf.items()}, losses
 
 

@@ -13,24 +13,16 @@ import pytest
 import torch
 
 from oracle import marl_oracle as O
-from tests.conftest import GOLDEN_DIR, load_golden, oracle_config, rel_l2
+from tests.conftest import GOLDEN_DIR, load_golden, rel_l2
+from tests.nets import C2_NET, MOVES1, MOVES3  # noqa: F401  (re-exported to the other GPU test modules)
+from tests.nets import model_config as _mc
+from tests.nets import oracle_case as _oracle_case
 
 pytestmark = pytest.mark.gpu
 
 TOL = 1e-3
 DEV = "cuda"
 
-MOVES1 = [[1, 0], [-1, 0], [0, 1], [0, -1]]
-MOVES3 = [[3, 0], [-3, 0], [0, 3], [0, -3]]
-
-
-def _mc(ft, f, n, n_m, n_m_o, n_d, nl_b, nl_a, nc, actions):
-    return dict(ft_extr_str=ft, window_size=f, hidden_size_belief=n, hidden_size_action=n, hidden_size_msg=n_m,
-                hidden_size_msg_output=n_m_o, hidden_size_state=n_d, state_dim=2, actions=actions, nb_class=nc,
-                hidden_size_linear_belief=nl_b, hidden_size_linear_action=nl_a)
-
-
-C2_NET = _mc("resisc45", 12, 256, 64, 96, 16, 384, 384, 45, MOVES1)
 CONFIGS = {
     # BASELINE.json configs 1-3 (README.md:39-43 hyper-parameters)
     "c1_mnist": dict(mc=_mc("mnist", 6, 64, 16, 24, 8, 96, 96, 10, MOVES1), na=3, nb=32, T=5, C=3, H=28, W=28),
@@ -53,21 +45,6 @@ CONFIGS = {
     "shipped_aid": dict(mc=_mc("aid", 24, 768, 128, 192, 16, 1024, 1024, 30, MOVES3 + [[0, 0]]),
                         na=16, nb=8, T=16, C=3, H=600, W=600),
 }
-
-
-def _oracle_case(spec, seed=99):
-    ocfg = oracle_config(spec["mc"])
-    params = O.init_params(ocfg, seed=7)
-    na, nb, T = spec["na"], spec["nb"], spec["T"]
-    g = torch.Generator().manual_seed(seed)
-    img = torch.rand(nb, spec["C"], spec["H"], spec["W"], generator=g)
-    y = torch.randint(ocfg.nb_class, (nb,), generator=g)
-    pos0 = torch.stack([torch.randint(spec["H"] - ocfg.f, (na, nb), generator=g),
-                        torch.randint(spec["W"] - ocfg.f, (na, nb), generator=g)], -1)
-    hidden0 = [torch.randn(na, nb, n, generator=g) for n in (ocfg.n_b, ocfg.n_b, ocfg.n_a, ocfg.n_a)]
-    # on-distribution trajectory: the oracle samples its own actions, both sides replay them
-    actions = O.rollout(params, ocfg, img, pos0, hidden0, None, T, generator=g).actions
-    return ocfg, params, img, y, pos0, hidden0, actions
 
 
 def _graphed_iteration(eng, img, y, pos0, hidden0, actions):
