@@ -106,6 +106,31 @@ int marlc_tc_lstm_pair_presplit(const float* u, const float* u_lo, int M, int Ki
 int marlc_cnn_forward(int layers, const int* cin, const int* cout, const int* groups, int f, int img_c,
                       const float* const* w, const float* const* b, const float* const* gn_w,
                       const float* const* gn_b, const float* patch, float* out, int N, void* stream);
+/* marlc_cnn_forward that also keeps what marlc_cnn_backward reads: y_save is a HOST array of `layers`
+ * nullable device pointers, y_save[l] f32[N, cout[l]*h_{l+1}^2] receiving layer l's pre-norm conv outputs in
+ * (channel, position) order.  The output is bit-identical to marlc_cnn_forward's. */
+int marlc_cnn_forward_save(int layers, const int* cin, const int* cout, const int* groups, int f, int img_c,
+                           const float* const* w, const float* const* b, const float* const* gn_w,
+                           const float* const* gn_b, const float* patch, float* const* y_save, float* out, int N,
+                           void* stream);
+/* Bytes of device workspace marlc_cnn_backward needs for N windows; want_param_grads != 0 when any d_w[l] will be
+ * given (the im2col rows of the weight gradients are included then).  Host only; 0 on a bad argument. */
+size_t marlc_cnn_backward_workspace_bytes(int layers, const int* cin, const int* cout, int f, int N,
+                                          int want_param_grads);
+/* Backward of marlc_cnn_forward_save (vision.py:47-49 under autograd) from d_out f32[N, out_size] on the same
+ * windows `patch`, parameters and y_save.  `workspace` (256-byte aligned, at least
+ * marlc_cnn_backward_workspace_bytes; its contents on entry do not matter) is scratch.  Outputs, each nullable
+ * (= not wanted): d_patch f32[N, img_c, f, f], every element written (exactly 0 in the channels >= cin[0] the
+ * network does not read); d_w / d_b / d_gn_w / d_gn_b, HOST arrays (or NULL) of `layers` nullable device pointers
+ * shaped like the parameters, ADDED to.  With no d_w[l] at all the input im2col and every weight-gradient GEMM
+ * are skipped.  The conv products run in 3xTF32 on the tensor cores (exact FFMA where an operand is not
+ * TMA-addressable).  One stream; neither allocates nor synchronises.  N = 0 is a no-op.  Argument and shape
+ * errors are reported before anything is launched. */
+int marlc_cnn_backward(int layers, const int* cin, const int* cout, const int* groups, int f, int img_c,
+                       const float* const* w, const float* const* b, const float* const* gn_w,
+                       const float* const* gn_b, const float* patch, const float* const* y_save, const float* d_out,
+                       int N, void* workspace, size_t workspace_bytes, float* d_patch, float* const* d_w,
+                       float* const* d_b, float* const* d_gn_w, float* const* d_gn_b, void* stream);
 
 /* ---- the episode engine ---------------------------------------------------- */
 

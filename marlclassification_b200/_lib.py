@@ -62,6 +62,13 @@ _SIGS = {
     "marlc_tc_lstm_pair_presplit": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int] + [C.POINTER(_P)] * 13 + [_P]),
     "marlc_cnn_forward": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int, C.c_int,
                                     C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), _P, _P, C.c_int, _P]),
+    "marlc_cnn_forward_save": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int,
+                                         C.c_int] + [C.POINTER(_P)] * 4 + [_P, C.POINTER(_P), _P, C.c_int, _P]),
+    "marlc_cnn_backward_workspace_bytes": (C.c_size_t, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int,
+                                                        C.c_int, C.c_int]),
+    "marlc_cnn_backward": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int,
+                                     C.c_int] + [C.POINTER(_P)] * 4 + [_P, C.POINTER(_P), _P, C.c_int, _P, C.c_size_t, _P]
+                           + [C.POINTER(_P)] * 4 + [_P]),
     "marlc_engine_create": (C.c_int, [C.POINTER(MarlcConfig), C.POINTER(_P)]),
     "marlc_engine_destroy": (None, [_P]),
     "marlc_engine_plan": (C.c_int, [_P, C.POINTER(MarlcPlan)]),

@@ -178,21 +178,36 @@ __global__ void __launch_bounds__(256) cnn_bwd_layer_kernel(const CnnBwdLayerKer
     }
 }
 
-int cnn_bwd_layer(const CnnBwdLayerArgs& a, cudaStream_t s) {
-    if (a.P <= 0) return 0;
-    CnnBwdLayerKernelArgs ka;
+// Launch geometry of cnn_bwd_layer (warps per CTA, shared memory); fails when the layer does not fit.
+static int bwd_layer_plan(const CnnBwdLayerArgs& a, CnnBwdLayerKernelArgs& ka, int& wpc, size_t& smem) {
     ka.a = a;
     ka.npos = a.ho * a.ho;
     ka.total = a.cout * ka.npos;
     ka.npn = a.ho_next * a.ho_next;
     ka.per_warp = 3 * ((ka.total + 3) & ~3) + (a.dOut ? 0 : ((ka.npn * a.cout * 9 + 3) & ~3));
-    int wpc = 8;
+    wpc = 8;
     while (wpc > 1 && (size_t)wpc * ka.per_warp * sizeof(float) > 160 * 1024) wpc >>= 1;
     MARLC_CHECK((a.d_gn_w != nullptr) == (a.d_gn_b != nullptr) && (a.d_gn_w != nullptr) == (a.d_conv_b != nullptr) &&
                     (a.d_gn_w != nullptr || a.gnpart != nullptr),
                 "cnn_bwd_layer: give either gnpart or all three accumulation targets");
-    const size_t smem = ((size_t)wpc * ka.per_warp + 3 * a.cout) * sizeof(float);
+    smem = ((size_t)wpc * ka.per_warp + 3 * a.cout) * sizeof(float);
     MARLC_CHECK(smem <= 200 * 1024, "cnn_bwd_layer: layer too large for shared memory (%zu B)", smem);
+    return 0;
+}
+
+int cnn_bwd_layer_check(const CnnBwdLayerArgs& a) {
+    CnnBwdLayerKernelArgs ka;
+    int wpc;
+    size_t smem;
+    return bwd_layer_plan(a, ka, wpc, smem);
+}
+
+int cnn_bwd_layer(const CnnBwdLayerArgs& a, cudaStream_t s) {
+    if (a.P <= 0) return 0;
+    CnnBwdLayerKernelArgs ka;
+    int wpc;
+    size_t smem;
+    MARLC_TRY(bwd_layer_plan(a, ka, wpc, smem));
     ka.d_npos = FastDiv((unsigned)ka.npos);
     ka.d_ho = FastDiv((unsigned)a.ho);
     ka.d_co = FastDiv((unsigned)a.cout);
@@ -552,21 +567,36 @@ __global__ void __launch_bounds__(PG_THREADS) cnn_patch_grad_kernel(const PatchG
     }
 }
 
-int cnn_patch_grad(const PatchGradArgs& a, cudaStream_t s) {
+// Launch geometry of cnn_patch_grad (padded channels, windows per CTA, shared memory); fails on shapes it refuses.
+static int patch_grad_plan(const PatchGradArgs& a, int& cinp, int& batch, size_t& smem) {
     MARLC_CHECK(a.dY0 && a.w0 && a.d_patch, "patch_grad: null pointer");
     MARLC_CHECK(a.cin >= 1 && a.cin <= a.C && a.cout >= 1 && a.f >= 1 && a.ho == (a.f - 1) / 2 + 1,
                 "patch_grad: bad CNN shape");
     MARLC_CHECK((a.cout & 3) == 0 && (reinterpret_cast<uintptr_t>(a.dY0) & 15) == 0,
                 "patch_grad: the first conv layer needs a multiple of 4 output channels (has %d)", a.cout);
-    if (a.M <= 0) return 0;
-    const int cinp = (a.cin + IG_CB - 1) / IG_CB * IG_CB;
+    cinp = (a.cin + IG_CB - 1) / IG_CB * IG_CB;
     const int blk = a.ho * a.ho * a.cout, ff = a.f * a.f;
-    const int batch = std::max(1, std::min(PG_MAX_BATCH, PG_STAGE_BYTES / (blk * (int)sizeof(float))));
+    batch = std::max(1, std::min(PG_MAX_BATCH, PG_STAGE_BYTES / (blk * (int)sizeof(float))));
     MARLC_CHECK(FastDiv::exact_up_to((long long)batch * ff, ff) && FastDiv::exact_up_to(ff, a.f) &&
                     FastDiv::exact_up_to((long long)a.cout * a.cin * 9, a.cin),
                 "patch_grad: window of %d x %d too large", a.f, a.f);
-    const size_t smem = ((size_t)9 * a.cout * cinp + (size_t)batch * blk) * sizeof(float);
+    smem = ((size_t)9 * a.cout * cinp + (size_t)batch * blk) * sizeof(float);
     MARLC_CHECK(smem <= 200 * 1024, "patch_grad: first-layer shapes too large for shared memory (%zu B)", smem);
+    return 0;
+}
+
+int cnn_patch_grad_check(const PatchGradArgs& a) {
+    int cinp, batch;
+    size_t smem;
+    return patch_grad_plan(a, cinp, batch, smem);
+}
+
+int cnn_patch_grad(const PatchGradArgs& a, cudaStream_t s) {
+    int cinp, batch;
+    size_t smem;
+    MARLC_TRY(patch_grad_plan(a, cinp, batch, smem));
+    if (a.M <= 0) return 0;
+    const int ff = a.f * a.f;
     static size_t attr = 0;
     if (smem > 48 * 1024 && smem > attr) {
         MARLC_CUDA(cudaFuncSetAttribute(cnn_patch_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

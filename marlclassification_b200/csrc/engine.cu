@@ -523,35 +523,104 @@ static int G_nt(const marlc_engine* e, const float* X, long ldx, const float* W,
     }
     return gemm_nt(X, ldx, W, ldw, bias, Y, ldy, M, N, K, accumulate, s);
 }
+// GEMM arithmetic of a backward product: tensor cores where the shape allows (use_tc), error-compensated 3xTF32
+// there (x3); everything else on the exact-fp32 FFMA kernels
+struct GemmMode { int use_tc, x3; };
+static inline GemmMode gemm_mode(const marlc_engine* e) { return {e->cfg.use_tc, x3_of(e)}; }
+
 // dX[M,K] (+)= dY[M,N] W[N,K]   (reduction over N; W is the MN-major B operand)
-static int G_nn(const marlc_engine* e, const float* dY, long lddy, const float* W, long ldw, float* dX, long lddx, int M,
-                int N, int K, int accumulate, cudaStream_t s) {
-    if (e->cfg.use_tc && tc_worth(M, K, N)) {
+static int G_nn(GemmMode m, const float* dY, long lddy, const float* W, long ldw, float* dX, long lddx, int M, int N,
+                int K, int accumulate, cudaStream_t s) {
+    if (m.use_tc && tc_worth(M, K, N)) {
         TcGemmArgs a;
         a.A = tc_op(dY, lddy); a.B = tc_op(W, ldw, true); a.K = N;
         a.C = dX; a.ldc = lddx; a.M = M; a.N = K; a.accumulate = accumulate;
-        a.x3 = x3_of(e);
+        a.x3 = m.x3;
         a.allow_split = accumulate ? 0 : 1;
         if (tc_operand_ok(a.A) && tc_operand_ok(a.B)) return tc_gemm(a, s);
     }
     return gemm_nn(dY, lddy, W, ldw, dX, lddx, M, N, K, accumulate, s);
 }
-static int G_nn_on(const marlc_engine* e, const float* dY, long lddy, const float* W, long ldw, float* dX, long lddx,
-                   int M, int N, int K, cudaStream_t s) {
-    return G_nn(e, dY, lddy, W, ldw, dX, lddx, M, N, K, 0, s);
+static int G_nn(const marlc_engine* e, const float* dY, long lddy, const float* W, long ldw, float* dX, long lddx, int M,
+                int N, int K, int accumulate, cudaStream_t s) {
+    return G_nn(gemm_mode(e), dY, lddy, W, ldw, dX, lddx, M, N, K, accumulate, s);
 }
 // dW[N,K] += dY[R,N]^T X[R,K]   (reduction over rows R; both operands MN-major)
-static int G_tn(const marlc_engine* e, const float* dY, long lddy, const float* X, long ldx, float* dW, long lddw, int R,
-                int N, int K, cudaStream_t s) {
-    if (e->cfg.use_tc && N > 8 && tc_worth(N, K, R) && K >= 16) {  // N <= 8: one-pass reduction (skinny.cu)
+static int G_tn(GemmMode m, const float* dY, long lddy, const float* X, long ldx, float* dW, long lddw, int R, int N,
+                int K, cudaStream_t s) {
+    if (m.use_tc && N > 8 && tc_worth(N, K, R) && K >= 16) {  // N <= 8: one-pass reduction (skinny.cu)
         TcGemmArgs a;
         a.A = tc_op(dY, lddy, true); a.B = tc_op(X, ldx, true); a.K = R;
         a.C = dW; a.ldc = lddw; a.M = N; a.N = K; a.accumulate = 1;
-        a.x3 = x3_of(e);
+        a.x3 = m.x3;
         a.allow_split = 1;
         if (tc_operand_ok(a.A) && tc_operand_ok(a.B)) return tc_gemm(a, s);
     }
     return gemm_tn(dY, lddy, X, ldx, dW, lddw, R, N, K, 1, s);
+}
+static int G_tn(const marlc_engine* e, const float* dY, long lddy, const float* X, long ldx, float* dW, long lddw, int R,
+                int N, int K, cudaStream_t s) {
+    return G_tn(gemm_mode(e), dY, lddy, X, ldx, dW, lddw, R, N, K, s);
+}
+
+// Layer-wise backward of the feature extractor over P windows (kernels of cnn_bwd2.cu), shared by the episode /
+// step backward and marlc_cnn_backward.  Every conv product is a GEMM: input gradient dCol_l = dY_l W_l, weight
+// gradient dW_l += dY_l^T col_l.  The serial chain on s0 is only layer kernel -> input-gradient GEMM -> next layer
+// kernel; the im2col of the input windows (s1) is independent of it, and the weight-gradient GEMMs wait at the end
+// and fan out over s0 / s1 / sL (through `done`; nullptr when the three are one stream).  GroupNorm-affine and
+// conv-bias gradients are accumulated inside the layer kernel, so d_b / d_gn_w / d_gn_b must all be set.  A null
+// d_w[l] skips layer l's weight-gradient GEMM and the im2col that feeds it (col[l] is not touched).
+struct CnnBwdLayers {
+    const CnnDesc* d;   // shapes and parameters
+    CnnWindows win;     // the input windows (operand of the first layer's weight gradient)
+    int P;              // windows
+    const float* ysave[MAX_CNN_LAYERS];  // [P, cout*ho^2] pre-norm conv outputs, (c, pos) order
+    const float* dOut;  // [P, lddo] gradient on the flattened output, (c, pos) order
+    long lddo;
+    float* dY[MAX_CNN_LAYERS];    // [P*ho^2, cout]
+    float* col[MAX_CNN_LAYERS];   // [P*ho^2, pitch]: pitch round_up(cin*9, 4) for layer 0, cin*9 above
+    float* dcol[MAX_CNN_LAYERS];  // l > 0: [P*ho^2, cin*9]
+    float* d_w[MAX_CNN_LAYERS];   // accumulated into; nullable
+    float* d_b[MAX_CNN_LAYERS];   // accumulated into
+    float* d_gn_w[MAX_CNN_LAYERS];
+    float* d_gn_b[MAX_CNN_LAYERS];
+};
+static int cnn_backward_layers(GemmMode m, const CnnBwdLayers& a, cudaStream_t s0, cudaStream_t s1, cudaStream_t sL,
+                               cudaEvent_t done) {
+    const CnnDesc& d = *a.d;
+    if (a.d_w[0]) MARLC_TRY(cnn_im2col_input(a.win, a.col[0], a.P, d.cin[0], d.hout[0], s1));
+    for (int l = d.L - 1; l >= 0; --l) {
+        CnnBwdLayerArgs la;
+        memset(&la, 0, sizeof(la));
+        la.cout = d.cout[l]; la.ho = d.hout[l]; la.groups = d.groups[l]; la.P = a.P;
+        la.Y = a.ysave[l]; la.gn_w = d.gn_w[l]; la.gn_b = d.gn_b[l];
+        const bool top = (l == d.L - 1);
+        la.dOut = top ? a.dOut : nullptr; la.lddo = a.lddo;
+        la.dColNext = top ? nullptr : a.dcol[l + 1];
+        la.ho_next = top ? 1 : d.hout[l + 1];
+        la.dY = a.dY[l]; la.gnpart = nullptr;
+        la.d_gn_w = a.d_gn_w[l]; la.d_gn_b = a.d_gn_b[l]; la.d_conv_b = a.d_b[l];
+        la.colNext = (top || !a.d_w[l + 1]) ? nullptr : a.col[l + 1];
+        MARLC_TRY(cnn_bwd_layer(la, s0));
+        if (l > 0) {
+            const int npos = d.hout[l] * d.hout[l], kk = d.cin[l] * 9;
+            MARLC_TRY(G_nn(m, a.dY[l], d.cout[l], d.w[l], kk, a.dcol[l], kk, a.P * npos, d.cout[l], kk, 0, s0));
+        }
+    }
+    if (done) {
+        MARLC_CUDA(cudaEventRecord(done, s0));
+        if (s1 != s0) MARLC_CUDA(cudaStreamWaitEvent(s1, done, 0));
+        if (sL != s0) MARLC_CUDA(cudaStreamWaitEvent(sL, done, 0));
+    }
+    // layer 0 reads the im2col of the input windows, produced on s1: it stays on s1
+    const cudaStream_t fan[3] = {s0, s1, sL};
+    for (int l = d.L - 1, i = 0; l >= 0; --l, ++i) {
+        if (!a.d_w[l]) continue;
+        const int npos = d.hout[l] * d.hout[l], kk = d.cin[l] * 9, co = d.cout[l];
+        const int pitch = l == 0 ? (kk + 3) & ~3 : kk;  // the batched im2col pads the input layer's rows
+        MARLC_TRY(G_tn(m, a.dY[l], co, a.col[l], pitch, a.d_w[l], kk, a.P * npos, co, kk, l == 0 ? s1 : fan[(i & 1) ? 2 : 0]));
+    }
+    return 0;
 }
 
 
@@ -1124,75 +1193,46 @@ static int episode_backward(marlc_engine* e, const float* img, int accumulate, c
                                  e->buf("d_pos_y") + r0 * c.n_d, s1));
         MARLC_TRY(G_tn(e, e->buf("d_pos_y") + r0 * c.n_d, c.n_d, e->buf("npos") + r0 * 2, 2, e->grd("map_pos.0.weight"), 2,
                        R, c.n_d, 2, s1));
-        // feature extractor: layer-wise, batched over the chunk's windows (cnn_bwd2.cu); every conv product
+        // feature extractor: layer-wise, batched over the chunk's windows (cnn_backward_layers); every conv product
         // (input gradient dCol_l = dY_l W_l, weight gradient dW_l = dY_l^T col_l) is a tensor-core GEMM
         const CnnDesc& d = e->cnn;
         CnnWindows win{img, e->buf<int>("pos_hist") + r0 * 2, se ? se->patch : nullptr, M, c.nb, c.C, c.H, c.W, c.f};
         if (win.patch) win.patch += r0 * c.C * c.f * c.f;
-        const float* ysave[MAX_CNN_LAYERS];
-        CnnBwdBuffers bb;
-        float* dcol[MAX_CNN_LAYERS] = {nullptr};
-        for (int l = 0; l < e->L; ++l) {
-            const size_t npos = (size_t)d.hout[l] * d.hout[l];
-            ysave[l] = e->buf("cnn_y" + std::to_string(l)) + (par ? r0 * e->cnn_sz[l] : 0);
-            bb.dY[l] = e->buf("cnn_dY" + std::to_string(l)) + (par ? r0 * npos * d.cout[l] : 0);
-            bb.col[l] = e->buf("cnn_col" + std::to_string(l)) + (par ? r0 * npos * (size_t)((d.cin[l] * 9 + 3) & ~3) : 0);
-            bb.gnpart[l] = e->buf("cnn_gnpart" + std::to_string(l)) + (par ? r0 * 2 * d.cout[l] : 0);
-            if (l > 0) dcol[l] = e->buf("cnn_dcol" + std::to_string(l)) + (par ? r0 * npos * d.cin[l] * 9 : 0);
-        }
-        auto conv_weight_grad = [&](int l, cudaStream_t st) -> int {
-            const int npos = d.hout[l] * d.hout[l], kk = d.cin[l] * 9, co = d.cout[l];
-            const int pitch = (par && l == 0) ? (kk + 3) & ~3 : kk;  // the batched im2col pads the input layer's rows
-            return G_tn(e, bb.dY[l], co, bb.col[l], pitch, e->grd(CNN_PREFIX + std::to_string(3 * l) + ".weight"), kk,
-                        R * npos, co, kk, st);
-        };
         if (!par) {  // unfused reference path: one whole-episode call of the per-window kernel
+            const float* ysave[MAX_CNN_LAYERS];
+            CnnBwdBuffers bb;
+            for (int l = 0; l < e->L; ++l) {
+                ysave[l] = e->buf("cnn_y" + std::to_string(l));
+                bb.dY[l] = e->buf("cnn_dY" + std::to_string(l));
+                bb.col[l] = e->buf("cnn_col" + std::to_string(l));
+                bb.gnpart[l] = e->buf("cnn_gnpart" + std::to_string(l));
+            }
             MARLC_TRY(cnn_bwd(e->cnn, win, 0, TM, ysave, dU, Kin, bb, s0));
             for (int l = 0; l < e->L; ++l) {
-                const int npos = d.hout[l] * d.hout[l], co = d.cout[l];
+                const int npos = d.hout[l] * d.hout[l], kk = d.cin[l] * 9, co = d.cout[l];
                 const std::string cw = CNN_PREFIX + std::to_string(3 * l), gn = CNN_PREFIX + std::to_string(3 * l + 1);
-                MARLC_TRY(conv_weight_grad(l, s0));
+                MARLC_TRY(G_tn(e, bb.dY[l], co, bb.col[l], kk, e->grd(cw + ".weight"), kk, R * npos, co, kk, s0));
                 MARLC_TRY(colsum_add(bb.dY[l], co, e->grd(cw + ".bias"), R * npos, co, s0));
                 MARLC_TRY(colsum_add(bb.gnpart[l], 2 * co, e->grd(gn + ".weight"), R, co, s0));
                 MARLC_TRY(colsum_add(bb.gnpart[l] + co, 2 * co, e->grd(gn + ".bias"), R, co, s0));
             }
             return 0;
         }
-        // The serial chain is only layer kernel -> input-gradient GEMM -> next layer kernel; the im2col
-        // of the input windows is independent of it (stream s1), and the weight-gradient GEMMs wait at
-        // the end and fan out over the three streams.  GroupNorm-affine and conv-bias gradients are
-        // accumulated inside the layer kernel.
-        MARLC_TRY(cnn_im2col_input(win, bb.col[0], R, d.cin[0], d.hout[0], s1));
-        for (int l = e->L - 1; l >= 0; --l) {
-            CnnBwdLayerArgs la;
-            memset(&la, 0, sizeof(la));
-            la.cout = d.cout[l]; la.ho = d.hout[l]; la.groups = d.groups[l]; la.P = R;
-            la.Y = ysave[l]; la.gn_w = d.gn_w[l]; la.gn_b = d.gn_b[l];
-            const bool top = (l == e->L - 1);
-            la.dOut = top ? dU + r0 * Kin : nullptr; la.lddo = Kin;
-            la.dColNext = top ? nullptr : dcol[l + 1];
-            la.ho_next = top ? 1 : d.hout[l + 1];
-            la.dY = bb.dY[l]; la.gnpart = nullptr;
-            la.d_gn_w = e->grd(CNN_PREFIX + std::to_string(3 * l + 1) + ".weight");
-            la.d_gn_b = e->grd(CNN_PREFIX + std::to_string(3 * l + 1) + ".bias");
-            la.d_conv_b = e->grd(CNN_PREFIX + std::to_string(3 * l) + ".bias");
-            la.colNext = top ? nullptr : bb.col[l + 1];
-            MARLC_TRY(cnn_bwd_layer(la, s0));
-            if (l > 0) {
-                const int npos = d.hout[l] * d.hout[l], kk = d.cin[l] * 9;
-                MARLC_TRY(G_nn_on(e, bb.dY[l], d.cout[l], d.w[l], kk, dcol[l], kk, R * npos, d.cout[l], kk, s0));
-            }
+        CnnBwdLayers cb;
+        memset(&cb, 0, sizeof(cb));
+        cb.d = &d; cb.win = win; cb.P = R;
+        cb.dOut = dU + r0 * Kin; cb.lddo = Kin;
+        for (int l = 0; l < e->L; ++l) {
+            const size_t npos = (size_t)d.hout[l] * d.hout[l];
+            const std::string cw = CNN_PREFIX + std::to_string(3 * l), gn = CNN_PREFIX + std::to_string(3 * l + 1);
+            cb.ysave[l] = e->buf("cnn_y" + std::to_string(l)) + r0 * e->cnn_sz[l];
+            cb.dY[l] = e->buf("cnn_dY" + std::to_string(l)) + r0 * npos * d.cout[l];
+            cb.col[l] = e->buf("cnn_col" + std::to_string(l)) + r0 * npos * (size_t)((d.cin[l] * 9 + 3) & ~3);
+            if (l > 0) cb.dcol[l] = e->buf("cnn_dcol" + std::to_string(l)) + r0 * npos * d.cin[l] * 9;
+            cb.d_w[l] = e->grd(cw + ".weight"); cb.d_b[l] = e->grd(cw + ".bias");
+            cb.d_gn_w[l] = e->grd(gn + ".weight"); cb.d_gn_b[l] = e->grd(gn + ".bias");
         }
-        {
-            cudaStream_t fan[3] = {s0, s1, sL};
-            cudaEvent_t done = e->next_event();
-            MARLC_CUDA(cudaEventRecord(done, s0));
-            if (s1 != s0) MARLC_CUDA(cudaStreamWaitEvent(s1, done, 0));
-            if (sL != s0) MARLC_CUDA(cudaStreamWaitEvent(sL, done, 0));
-            // layer 0 reads the im2col of the input windows, produced on s1: it stays on s1
-            for (int l = e->L - 1, i = 0; l >= 0; --l, ++i) MARLC_TRY(conv_weight_grad(l, l == 0 ? s1 : fan[(i & 1) ? 2 : 0]));
-        }
-        return 0;
+        return cnn_backward_layers(gemm_mode(e), cb, s0, s1, sL, e->next_event());
     };
     // ---- BPTT sweep
     NvtxRange nvtx_sweep("marlc/backward/sweep");
@@ -1602,23 +1642,152 @@ extern "C" int marlc_msg_mean(const float* msg, float* out, int Na, int Nb, int 
     return msg_mean(msg, out, Na, Nb, n, (cudaStream_t)stream);
 }
 
-// _Generic2dCnnModule.forward, vision.py:47-49 on N stand-alone windows [N, img_c, f, f]
-extern "C" int marlc_cnn_forward(int layers, const int* cin, const int* cout, const int* groups, int f, int img_c,
-                                 const float* const* w, const float* const* b, const float* const* gn_w,
-                                 const float* const* gn_b, const float* patch, float* out, int N, void* stream) {
-    MARLC_CHECK(layers >= 1 && layers <= MAX_CNN_LAYERS, "cnn_forward: %d layers unsupported", layers);
-    MARLC_CHECK(patch && out, "cnn_forward: null pointer");
-    CnnDesc d;
+// Description of a stand-alone feature extractor (no engine) from the caller's host arrays; the shapes are checked
+static int standalone_cnn_desc(CnnDesc& d, const char* who, int layers, const int* cin, const int* cout,
+                               const int* groups, int f, int img_c, const float* const* w, const float* const* b,
+                               const float* const* gn_w, const float* const* gn_b) {
+    MARLC_CHECK(layers >= 1 && layers <= MAX_CNN_LAYERS, "%s: %d layers unsupported", who, layers);
+    MARLC_CHECK(cin && cout && groups && w && b && gn_w && gn_b, "%s: null pointer", who);
     memset(&d, 0, sizeof(d));
     d.L = layers; d.f = f; d.img_c = img_c;
     int h = f;
     for (int l = 0; l < layers; ++l) {
+        MARLC_CHECK(cin[l] >= 1 && cout[l] >= 1 && groups[l] >= 1 && cout[l] % groups[l] == 0 &&
+                        (l == 0 || cin[l] == cout[l - 1]),
+                    "%s: bad shape of layer %d (cin %d, cout %d, groups %d)", who, l, cin[l], cout[l], groups[l]);
         d.cin[l] = cin[l]; d.cout[l] = cout[l]; d.groups[l] = groups[l];
         d.hin[l] = h; h = (h - 1) / 2 + 1; d.hout[l] = h;
         d.w[l] = w[l]; d.b[l] = b[l]; d.gn_w[l] = gn_w[l]; d.gn_b[l] = gn_b[l];
     }
+    MARLC_CHECK(f >= 1 && img_c >= cin[0], "%s: window %d x %d with %d channels, the first layer reads %d", who, f, f,
+                img_c, cin[0]);
     d.out_size = d.cout[layers - 1] * h * h;
-    return cnn_fwd(d, nullptr, nullptr, patch, 1, f, f, N, nullptr, out, d.out_size, (cudaStream_t)stream);
+    return 0;
+}
+
+// _Generic2dCnnModule.forward, vision.py:47-49 on N stand-alone windows [N, img_c, f, f]
+extern "C" int marlc_cnn_forward_save(int layers, const int* cin, const int* cout, const int* groups, int f, int img_c,
+                                      const float* const* w, const float* const* b, const float* const* gn_w,
+                                      const float* const* gn_b, const float* patch, float* const* y_save, float* out,
+                                      int N, void* stream) {
+    CnnDesc d;
+    MARLC_TRY(standalone_cnn_desc(d, "cnn_forward", layers, cin, cout, groups, f, img_c, w, b, gn_w, gn_b));
+    MARLC_CHECK(patch && out, "cnn_forward: null pointer");
+    return cnn_fwd(d, nullptr, nullptr, patch, 1, f, f, N, y_save, out, d.out_size, (cudaStream_t)stream);
+}
+extern "C" int marlc_cnn_forward(int layers, const int* cin, const int* cout, const int* groups, int f, int img_c,
+                                 const float* const* w, const float* const* b, const float* const* gn_w,
+                                 const float* const* gn_b, const float* patch, float* out, int N, void* stream) {
+    return marlc_cnn_forward_save(layers, cin, cout, groups, f, img_c, w, b, gn_w, gn_b, patch, nullptr, out, N, stream);
+}
+
+// Workspace of marlc_cnn_backward: 256-byte aligned sections, per layer dY [N*ho^2, cout], dCol (l > 0)
+// [N*ho^2, cin*9], with parameter gradients the im2col rows col [N*ho^2, pitch] (pitch round_up(cin*9, 4) for the
+// first layer, cin*9 above), and 3 x cout floats of accumulation targets for the conv-bias / GroupNorm-affine
+// gradients the caller did not ask for (the layer kernel always accumulates them).
+struct CnnBwdWorkspace {
+    size_t dY[MAX_CNN_LAYERS], dcol[MAX_CNN_LAYERS], col[MAX_CNN_LAYERS], scratch[MAX_CNN_LAYERS];
+    size_t bytes;
+};
+static CnnBwdWorkspace cnn_bwd_workspace(const CnnDesc& d, long N, bool param_grads) {
+    CnnBwdWorkspace ws;
+    memset(&ws, 0, sizeof(ws));
+    auto take = [&](size_t floats) {
+        const size_t at = ws.bytes;
+        ws.bytes += (floats * sizeof(float) + 255) / 256 * 256;
+        return at;
+    };
+    for (int l = 0; l < d.L; ++l) {
+        const size_t rows = (size_t)N * d.hout[l] * d.hout[l], kk = (size_t)d.cin[l] * 9;
+        ws.dY[l] = take(rows * d.cout[l]);
+        if (l > 0) ws.dcol[l] = take(rows * kk);
+        if (param_grads) ws.col[l] = take(rows * (l == 0 ? (kk + 3) & ~(size_t)3 : kk));
+        ws.scratch[l] = take(3 * (size_t)d.cout[l]);
+    }
+    return ws;
+}
+
+extern "C" size_t marlc_cnn_backward_workspace_bytes(int layers, const int* cin, const int* cout, int f, int N,
+                                                     int want_param_grads) {
+    // 0 = bad argument: a valid request always includes the scratch targets
+    if (!(layers >= 1 && layers <= MAX_CNN_LAYERS && cin && cout && f >= 1 && N >= 0)) {
+        set_error("cnn_backward_workspace_bytes: bad argument (layers %d, f %d, N %d)", layers, f, N);
+        return 0;
+    }
+    CnnDesc d;
+    memset(&d, 0, sizeof(d));
+    d.L = layers;
+    for (int l = 0, h = f; l < layers; ++l) {
+        if (cin[l] < 1 || cout[l] < 1) {
+            set_error("cnn_backward_workspace_bytes: bad shape of layer %d (cin %d, cout %d)", l, cin[l], cout[l]);
+            return 0;
+        }
+        d.cin[l] = cin[l]; d.cout[l] = cout[l];
+        h = (h - 1) / 2 + 1; d.hout[l] = h;
+    }
+    return cnn_bwd_workspace(d, N, want_param_grads != 0).bytes;
+}
+
+// Backward of marlc_cnn_forward_save on the caller's windows: the layer-wise path of the episode backward
+// (cnn_backward_layers) on one stream, in 3xTF32 on the tensor cores where operands are TMA-addressable, then the
+// first layer's transposed convolution into d_patch (see include/marlc.h).
+extern "C" int marlc_cnn_backward(int layers, const int* cin, const int* cout, const int* groups, int f, int img_c,
+                                  const float* const* w, const float* const* b, const float* const* gn_w,
+                                  const float* const* gn_b, const float* patch, const float* const* y_save,
+                                  const float* d_out, int N, void* workspace, size_t workspace_bytes, float* d_patch,
+                                  float* const* d_w, float* const* d_b, float* const* d_gn_w,
+                                  float* const* d_gn_b, void* stream) {
+    CnnDesc d;
+    MARLC_TRY(standalone_cnn_desc(d, "cnn_backward", layers, cin, cout, groups, f, img_c, w, b, gn_w, gn_b));
+    MARLC_CHECK(N >= 0 && (long)N * d.hout[0] * d.hout[0] <= INT32_MAX, "cnn_backward: %d windows unsupported", N);
+    MARLC_CHECK(y_save && workspace, "cnn_backward: null pointer");
+    if (N == 0) return 0;
+    MARLC_CHECK(patch && d_out, "cnn_backward: null pointer");
+    bool param_grads = false;
+    for (int l = 0; l < layers; ++l) {
+        MARLC_CHECK(w[l] && b[l] && gn_w[l] && gn_b[l] && y_save[l], "cnn_backward: null pointer (layer %d)", l);
+        param_grads = param_grads || (d_w && d_w[l]);
+    }
+    const CnnBwdWorkspace ws = cnn_bwd_workspace(d, N, param_grads);
+    MARLC_CHECK((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "cnn_backward: workspace not 256-byte aligned");
+    MARLC_CHECK(workspace_bytes >= ws.bytes,
+                "cnn_backward: workspace of %zu bytes, need %zu (marlc_cnn_backward_workspace_bytes with "
+                "want_param_grads = %d)", workspace_bytes, ws.bytes, param_grads ? 1 : 0);
+    char* base = static_cast<char*>(workspace);
+    CnnBwdLayers cb;
+    memset(&cb, 0, sizeof(cb));
+    cb.d = &d; cb.win = CnnWindows{nullptr, nullptr, patch, N, 1, img_c, f, f, f}; cb.P = N;
+    cb.dOut = d_out; cb.lddo = d.out_size;
+    for (int l = 0; l < layers; ++l) {
+        float* scratch = reinterpret_cast<float*>(base + ws.scratch[l]);
+        cb.ysave[l] = y_save[l];
+        cb.dY[l] = reinterpret_cast<float*>(base + ws.dY[l]);
+        cb.dcol[l] = l > 0 ? reinterpret_cast<float*>(base + ws.dcol[l]) : nullptr;
+        cb.col[l] = param_grads ? reinterpret_cast<float*>(base + ws.col[l]) : nullptr;
+        cb.d_w[l] = d_w ? d_w[l] : nullptr;
+        cb.d_b[l] = (d_b && d_b[l]) ? d_b[l] : scratch + 2 * d.cout[l];
+        cb.d_gn_w[l] = (d_gn_w && d_gn_w[l]) ? d_gn_w[l] : scratch;
+        cb.d_gn_b[l] = (d_gn_b && d_gn_b[l]) ? d_gn_b[l] : scratch + d.cout[l];
+    }
+    // every launcher's host-side checks before the first launch
+    for (int l = layers - 1; l >= 0; --l) {
+        CnnBwdLayerArgs la;
+        memset(&la, 0, sizeof(la));
+        la.cout = d.cout[l]; la.ho = d.hout[l]; la.P = N;
+        la.dOut = l == layers - 1 ? d_out : nullptr;
+        la.ho_next = l == layers - 1 ? 1 : d.hout[l + 1];
+        la.d_gn_w = cb.d_gn_w[l]; la.d_gn_b = cb.d_gn_b[l]; la.d_conv_b = cb.d_b[l];
+        MARLC_TRY(cnn_bwd_layer_check(la));
+    }
+    PatchGradArgs pg;
+    pg.dY0 = cb.dY[0]; pg.w0 = d.w[0]; pg.d_patch = d_patch;
+    pg.M = N; pg.C = img_c; pg.f = f; pg.cin = d.cin[0]; pg.cout = d.cout[0]; pg.ho = d.hout[0];
+    if (d_patch) MARLC_TRY(cnn_patch_grad_check(pg));
+    cudaStream_t s = (cudaStream_t)stream;
+    NvtxRange nvtx("marlc/cnn_backward");
+    MARLC_TRY(cnn_backward_layers(GemmMode{1, 1}, cb, s, s, s, nullptr));
+    if (d_patch) MARLC_TRY(cnn_patch_grad(pg, s));
+    return 0;
 }
 
 // Tensor-core GEMM, exposed for unit tests: C[M,N] (+)= A.B^T (+ A2.B2^T) (+ bias).

@@ -128,6 +128,8 @@ struct CnnBwdLayerArgs {
     float* colNext;         // out im2col of this layer's activation for layer l+1 (nullptr for the top layer)
 };
 int cnn_bwd_layer(const CnnBwdLayerArgs& a, cudaStream_t s);
+// The host-side checks of cnn_bwd_layer alone (accumulation targets, shared memory): nothing is launched.
+int cnn_bwd_layer_check(const CnnBwdLayerArgs& a);
 int cnn_im2col_input(const CnnWindows& win, float* col, int P, int cin, int ho, cudaStream_t s);
 // Gradient on the image batch from the first layer's conv-output gradients of all T*M windows: the transposed
 // convolution with W_0 fused with the adjoint of the window gather (a pixel sums every window covering it).
@@ -148,6 +150,8 @@ struct PatchGradArgs {
     int M, C, f, cin, cout, ho;
 };
 int cnn_patch_grad(const PatchGradArgs& a, cudaStream_t s);
+// The host-side checks of cnn_patch_grad alone (pointers, shapes, shared memory): nothing is launched.
+int cnn_patch_grad_check(const PatchGradArgs& a);
 
 // ---- loss.cu ------------------------------------------------------------------
 struct LossArgs {

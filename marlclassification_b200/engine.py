@@ -14,9 +14,11 @@ the reference's own loss code (``loss.backward()``) works unchanged.
 from __future__ import annotations
 
 import ctypes as ct
+import weakref
 from typing import Optional, Sequence
 
 import torch as th
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 from ._lib import MarlcConfig
@@ -354,6 +356,23 @@ def _step_outputs(eng: EpisodeEngine):
             eng.H_state[1].clone(), eng.C_state[1].clone(), eng.Hc_state[1].clone(), eng.Cc_state[1].clone())
 
 
+def _grad_into_bucket(p, flat_params: th.Tensor, flat_grads: th.Tensor) -> None:
+    """Before a backward node returns a gradient for ``p``, a view of a ModelsWrapper's ``flat_params``: autograd adds
+    each parameter gradient into param.grad in place, so make param.grad the parameter's slot of ``flat_grads`` and
+    the bucket the fused Adam (and the data-parallel all-reduce) reads and param.grad stay one tensor.  After
+    zero_grad(set_to_none=True) param.grad is None: the slot starts from zero.  A gradient held outside the bucket
+    (e.g. the one a run_episode backward left after set_to_none) moves into the slot."""
+    if p.grad is not None and p.grad.untyped_storage().data_ptr() == flat_grads.untyped_storage().data_ptr():
+        return
+    off = (p.data.data_ptr() - flat_params.data_ptr()) // 4
+    slot = flat_grads[off: off + p.numel()].view(p.shape)
+    if p.grad is None:
+        slot.zero_()
+    else:
+        slot.copy_(p.grad)
+    p.grad = slot
+
+
 class _StepFn(th.autograd.Function):
     """ModelsWrapper.forward as one autograd node (``model.differentiable_steps``).  Forward = marlc_model_step;
     backward = marlc_model_step_backward, which re-runs the step from the saved inputs (the next step-wise call
@@ -391,24 +410,14 @@ class _StepFn(th.autograd.Function):
         d_npos = th.empty_like(npos) if need[4] else None
         if need[2] or need[4]:
             eng.step_input_grad(d_patch, d_npos)
-        # autograd adds each parameter gradient into param.grad in place: make sure param.grad is the parameter's
-        # slot of model.flat_grads, so the bucket the fused Adam reads and param.grad stay one tensor.  After
-        # zero_grad(set_to_none=True) param.grad is None: the slot starts from zero.  A gradient held outside
-        # the bucket (e.g. the one a run_episode backward left after set_to_none) moves into the slot.
-        base, bucket = flat.data_ptr(), model.flat_grads
+        base = flat.data_ptr()
         out = []
         for i, p in enumerate(ctx.params):
             if not need[9 + i]:
                 out.append(None)
                 continue
+            _grad_into_bucket(p, flat, model.flat_grads)
             off = (p.data.data_ptr() - base) // 4
-            if p.grad is None or p.grad.untyped_storage().data_ptr() != bucket.untyped_storage().data_ptr():
-                slot = bucket[off: off + p.numel()].view(p.shape)
-                if p.grad is None:
-                    slot.zero_()
-                else:
-                    slot.copy_(p.grad)
-                p.grad = slot
             out.append(grads[off: off + p.numel()].view(p.shape))
         return (None, None, d_patch, d_in[0], d_npos, *d_in[1:], *out)
 
@@ -449,26 +458,117 @@ def model_step(model, img_patch, msg_t, norm_pos, hidden):
     return out, rec
 
 
+# feature extractor -> weak reference to the ModelsWrapper whose flat buckets hold its parameters
+# (registered by ModelsWrapper.ensure_flat; a weak mapping so that neither module is kept alive or pickled by it)
+_FLAT_OWNER: "weakref.WeakKeyDictionary" = weakref.WeakKeyDictionary()
+
+
+def register_flat_owner(module, model) -> None:
+    _FLAT_OWNER[module] = weakref.ref(model)
+
+
+class _CnnArgs:
+    """The C-ABI arguments of one stand-alone feature extractor: shapes as ctypes arrays, and the parameters in
+    module order (conv.weight, conv.bias, norm.weight, norm.bias per layer)."""
+
+    def __init__(self, module, x: th.Tensor) -> None:
+        f, layers, groups, _ = module.cnn_spec
+        self.L, self.f, self.n, self.c_img = len(layers), f, x.shape[0], x.shape[1]
+        if x.shape[2] != f or x.shape[3] != f or self.c_img < layers[0][0]:
+            raise RuntimeError(f"CNN expects [N,>={layers[0][0]},{f},{f}], got {tuple(x.shape)}")
+        self.out_size = module.out_size
+        arr = lambda vals: (ct.c_int * self.L)(*vals)  # noqa: E731
+        self.cin, self.cout, self.groups = arr([ci for ci, _ in layers]), arr([co for _, co in layers]), arr(groups)
+        self.y_sizes = []
+        side = f
+        for _, co in layers:
+            side = (side - 1) // 2 + 1
+            self.y_sizes.append(co * side * side)
+        seq = [m for m in module.modules() if isinstance(m, (th.nn.Conv2d, th.nn.GroupNorm))]
+        self.params = [t for conv, norm in zip(seq[0::2], seq[1::2])
+                       for t in (conv.weight, conv.bias, norm.weight, norm.bias)]
+
+    def ptrs(self, ts) -> ct.Array:
+        """Host array of the device pointers of ts[0], ts[4], ... (one per layer; None -> nullptr)."""
+        return (ct.c_void_p * self.L)(*[_lib.ptr(t) for t in ts])
+
+    def param_ptrs(self, ps):
+        ps = [t.detach().contiguous() for t in ps]
+        for t in ps:
+            _lib.require_cuda(t, "CNN parameter", th.float32)
+        return ps, [self.ptrs(ps[k::4]) for k in range(4)]
+
+    def forward(self, x: th.Tensor, ps, y_save=None) -> th.Tensor:
+        ps, (w, b, gw, gb) = self.param_ptrs(ps)
+        out = th.empty(self.n, self.out_size, dtype=th.float32, device=x.device)
+        stream = _lib.stream_ptr(x.device)
+        L = _lib.lib()
+        if y_save is None:
+            _lib.check(L.marlc_cnn_forward(self.L, self.cin, self.cout, self.groups, self.f, self.c_img, w, b, gw, gb,
+                                           x.data_ptr(), out.data_ptr(), self.n, stream))
+        else:
+            _lib.check(L.marlc_cnn_forward_save(self.L, self.cin, self.cout, self.groups, self.f, self.c_img, w, b, gw,
+                                                gb, x.data_ptr(), self.ptrs(y_save), out.data_ptr(), self.n, stream))
+        return out
+
+
+class _CnnFn(th.autograd.Function):
+    """_Generic2dCnnModule.forward as one autograd node.  Forward = marlc_cnn_forward_save (the same bits as the
+    forward-only call) keeping every layer's pre-norm conv outputs; backward = marlc_cnn_backward, into the windows
+    and, when any parameter needs a gradient, into all of them.  The parameters are saved for backward, so an
+    in-place update between forward and backward raises (torch's version check).  Parameters of a feature
+    extractor inside a flattened ModelsWrapper get their gradients in their slots of the wrapper's flat_grads."""
+
+    @staticmethod
+    def forward(ctx, module, x, *params):
+        a = _CnnArgs(module, x)
+        y_save = [th.empty(x.shape[0], n, dtype=th.float32, device=x.device) for n in a.y_sizes]
+        out = a.forward(x, params, y_save)
+        ctx.module, ctx.params = module, params
+        ctx.save_for_backward(x, *params, *y_save)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, d_out):
+        module = ctx.module
+        x, *rest = ctx.saved_tensors
+        a = _CnnArgs(module, x)
+        params, y_save = rest[:4 * a.L], rest[4 * a.L:]
+        need = ctx.needs_input_grad
+        want_params = any(need[2:])
+        d_out = d_out.float().contiguous()
+        L = _lib.lib()
+        nbytes = L.marlc_cnn_backward_workspace_bytes(a.L, a.cin, a.cout, a.f, a.n, int(want_params))
+        if nbytes == 0:
+            raise RuntimeError("libmarlc: " + L.marlc_last_error().decode())
+        ws = th.empty(nbytes, dtype=th.uint8, device=x.device)
+        d_x = th.empty_like(x) if need[1] else None
+        grads = [th.zeros_like(p) for p in params] if want_params else [None] * len(params)
+        g_ptrs = [a.ptrs(grads[k::4]) for k in range(4)] if want_params else [None] * 4
+        ps, (w, b, gw, gb) = a.param_ptrs(params)
+        _lib.check(L.marlc_cnn_backward(a.L, a.cin, a.cout, a.groups, a.f, a.c_img, w, b, gw, gb, x.data_ptr(),
+                                        a.ptrs(y_save), d_out.data_ptr(), a.n, ws.data_ptr(), nbytes, _lib.ptr(d_x),
+                                        *g_ptrs, _lib.stream_ptr(x.device)))
+        owner = _FLAT_OWNER.get(module)
+        model = owner() if owner is not None else None
+        flat = model._flat_params if model is not None else None
+        out = []
+        for i, (p, g) in enumerate(zip(ctx.params, grads)):
+            if not need[2 + i]:
+                out.append(None)
+                continue
+            if flat is not None and p.data.untyped_storage().data_ptr() == flat.untyped_storage().data_ptr():
+                _grad_into_bucket(p, flat, model._flat_grads)
+            out.append(g)
+        return (None, d_x, *out)
+
+
 def cnn_forward(module, o_t: th.Tensor) -> th.Tensor:
-    """_Generic2dCnnModule.forward (vision.py:47-49) on [N,C,f,f] windows."""
+    """_Generic2dCnnModule.forward (vision.py:47-49) on [N,C,f,f] windows.  In grad mode, when the windows or a
+    conv / GroupNorm parameter require grad, the output carries a backward (_CnnFn); otherwise forward only."""
     x = _lib.require_cuda(o_t, "o_t", th.float32)
-    f, layers, groups, _ = module.cnn_spec
-    n, c_img = x.shape[0], x.shape[1]
-    if x.shape[2] != f or x.shape[3] != f or c_img < layers[0][0]:
-        raise RuntimeError(f"CNN expects [N,>={layers[0][0]},{f},{f}], got {tuple(x.shape)}")
-    L = len(layers)
-    seq = [m for m in module.modules() if isinstance(m, (th.nn.Conv2d, th.nn.GroupNorm))]
-    convs, norms = seq[0::2], seq[1::2]
-    arr = lambda vals: (ct.c_int * L)(*vals)  # noqa: E731
-    parr = lambda ts: (ct.c_void_p * L)(*[t.data_ptr() for t in ts])  # noqa: E731
-    w = [m.weight.detach().contiguous() for m in convs]
-    b = [m.bias.detach().contiguous() for m in convs]
-    gw = [m.weight.detach().contiguous() for m in norms]
-    gb = [m.bias.detach().contiguous() for m in norms]
-    for t in w + b + gw + gb:
-        _lib.require_cuda(t, "CNN parameter", th.float32)
-    out = th.empty(n, module.out_size, dtype=th.float32, device=x.device)
-    _lib.check(_lib.lib().marlc_cnn_forward(
-        L, arr([ci for ci, _ in layers]), arr([co for _, co in layers]), arr(groups), f, c_img,
-        parr(w), parr(b), parr(gw), parr(gb), x.data_ptr(), out.data_ptr(), n, _lib.stream_ptr(x.device)))
-    return out
+    a = _CnnArgs(module, x)
+    if th.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in a.params)):
+        return _CnnFn.apply(module, x, *a.params)
+    return a.forward(x, a.params)

@@ -88,13 +88,35 @@ def init_layers(m: nn.Module) -> None:
             nn.init.zeros_(m.bias)
 
 
-def aggregate_messages(messages: th.Tensor) -> th.Tensor:
-    """Mean of the OTHER agents' messages (message.py:5-17), CUDA kernel
-    csrc/rowwise.cu::msg_mean_kernel (warp-shuffle reduction over agents)."""
+def _msg_mean(msg: th.Tensor) -> th.Tensor:
     from .. import _lib
 
-    msg = _lib.require_cuda(messages, "aggregate_messages", th.float32)
     out = th.empty_like(msg)
     na, nb, n = msg.shape
     _lib.check(_lib.lib().marlc_msg_mean(msg.data_ptr(), out.data_ptr(), na, nb, n, _lib.stream_ptr(msg.device)))
     return out
+
+
+class _MsgMeanFn(th.autograd.Function):
+    """The mean of the other agents' messages is a symmetric linear map over the agents (out_a = (S - m_a) /
+    (Na - 1)), so it is its own adjoint: the backward is the same kernel on the incoming gradient (exactly 0 for
+    Na = 1)."""
+
+    @staticmethod
+    def forward(ctx, msg):
+        return _msg_mean(msg)
+
+    @staticmethod
+    def backward(ctx, grad):
+        return _MsgMeanFn.apply(grad.float().contiguous())
+
+
+def aggregate_messages(messages: th.Tensor) -> th.Tensor:
+    """Mean of the OTHER agents' messages (message.py:5-17), CUDA kernel
+    csrc/rowwise.cu::msg_mean_kernel (warp-shuffle reduction over agents); differentiable in ``messages``."""
+    from .. import _lib
+
+    msg = _lib.require_cuda(messages, "aggregate_messages", th.float32)
+    if th.is_grad_enabled() and msg.requires_grad:
+        return _MsgMeanFn.apply(msg)
+    return _msg_mean(msg)

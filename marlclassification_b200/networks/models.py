@@ -204,6 +204,9 @@ class ModelsWrapper(nn.Module):
                 p.grad = grads[off:off + n].view(shape)
         self._flat_params, self._flat_grads = flat, grads
         self._engines.clear()
+        from ..engine import register_flat_owner
+
+        register_flat_owner(self.__map_obs, self)  # a stand-alone feature-extractor backward fills this bucket too
 
     def attach_grads(self) -> None:
         """Point every ``param.grad`` at its slot of the flat bucket (after
